@@ -3,6 +3,12 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (one process per GPU under torchrun)
     python bench.py --impl reference [--gpus N] [--steps K] ...     # the reference's CPU path (oracle restatement)
+    python bench.py ... --dump-outputs DIR     # also write the last timed step's loss and weights as DIR/<name>.npy
+
+The same arguments give the same seeded batches and initial weights on every run.  The timed step adds its gradients
+with float atomics, whose rounding changes from run to run, and the max over the negatives grows that into different
+training trajectories within a few steps.  With --dump-outputs the last timed step therefore starts again from the
+seeded weights and Adagrad accumulators, so what it writes differs between two runs of one build by rounding only.
 
 Workload (BASELINE.json configs[1]): OurModel7 (HHFM) training on frappe-10-shaped synthetic data -- 10 fields
 (user 957, item 4082, 8 context columns, 343 values), features_M = 5382, K = 64, NG = 10 negatives, Adagrad lr 0.1,
@@ -522,6 +528,15 @@ def measured_traffic(kernel):
     return d.get("dram_bytes_per_launch"), d.get("capture")
 
 
+def dump_outputs(out_dir, arrays):
+    """Write every array as `out_dir/<name>.npy` (float64 stays float64, everything else becomes float32), so that two
+    builds run with the same arguments -- and therefore the same seeded inputs -- can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
+
+
 def dp_check(model, rec, n_ctx, world, dev):
     """N > 1 correctness evidence carried by the bench line itself (the driver's test box has one GPU): one more step whose
     update is recomputed from an NCCL all-reduce of the ranks' gradients, and a bit-comparison of the replicas."""
@@ -649,6 +664,8 @@ def run_ours(args):
     if world > 1:
         model.enable_data_parallel()
     host_batches = [make_batch(rng, B) for _ in range(n_batches)]
+    # --dump-outputs: the seeded weights the last timed step restarts from (see the module docstring)
+    V_seed = model.weights["feature_embeddings"].clone() if args.dump_outputs else None
 
     # device-resident records (the `value` arm): same packing as partial_fit, done once
     dev_batches = []
@@ -697,6 +714,9 @@ def run_ours(args):
     calls0 = dict(_lib.CALLS)
     t_start.record()
     for i in range(args.steps):
+        if V_seed is not None and i == args.steps - 1:
+            model.weights["feature_embeddings"].copy_(V_seed)
+            model._opt.slots("feature_embeddings", model.weights["feature_embeddings"])[0].fill_(model._opt.acc0)
         device_step(args.warmup + i, timed_idx=i)
     t_end.record()
     calls1 = dict(_lib.CALLS)
@@ -707,6 +727,12 @@ def run_ours(args):
     kern_ms = sum(ev[2 * i].elapsed_time(ev[2 * i + 1]) for i in range(args.steps)) / args.steps
     loss_value = model._read_loss()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed step holds after its last step: that step's loss and the updated weights
+        # (the replicas are bit-identical under data parallelism, so rank 0 speaks for all)
+        outs = {"loss": np.array([loss_value], dtype=np.float32)}
+        outs.update(model.get_weights())
+        dump_outputs(args.dump_outputs, outs)
     # every timed entry point launches exactly one kernel (pairrank_sum_train_kernel, dp_step_kernel; without the fused
     # tail: hot_fold, opt_dense, loss_finalize)
     launches = sum(calls1.get(k, 0) - calls0.get(k, 0) for k in calls1)
@@ -857,7 +883,13 @@ def main():
     ap.add_argument("--no-models", dest="no_models", action="store_true", help="skip the per-model secondary lines")
     ap.add_argument("--no-bands", dest="no_bands", action="store_true", help="skip the reference-band / epoch legs")
     ap.add_argument("--quick", action="store_true", help="profiling aid: skip the e2e and cpu_baseline legs")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss and the updated weights as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the timed GPU step computed; it needs --impl ours")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
