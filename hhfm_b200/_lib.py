@@ -50,6 +50,9 @@ SIGNATURES = {
     "hhfm_pairrank_fwd_bwd_st": [vp, i64, i64, i32, i32, i32, i32, i32, i32, vp, i64, i64, vp, vp, vp, vp, vp, i32, vp,
                                  vp, vp, vp, i32, i32, i32, vp, vp],
     "hhfm_pairrank_bwd": [vp, i64, i64, i32, i32, i32, i32, i32, i32, vp, i64, i64, vp, vp, vp, i32, vp],
+    "hhfm_pool_groups_attach": [vp, i64, i64, i32, i64, vp, vp, vp, vp],
+    "hhfm_pool_groups_detach": [vp, i64],
+    "hhfm_pool_groups_tables": [vp, vp, vp, vp],
     "hhfm_scatter_add_rows": [vp, vp, i64, i64, vp, i64, vp],
     "hhfm_gather_rows": [vp, vp, i64, i64, i64, vp, i32, vp],
     "hhfm_touch_rows": [vp, i64, vp, i32, vp, vp, vp],

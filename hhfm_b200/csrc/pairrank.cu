@@ -5,6 +5,10 @@
 // Record (int32, `stride` ints, 16-byte aligned): [user, item+, ctx.., time.., neg.., pad].
 #include <stdlib.h>
 
+#include <algorithm>
+#include <mutex>
+#include <vector>
+
 #include "common.cuh"
 #include "opt_elem.cuh"
 #include "staged.cuh"
@@ -303,12 +307,34 @@ __global__ void __launch_bounds__(kBlock) pairrank_kernel(const PrArgs a) {
 // The hybrid feature is summed in record order, ((u + c0) + c1) + ..., where the generic kernel pools the group first,
 // u + (c0 + c1 + ...): the two differ in the last bit, both are within the 1e-5 parity bar.
 // (~3x fewer instructions per sample; see profiles/.)
+//
+// Pooled context groups (NS < NP, hhfm_pool_groups_attach): the NP pooled columns collapse into NS pooled rows.  Columns
+// of a group are replaced by one row of the group table S_g, indexed by the mixed-radix combination of their values
+// (pool_groups_presum_kernel sums the member rows into S_g before this kernel), and d_hyb goes to one row of G_g
+// (pool_groups_expand_kernel hands it back to the member rows afterwards).  An ungrouped column is a slot of its own that
+// reads V directly.  hyb = (u + slot_0) + slot_1 + ..., where a group slot already holds its members' sum.  A sample
+// whose member id lies outside the planned range pools and scatters that group's member rows one by one (same order as
+// the pre-sum, so the pooled value is the same).
 // ---------------------------------------------------------------------------------------------------
-template <int LPS, int NP, int NNEG>
-__global__ void __launch_bounds__(kBlock, 2) pairrank_sum_train_kernel(const PrArgs a) {
+constexpr int kPgMaxCols = 16;    // pooled columns (context + time) a plan describes
+constexpr int kPgMaxSlots = 4;    // pooled rows per sample after grouping
+
+struct PoolGroups {
+  int slot_of[kPgMaxCols];        // pooled column -> slot
+  int lo[kPgMaxCols];             // grouped column: first id of its range; ungrouped: 0
+  unsigned card[kPgMaxCols];      // grouped column: ids in the range; ungrouped: 0xffffffff (every id qualifies)
+  int mult[kPgMaxCols];           // grouped column: mixed-radix weight of its digit; ungrouped: 1
+  const float* T[kPgMaxSlots];    // slot table: S_g (group) or V (ungrouped column)
+  float* G[kPgMaxSlots];          // group gradient table G_g, nullptr for an ungrouped column
+};
+
+template <int LPS, int NP, int NNEG, int NS = NP>
+__global__ void __launch_bounds__(kBlock, 2) pairrank_sum_train_kernel(const PrArgs a, const PoolGroups pg) {
+  static_assert(NS <= NP, "grouping never adds pooled rows");
+  constexpr bool GROUPED = NS < NP;
   __shared__ float scratch[32];
-  constexpr int W = 2 + NP + NNEG;
-  constexpr int W4 = (W + 3) / 4;
+  constexpr int W = 2 + NS + NNEG;                     // gathered rows
+  constexpr int W4 = (2 + NP + NNEG + 3) / 4;          // int4 chunks of the record
   const int lane = threadIdx.x & 31, lg = lane % LPS, grp = lane / LPS;
   const int64_t warp_g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int64_t n_warps = (int64_t)gridDim.x * (blockDim.x >> 5);
@@ -340,16 +366,50 @@ __global__ void __launch_bounds__(kBlock, 2) pairrank_sum_train_kernel(const PrA
       idx[4 * i] = t.x; idx[4 * i + 1] = t.y; idx[4 * i + 2] = t.z; idx[4 * i + 3] = t.w;
     }
     float4 e[W];
+    int key[NS > 0 ? NS : 1];       // GROUPED: row of each slot's table
+    unsigned miss = 0u;             // GROUPED: bit s <=> a member id of slot s lies outside the planned range
+    if constexpr (!GROUPED) {
 #pragma unroll
-    for (int i = 0; i < W; i++) e[i] = __ldg(Vp + (size_t)idx[i] * LPS);
+      for (int i = 0; i < W; i++) e[i] = __ldg(Vp + (size_t)idx[i] * LPS);
+    } else {
+#pragma unroll
+      for (int q = 0; q < NS; q++) key[q] = 0;
+#pragma unroll
+      for (int c = 0; c < NP; c++) {              // selects, not a store through slot_of[c]: key stays in registers
+        const int d = idx[2 + c] - pg.lo[c], s = pg.slot_of[c], dm = d * pg.mult[c];
+        if ((unsigned)d >= pg.card[c]) miss |= 1u << s;
+#pragma unroll
+        for (int q = 0; q < NS; q++) key[q] += (s == q) ? dm : 0;
+      }
+      e[0] = __ldg(Vp + (size_t)idx[0] * LPS);
+      e[1] = __ldg(Vp + (size_t)idx[1] * LPS);
+#pragma unroll
+      for (int q = 0; q < NS; q++)
+        e[2 + q] = ((miss >> q) & 1u) ? f4_zero()
+                                       : __ldg(reinterpret_cast<const float4*>(pg.T[q]) + lg + (size_t)key[q] * LPS);
+#pragma unroll
+      for (int j = 0; j < NNEG; j++) e[2 + NS + j] = __ldg(Vp + (size_t)idx[2 + NP + j] * LPS);
+      if (miss) {                   // fallback: pool the members of the missed slots row by row, in record order
+        const int32_t* rec = a.idx + sc * a.stride + 2;
+        for (int c = 0; c < NP; c++) {
+          const int q = pg.slot_of[c];
+          if ((miss >> q) & 1u) {
+            const float4 v = __ldg(Vp + (size_t)__ldg(rec + c) * LPS);
+#pragma unroll
+            for (int qq = 0; qq < NS; qq++)
+              if (qq == q) e[2 + qq] = f4_add(e[2 + qq], v);
+          }
+        }
+      }
+    }
 
-    float4 hyb = e[0];                                   // user, then ctx.., time.. in record order
+    float4 hyb = e[0];                                   // user, then ctx.., time.. (or their slots) in record order
 #pragma unroll
-    for (int i = 0; i < NP; i++) hyb = f4_add(hyb, e[2 + i]);
+    for (int i = 0; i < NS; i++) hyb = f4_add(hyb, e[2 + i]);
     float p[1 + NNEG];
     p[0] = f4_dot(hyb, e[1]);
 #pragma unroll
-    for (int j = 0; j < NNEG; j++) p[1 + j] = f4_dot(hyb, e[2 + NP + j]);
+    for (int j = 0; j < NNEG; j++) p[1 + j] = f4_dot(hyb, e[2 + NS + j]);
 #pragma unroll
     for (int j = 0; j <= NNEG; j++) p[j] = group_sum<LPS>(p[j]);
 
@@ -379,24 +439,37 @@ __global__ void __launch_bounds__(kBlock, 2) pairrank_sum_train_kernel(const PrA
         scatter(id, tn);
       }
       scatter(idx[0], dh);
+      if constexpr (!GROUPED) {
 #pragma unroll
-      for (int i = 0; i < NP; i++) scatter(idx[2 + i], dh);
+        for (int i = 0; i < NP; i++) scatter(idx[2 + i], dh);
+      } else {
+#pragma unroll
+        for (int q = 0; q < NS; q++) {
+          if (pg.G[q] == nullptr) scatter(key[q], dh);                          // ungrouped column: key is the row id
+          else if (!((miss >> q) & 1u)) red_add_v4(pg.G[q] + (size_t)key[q] * (4 * LPS) + 4 * lg, dh);
+        }
+        if (miss) {
+          const int32_t* rec = a.idx + sc * a.stride + 2;
+          for (int c = 0; c < NP; c++)
+            if ((miss >> pg.slot_of[c]) & 1u) scatter(__ldg(rec + c), dh);
+        }
+      }
     }
   }
   const float bl = block_sum(loss_acc, scratch);
   write_partial(a.loss_partials, bl);
 }
 
-template <int LPS, int NP, int NNEG>
-static int launch_pr_fast(const PrArgs& a, cudaStream_t st) {
+template <int LPS, int NP, int NNEG, int NS = NP>
+static int launch_pr_fast(const PrArgs& a, cudaStream_t st, const PoolGroups& pg = PoolGroups{}) {
   static int occ = 0;
   if (occ == 0) {
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pairrank_sum_train_kernel<LPS, NP, NNEG>, kBlock, 0);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pairrank_sum_train_kernel<LPS, NP, NNEG, NS>, kBlock, 0);
     if (occ < 1) occ = 1;
   }
   constexpr int G = 32 / LPS;
   const int grid = grid_for(a.B, (kBlock / 32) * G, occ);
-  pairrank_sum_train_kernel<LPS, NP, NNEG><<<grid, kBlock, 0, st>>>(a);
+  pairrank_sum_train_kernel<LPS, NP, NNEG, NS><<<grid, kBlock, 0, st>>>(a, pg);
   return check_launch("pairrank_sum_train_kernel");
 }
 
@@ -425,6 +498,199 @@ static int dispatch_pr_fast(const PrArgs& a, cudaStream_t st, int* rc) {
     case 128: return dispatch_pr_fast_np<32>(a, st, rc);
     default: return 1;
   }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Pooled context groups (include/hhfm_sm100.h hhfm_pool_groups_attach).  A plan is registered under the table pointer V
+// and owns its group tables: S (pooled member rows) and G (group gradients, zero between calls), both [rows, K], the
+// groups one after another.  One call of the training pass with a matching plan runs
+//   pool_groups_presum_kernel  S_g[k] = V[lo_0 + d_0(k)] + V[lo_1 + d_1(k)] + ...   (members in record order)
+//   pairrank_sum_train_kernel<LPS, NP, NNEG, NS>
+//   pool_groups_expand_kernel  gV[lo_c + d] += sum of G_g[k] over the combinations k with digit d_c(k) == d, fixed order
+//   memset(G, 0)
+// Nothing else writes a member row of gV during the call (the planner keeps member rows out of the hot-row plan; fallback
+// samples reduce into it before the expansion starts, on the same stream), so the expansion adds with a plain
+// read-modify-write, and the ranges of grouped columns are disjoint, so no two CTAs of it share a row.
+// ---------------------------------------------------------------------------------------------------
+struct PgDesc {
+  int n_groups;
+  int n_mem[kPgMaxSlots];                   // member columns of group g, in record order
+  int mem_lo[kPgMaxSlots][kPgMaxCols];
+  int mem_card[kPgMaxSlots][kPgMaxCols];
+  int64_t row0[kPgMaxSlots + 1];            // first row of group g in S / G; row0[n_groups] = all rows
+  int64_t mrow0[kPgMaxSlots + 1];           // first member row of group g in the expansion grid
+};
+
+__global__ void __launch_bounds__(kBlock) pool_groups_presum_kernel(const float* __restrict__ V, int K, float* __restrict__ S,
+                                                                    const PgDesc d) {
+  const int kv = K >> 2;
+  const int n = (int)d.row0[d.n_groups] * kv;   // 32-bit index math: at most 2^24 combinations x 32 float4 columns
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int row = i / kv;
+    const int j = i - row * kv;
+    int g = 0;
+    while (g + 1 < d.n_groups && row >= d.row0[g + 1]) g++;
+    unsigned k = (unsigned)(row - d.row0[g]);
+    float4 acc = f4_zero();
+    for (int m = 0; m < d.n_mem[g]; m++) {
+      const unsigned c = (unsigned)d.mem_card[g][m], q = k / c;
+      const int digit = (int)(k - q * c);
+      k = q;
+      const float4 v = __ldg(reinterpret_cast<const float4*>(V + (size_t)(d.mem_lo[g][m] + digit) * K) + j);
+      acc = (m == 0) ? v : f4_add(acc, v);
+    }
+    reinterpret_cast<float4*>(S + (size_t)row * K)[j] = acc;
+  }
+}
+
+// One CTA per member row; thread (lane t % kv, chunk t / kv) sums the float4 column of every combination of its chunk,
+// then the chunks are added by a fixed shared-memory tree.
+constexpr int kPgExpandThreads = 1024;
+
+__global__ void __launch_bounds__(kPgExpandThreads) pool_groups_expand_kernel(const float* __restrict__ G, int K,
+                                                                              float* __restrict__ gV, const PgDesc d) {
+  __shared__ float4 part[kPgExpandThreads];
+  const int kv = K >> 2;
+  const int nchunk = kPgExpandThreads / kv;
+  const int j = threadIdx.x % kv, chunk = threadIdx.x / kv;
+  const int64_t r = blockIdx.x;
+  int g = 0;
+  while (g + 1 < d.n_groups && r >= d.mrow0[g + 1]) g++;
+  int rem = (int)(r - d.mrow0[g]);          // 32-bit index math: a plan has at most 2^24 combinations
+  int m = 0;
+  unsigned inner = 1;                       // mixed-radix weight of member m
+  while (rem >= d.mem_card[g][m]) { rem -= d.mem_card[g][m]; inner *= (unsigned)d.mem_card[g][m]; m++; }
+  const unsigned digit = (unsigned)rem;
+  const unsigned span = inner * (unsigned)d.mem_card[g][m];
+  const unsigned n = (unsigned)(d.row0[g + 1] - d.row0[g]) / (unsigned)d.mem_card[g][m];   // combinations holding this row
+  const float4* Gg = reinterpret_cast<const float4*>(G + (size_t)d.row0[g] * K) + j;
+  constexpr int U = 8;
+  float4 acc[U];
+#pragma unroll
+  for (int u = 0; u < U; u++) acc[u] = f4_zero();
+  unsigned t = chunk;
+  for (; t + (U - 1) * nchunk < n; t += U * nchunk) {
+    float4 v[U];
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+      const unsigned tt = t + u * nchunk, hi = tt / inner;
+      v[u] = __ldcg(Gg + (size_t)(tt - hi * inner + digit * inner + hi * span) * kv);
+    }
+#pragma unroll
+    for (int u = 0; u < U; u++) acc[u] = f4_add(acc[u], v[u]);
+  }
+  for (; t < n; t += nchunk) {
+    const unsigned hi = t / inner;
+    acc[0] = f4_add(acc[0], __ldcg(Gg + (size_t)(t - hi * inner + digit * inner + hi * span) * kv));
+  }
+#pragma unroll
+  for (int h = U / 2; h > 0; h >>= 1)
+#pragma unroll
+    for (int u = 0; u < h; u++) acc[u] = f4_add(acc[u], acc[u + h]);
+  part[threadIdx.x] = acc[0];
+  __syncthreads();
+  for (int h = nchunk / 2; h > 0; h >>= 1) {
+    if (chunk < h) part[threadIdx.x] = f4_add(part[threadIdx.x], part[threadIdx.x + h * kv]);
+    __syncthreads();
+  }
+  if (chunk == 0) {
+    int lo = d.mem_lo[g][m];
+    float4* dst = reinterpret_cast<float4*>(gV + (size_t)(lo + digit) * K) + j;
+    *dst = f4_add(*dst, part[j]);
+  }
+}
+
+struct PgPlan {
+  const float* V;
+  int64_t M;
+  int K, n_pool, stride, device;
+  int64_t handle;
+  int n_slots;
+  PoolGroups pg;                            // kernel view of the training pass
+  PgDesc desc;                              // pre-sum / expansion view
+  float* S;
+  float* G;
+};
+
+static std::mutex g_pg_mu;
+static std::vector<PgPlan*> g_pg_plans;
+static int64_t g_pg_next = 1;
+
+static void pg_free(PgPlan* p) {
+  cudaFree(p->S);
+  cudaFree(p->G);
+  delete p;
+}
+
+// HHFM_POOL_GROUPS=0 forces the ungrouped kernel (A/B measurements).
+static bool pool_groups_enabled() {
+  const char* e = getenv("HHFM_POOL_GROUPS");
+  return !(e && e[0] == '0');
+}
+
+template <int LPS, int NP>
+static int launch_pr_grouped_ns(const PrArgs& a, const PgPlan& p, cudaStream_t st, int* rc) {
+  switch (p.n_slots) {
+    case 1: *rc = launch_pr_fast<LPS, NP, 10, 1>(a, st, p.pg); return 0;
+    case 2: *rc = launch_pr_fast<LPS, NP, 10, 2>(a, st, p.pg); return 0;
+    case 3: if constexpr (NP > 3) { *rc = launch_pr_fast<LPS, NP, 10, 3>(a, st, p.pg); return 0; } else return 1;
+    case 4: if constexpr (NP > 4) { *rc = launch_pr_fast<LPS, NP, 10, 4>(a, st, p.pg); return 0; } else return 1;
+    default: return 1;
+  }
+}
+
+template <int LPS>
+static int launch_pr_grouped_np(const PrArgs& a, const PgPlan& p, cudaStream_t st, int* rc) {
+  switch (a.n_ctx + a.n_time) {
+    case 3: return launch_pr_grouped_ns<LPS, 3>(a, p, st, rc);
+    case 8: return launch_pr_grouped_ns<LPS, 8>(a, p, st, rc);
+    case 10: return launch_pr_grouped_ns<LPS, 10>(a, p, st, rc);
+    default: return 1;
+  }
+}
+
+// returns 1 if no plan applies (the caller then runs the ungrouped kernels)
+static int dispatch_pr_grouped(const PrArgs& a, int64_t M, cudaStream_t st, int* rc) {
+  if (!pool_groups_enabled()) return 1;
+  const bool all_sum = (a.n_ctx == 0 || a.pc == HHFM_POOL_SUM) && (a.n_time == 0 || a.pt == HHFM_POOL_SUM) &&
+                       ((a.n_ctx == 0 && a.n_time == 0) || a.pf == HHFM_POOL_SUM);
+  if (!all_sum || a.touch_stamp || a.pos_out || a.neg_out || a.st1.ref_count || a.n_neg != 10) return 1;
+  if (a.K != 32 && a.K != 64 && a.K != 128) return 1;
+  int dev = -1;
+  cudaGetDevice(&dev);
+  PgPlan* p = nullptr;
+  {
+    std::lock_guard<std::mutex> lk(g_pg_mu);
+    for (PgPlan* q : g_pg_plans)
+      if (q->V == a.V) { p = q; break; }
+  }
+  if (p == nullptr || p->M != M || p->K != a.K || p->n_pool != a.n_ctx + a.n_time || p->stride != a.stride || p->device != dev)
+    return 1;
+  const int kv = a.K / 4;
+  const int64_t rows = p->desc.row0[p->desc.n_groups];
+  const int pre_grid = (int)std::min<int64_t>((rows * kv + kBlock - 1) / kBlock, (int64_t)sm_count() * 8);
+  pool_groups_presum_kernel<<<pre_grid, kBlock, 0, st>>>(a.V, a.K, p->S, p->desc);
+  int r = check_launch("pool_groups_presum_kernel");
+  if (r != HHFM_OK) { *rc = r; return 0; }
+  int miss = 1;
+  switch (a.K) {
+    case 32: miss = launch_pr_grouped_np<8>(a, *p, st, &r); break;
+    case 64: miss = launch_pr_grouped_np<16>(a, *p, st, &r); break;
+    default: miss = launch_pr_grouped_np<32>(a, *p, st, &r); break;
+  }
+  if (miss) return 1;                       // the planned slot count has no instance: S is rebuilt next call anyway
+  if (r != HHFM_OK) { *rc = r; return 0; }
+  pool_groups_expand_kernel<<<(int)p->desc.mrow0[p->desc.n_groups], kPgExpandThreads, 0, st>>>(p->G, a.K, a.gV, p->desc);
+  r = check_launch("pool_groups_expand_kernel");
+  if (r != HHFM_OK) { *rc = r; return 0; }
+  const cudaError_t e = cudaMemsetAsync(p->G, 0, (size_t)rows * a.K * sizeof(float), st);
+  if (e != cudaSuccess) {
+    set_error("pool_groups: clearing G: %s", cudaGetErrorString(e));
+    *rc = HHFM_ERR_LAUNCH;
+    return 0;
+  }
+  *rc = HHFM_OK;
+  return 0;
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -797,9 +1063,127 @@ extern "C" int hhfm_pairrank_fwd_bwd_st(const int32_t* idx, int64_t B, int64_t s
   if (!deterministic && hhfm_fast_path_enabled()) {
     int frc = dispatch_pr_staged(a, M, (cudaStream_t)stream);
     if (frc != HHFM_ERR_UNSUPPORTED) return frc;
+    if (dispatch_pr_grouped(a, M, (cudaStream_t)stream, &frc) == 0) return frc;
     if (dispatch_pr_fast(a, (cudaStream_t)stream, &frc) == 0) return frc;
   }
   return dispatch_pr<PR_TRAIN>(a, deterministic, (cudaStream_t)stream);
+}
+
+extern "C" int hhfm_pool_groups_attach(const float* V, int64_t M, int64_t K, int32_t n_pool, int64_t stride,
+                                       const int32_t* col_group, const int32_t* col_lo, const int32_t* col_card,
+                                       int64_t* handle) {
+  HHFM_REQUIRE(V && col_group && col_lo && col_card && handle, "pool_groups_attach: NULL argument");
+  HHFM_REQUIRE(K == 32 || K == 64 || K == 128, "pool_groups_attach: K=%lld unsupported (32, 64, 128)", (long long)K);
+  HHFM_REQUIRE(n_pool == 3 || n_pool == 8 || n_pool == 10, "pool_groups_attach: n_pool=%d unsupported (3, 8, 10)", n_pool);
+  HHFM_REQUIRE(M > 0 && stride >= 2 + n_pool && stride % 4 == 0, "pool_groups_attach: bad sizes");
+  PgPlan* p = new PgPlan{};
+  p->V = V; p->M = M; p->K = (int)K; p->n_pool = n_pool; p->stride = (int)stride;
+  cudaGetDevice(&p->device);
+  int group_slot[kPgMaxCols];
+  int n_groups = 0, n_slots = 0;
+  for (int c = 0; c < kPgMaxCols; c++) group_slot[c] = -1;
+  PgDesc& d = p->desc;
+  int grp_of_slot[kPgMaxSlots];
+  bool ok = true;
+  for (int c = 0; c < n_pool && ok; c++) {
+    const int gid = col_group[c];
+    if (gid < 0) {
+      if (n_slots == kPgMaxSlots) { ok = false; break; }
+      p->pg.slot_of[c] = n_slots; p->pg.lo[c] = 0; p->pg.card[c] = 0xffffffffu; p->pg.mult[c] = 1;
+      p->pg.T[n_slots] = V; p->pg.G[n_slots] = nullptr;
+      n_slots++;
+      continue;
+    }
+    if (gid >= n_pool || col_card[c] < 1 || col_lo[c] < 0 || (int64_t)col_lo[c] + col_card[c] > M) { ok = false; break; }
+    if (group_slot[gid] < 0) {
+      if (n_slots == kPgMaxSlots) { ok = false; break; }
+      group_slot[gid] = n_slots;
+      grp_of_slot[n_slots] = n_groups;
+      d.n_mem[n_groups] = 0;
+      n_groups++;
+      n_slots++;
+    }
+    const int s = group_slot[gid], g = grp_of_slot[s];
+    p->pg.slot_of[c] = s; p->pg.lo[c] = col_lo[c]; p->pg.card[c] = (unsigned)col_card[c];
+    d.mem_lo[g][d.n_mem[g]] = col_lo[c];
+    d.mem_card[g][d.n_mem[g]] = col_card[c];
+    d.n_mem[g]++;
+  }
+  // mixed-radix weights (members in record order), table rows, member rows
+  d.n_groups = n_groups;
+  d.row0[0] = 0; d.mrow0[0] = 0;
+  for (int g = 0; g < n_groups && ok; g++) {
+    int64_t P = 1, mr = 0;
+    for (int m = 0; m < d.n_mem[g]; m++) { P *= d.mem_card[g][m]; mr += d.mem_card[g][m]; if (P > (1 << 24)) ok = false; }
+    d.row0[g + 1] = d.row0[g] + P;
+    d.mrow0[g + 1] = d.mrow0[g] + mr;
+  }
+  for (int c = 0; c < n_pool && ok; c++) {
+    if (col_group[c] < 0) continue;
+    const int s = p->pg.slot_of[c];
+    int mult = 1;
+    for (int c2 = 0; c2 < c; c2++)
+      if (col_group[c2] >= 0 && p->pg.slot_of[c2] == s) mult *= col_card[c2];
+    p->pg.mult[c] = mult;
+    for (int c2 = c + 1; c2 < n_pool; c2++)          // member rows of different columns must not overlap
+      if (col_group[c2] >= 0 && col_lo[c2] < col_lo[c] + col_card[c] && col_lo[c] < col_lo[c2] + col_card[c2]) ok = false;
+  }
+  const int max_slots = n_pool == 3 ? 2 : kPgMaxSlots;   // compiled instances: NS < NP, NS <= 4
+  if (!ok || n_groups == 0 || n_slots > max_slots || d.row0[n_groups] > (1 << 24)) {
+    delete p;
+    set_error("pool_groups_attach: the plan is not supported (at most %d pooled rows, at least one group, group ranges "
+              "inside [0, M) and disjoint, at most 2^24 combinations)", max_slots);
+    return HHFM_ERR_BAD_ARG;
+  }
+  p->n_slots = n_slots;
+  const size_t bytes = (size_t)d.row0[n_groups] * K * sizeof(float);
+  cudaError_t e = cudaMalloc(&p->S, bytes);
+  if (e == cudaSuccess) e = cudaMalloc(&p->G, bytes);
+  if (e == cudaSuccess) e = cudaMemset(p->G, 0, bytes);
+  if (e != cudaSuccess) {
+    pg_free(p);
+    set_error("pool_groups_attach: %s", cudaGetErrorString(e));
+    return HHFM_ERR_LAUNCH;
+  }
+  for (int s = 0; s < n_slots; s++)
+    if (p->pg.T[s] == nullptr) {                   // group slot
+      p->pg.T[s] = p->S + (size_t)d.row0[grp_of_slot[s]] * K;
+      p->pg.G[s] = p->G + (size_t)d.row0[grp_of_slot[s]] * K;
+    }
+  std::lock_guard<std::mutex> lk(g_pg_mu);
+  for (size_t i = 0; i < g_pg_plans.size(); i++)
+    if (g_pg_plans[i]->V == V) {                   // a new plan for the same table replaces the old one
+      pg_free(g_pg_plans[i]);
+      g_pg_plans.erase(g_pg_plans.begin() + i);
+      break;
+    }
+  p->handle = g_pg_next++;
+  g_pg_plans.push_back(p);
+  *handle = p->handle;
+  return HHFM_OK;
+}
+
+extern "C" int hhfm_pool_groups_detach(const float* V, int64_t handle) {
+  std::lock_guard<std::mutex> lk(g_pg_mu);
+  for (size_t i = 0; i < g_pg_plans.size(); i++)
+    if (g_pg_plans[i]->V == V && g_pg_plans[i]->handle == handle) {
+      pg_free(g_pg_plans[i]);
+      g_pg_plans.erase(g_pg_plans.begin() + i);
+      break;
+    }
+  return HHFM_OK;
+}
+
+extern "C" int hhfm_pool_groups_tables(const float* V, float** S, float** G, int64_t* rows) {
+  HHFM_REQUIRE(S && G && rows, "pool_groups_tables: NULL argument");
+  std::lock_guard<std::mutex> lk(g_pg_mu);
+  for (PgPlan* p : g_pg_plans)
+    if (p->V == V) {
+      *S = p->S; *G = p->G; *rows = p->desc.row0[p->desc.n_groups];
+      return HHFM_OK;
+    }
+  set_error("pool_groups_tables: no plan is attached to this table");
+  return HHFM_ERR_BAD_ARG;
 }
 
 extern "C" int hhfm_pairrank_bwd(const int32_t* idx, int64_t B, int64_t stride, int32_t n_ctx, int32_t n_time,

@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
+import weakref
 
 import numpy as np
 import torch
@@ -366,12 +367,15 @@ class HotRows:
         self.ghot_bias = torch.zeros(self.n_rep, self.n_hot, dtype=torch.float32, device=device) if with_bias else None
 
     @classmethod
-    def from_batch(cls, idx_dev, M, K, device, with_bias=False):
+    def from_batch(cls, idx_dev, M, K, device, with_bias=False, exclude=None):
         """Pick the hot rows from the id histogram of one packed batch (one-time plumbing, not on the hot path):
-        rows hit at least MIN_COUNT times, the MAX_HOT most frequent of them.  Returns None if there are none."""
+        rows hit at least MIN_COUNT times, the MAX_HOT most frequent of them, never a row of `exclude` (the member rows
+        of pooled context groups, which the scatter kernel does not reduce into).  Returns None if there are none."""
         flat = idx_dev.reshape(-1)
         flat = flat[flat >= 0].long()
         counts = torch.bincount(flat, minlength=M)
+        if exclude is not None:
+            counts[exclude.to(counts.device)] = 0
         hot = torch.nonzero(counts >= cls.MIN_COUNT).reshape(-1)
         if hot.numel() == 0:
             return None
@@ -391,6 +395,122 @@ class HotRows:
 
 NO_HOT = (None, None, 0, 0)
 NO_HOT_BIAS = (None, None, None, 0, 0)
+
+
+# --------------------------------------------------------------------------------------------------
+# K3: pooled context groups (include/hhfm_sm100.h hhfm_pool_groups_attach)
+# --------------------------------------------------------------------------------------------------
+POOL_GROUP_CAP = 1 << 15          # combinations of one group
+POOL_GROUP_TOTAL_CAP = 1 << 16    # combinations of all groups: 2^16 rows x K = 128 x 4 B = 32 MB per table, L2-resident
+POOL_GROUP_MAX_SLOTS = 4          # pooled rows per sample after grouping that the kernels are compiled for
+
+
+def plan_pool_groups(lo, card, cap=POOL_GROUP_CAP, total_cap=POOL_GROUP_TOTAL_CAP, max_slots=POOL_GROUP_MAX_SLOTS):
+    """Group assignment of the pooled columns with id ranges [lo[c], lo[c] + card[c]) (card[c] < 1: not groupable).
+
+    Columns are packed smallest first, each onto the open group while its cardinality product stays <= cap and the
+    combinations of all groups <= total_cap, otherwise the group is closed and a new one opened.  Columns whose range
+    overlaps another groupable column's are not grouped (their member rows must be distinct), a group of one column is
+    dissolved (it would remove nothing), and if the pooled rows per sample after grouping would exceed max_slots or not
+    drop, nothing is grouped.  Returns a list: group number per column, -1 = ungrouped."""
+    n = len(card)
+    ok = [card[c] >= 1 and lo[c] >= 0 for c in range(n)]
+    for a in range(n):
+        for b in range(a + 1, n):
+            if ok[a] and ok[b] and lo[a] < lo[b] + card[b] and lo[b] < lo[a] + card[a]:
+                ok[a] = ok[b] = False
+    groups, cur, prod, total = [], [], 1, 0
+    for c in sorted((c for c in range(n) if ok[c]), key=lambda c: (card[c], c)):
+        if cur and prod * card[c] <= cap and total + prod * card[c] <= total_cap:
+            cur.append(c)
+            prod *= card[c]
+            continue
+        if len(cur) >= 2:
+            groups.append(cur)
+            total += prod
+        cur, prod = ([c], card[c]) if (card[c] <= cap and total + card[c] <= total_cap) else ([], 1)
+    if len(cur) >= 2:
+        groups.append(cur)
+    out = [-1] * n
+    for g, cols in enumerate(groups):
+        for c in cols:
+            out[c] = g
+    n_slots = len(groups) + out.count(-1)
+    if not groups or n_slots > max_slots or n_slots >= n:
+        return [-1] * n
+    return out
+
+
+def pool_group_index(ids, lo, card, members):
+    """Mixed-radix combination index of one group for rows of pooled ids [B, n_pool] (numpy): first member least
+    significant, members in record order.  Returns (index [B], in_range [B]); out-of-range rows are the fallback samples."""
+    ids = np.asarray(ids, dtype=np.int64)
+    k = np.zeros(ids.shape[0], dtype=np.int64)
+    ok = np.ones(ids.shape[0], dtype=bool)
+    mult = 1
+    for c in sorted(members):
+        d = ids[:, c] - lo[c]
+        ok &= (d >= 0) & (d < card[c])
+        k += d * mult
+        mult *= card[c]
+    return k, ok
+
+
+class PoolGroups:
+    """Pooled context groups of one table (hhfm_pool_groups_attach), planned from the id ranges of one packed batch.
+    The library owns the group tables; the plan is detached when this object goes away."""
+
+    def __init__(self, V, n_pool, stride, lo, card, groups):
+        self.V = V
+        self.groups = list(groups)
+        self.lo, self.card = list(lo), list(card)
+        M, K = V.shape
+        arr = lambda xs: np.ascontiguousarray(np.asarray(xs, dtype=np.int32))
+        self._g, self._lo, self._card = arr(groups), arr(lo), arr(card)
+        h = C.c_int64(0)
+        _lib.call("hhfm_pool_groups_attach", ptr(V), M, K, n_pool, stride, ptr(self._g), ptr(self._lo), ptr(self._card),
+                  C.byref(h))
+        self.handle = h.value
+        self._fin = weakref.finalize(self, PoolGroups._detach, V.data_ptr(), self.handle)
+        self._fin.atexit = False
+
+    @staticmethod
+    def _detach(v_ptr, handle):
+        _lib.load().hhfm_pool_groups_detach(C.c_void_p(v_ptr), handle)
+
+    def member_rows(self):
+        """Table rows covered by a group (int64 numpy)."""
+        return np.concatenate([np.arange(self.lo[c], self.lo[c] + self.card[c]) for c in range(len(self.groups))
+                               if self.groups[c] >= 0]).astype(np.int64)
+
+    def tables(self):
+        """(S, G): copies of the library's group tables, [rows, K] float32 on the table's device (tests, inspection)."""
+        S, G, rows = C.c_void_p(), C.c_void_p(), C.c_int64()
+        _lib.call("hhfm_pool_groups_tables", ptr(self.V), C.byref(S), C.byref(G), C.byref(rows))
+        shape = (rows.value, self.V.shape[1])
+
+        class _View:           # __cuda_array_interface__ of a library-owned buffer
+            def __init__(self, p):
+                self.__cuda_array_interface__ = {"shape": shape, "typestr": "<f4", "data": (p, False), "version": 2}
+
+        with torch.cuda.device(self.V.device):
+            return tuple(torch.as_tensor(_View(p.value), device=self.V.device).clone() for p in (S, G))
+
+    @classmethod
+    def from_batch(cls, V, idx_dev, n_pool):
+        """Plan from the pooled columns [2, 2 + n_pool) of one packed batch: each column's range is [min, max].  Returns
+        None when HHFM_POOL_GROUPS=0, the configuration is not covered, or no group forms."""
+        if os.environ.get("HHFM_POOL_GROUPS") == "0" or n_pool not in (3, 8, 10) or V.shape[1] not in (32, 64, 128):
+            return None
+        cols = idx_dev[:, 2:2 + n_pool]
+        lo = cols.min(0).values.cpu().numpy().astype(np.int64)
+        hi = cols.max(0).values.cpu().numpy().astype(np.int64)
+        card = [int(h - l + 1) if l >= 0 else 0 for l, h in zip(lo, hi)]
+        groups = plan_pool_groups([int(x) for x in lo], card)
+        if all(g < 0 for g in groups):
+            return None
+        return cls(V, n_pool, idx_dev.shape[1], [int(x) if g >= 0 else 0 for x, g in zip(lo, groups)],
+                   [c if g >= 0 else 0 for c, g in zip(card, groups)], groups)
 
 
 # --------------------------------------------------------------------------------------------------

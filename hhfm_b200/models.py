@@ -19,8 +19,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from .engine import (NO_HOT, NO_HOT_BIAS, POOL_SUM, QUERY_FM, QUERY_HHFM, QUERY_USER, HotRows, Optimizer, RecordUploader,
-                     SingleTouchPlan, Staging, TopN, TouchTracker, cur_stream, pack_records, ptr, require_cuda)
+from .engine import (NO_HOT, NO_HOT_BIAS, POOL_SUM, QUERY_FM, QUERY_HHFM, QUERY_USER, HotRows, Optimizer, PoolGroups,
+                     RecordUploader, SingleTouchPlan, Staging, TopN, TouchTracker, cur_stream, pack_records, ptr, require_cuda)
 
 
 class PendingLoss:
@@ -217,13 +217,19 @@ class _Base:
         """Hot-row plan for the two-level scatter (engine.HotRows), built once from the first batch."""
         if not self._hot_planned:
             self._hot_planned = True
+            groups = self._pool_groups_plan(idx_dev)
             if self.hot_rows is None or self.deterministic:
                 self._hot = None
             elif isinstance(self.hot_rows, str):
-                self._hot = HotRows.from_batch(idx_dev, self._M, self._K, self.device, with_bias)
+                exclude = torch.from_numpy(groups.member_rows()) if groups is not None else None
+                self._hot = HotRows.from_batch(idx_dev, self._M, self._K, self.device, with_bias, exclude)
             else:
                 self._hot = HotRows(self.hot_rows, self._M, self._K, self.device, with_bias)
         return self._hot
+
+    def _pool_groups_plan(self, idx_dev):
+        """Pooled context groups of the table (engine.PoolGroups), planned with the hot rows; None where not applicable."""
+        return None
 
     # ---- data parallel (SURVEY.md 8e): batch rows sharded across ranks, one all-reduce of the arena ----
     def enable_data_parallel(self, group=None, fused="auto", sparse="auto", p2p=None):
@@ -854,6 +860,18 @@ class OUR(_PairRank):
         # feature_bias exists in the reference graph (OurModel7.py:213-214) but receives no gradient
         self._with_bias_grad = False
         self._gb = None
+
+    def _pool_groups_plan(self, idx_dev):
+        """Sum pooling everywhere (the reference default): low-cardinality context / time columns are pre-pooled into
+        group tables (engine.PoolGroups), so each positive gathers and reduces one row per group instead of one per
+        column.  Not for the deterministic kernel or tables large enough for the staged kernel."""
+        n_pool = self._n_ctx + self._n_time
+        self._pool_groups = None
+        if (self.deterministic or n_pool == 0 or any(p != POOL_SUM for p in self.pools) or self.device.type != "cuda"
+                or self._M * self._K * 4 >= (96 << 20)):
+            return None
+        self._pool_groups = PoolGroups.from_batch(self.weights["feature_embeddings"], idx_dev, n_pool)
+        return self._pool_groups
 
     def _parts(self, X, F1, F2, Y=None):
         parts = [np.asarray(X)[:, :2]]

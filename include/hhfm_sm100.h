@@ -308,6 +308,31 @@ int hhfm_pairrank_fwd_bwd_st(const int32_t* idx, int64_t B, int64_t stride, int3
                           const int32_t* hot_slot, float* ghot, int32_t n_rep, int32_t n_hot,
                           int32_t deterministic, const hhfm_single_touch* plan, hhfm_stream_t stream);
 
+/* Pooled context groups of the sum-pooling training pass.  With every pool mode HHFM_POOL_SUM only the sum of the pooled
+ * rows enters the model, so pooled columns with small vocabularies can be pre-pooled: the columns of a group (id ranges
+ * [col_lo[c], col_lo[c] + col_card[c]), disjoint, inside [0, M)) are replaced by one row of the group table
+ *   S_g[k] = sum over the members c, in record order, of V[col_lo[c] + d_c(k)],
+ * k = sum_c d_c * prod_{c' before c} col_card[c'] (mixed radix, first member least significant), and the gradient of that
+ * row is handed back to the member rows after the pass.  Per positive this gathers and reduces one row per group instead
+ * of one per column.
+ *   hhfm_pool_groups_attach registers the plan under the table pointer V (col_group[c]: group number of pooled column c,
+ *     c < n_pool = n_ctx + n_time, or -1 = ungrouped) and allocates S and G ([rows, K] each, G zero).  A later plan for
+ *     the same V replaces it.  *handle identifies the plan for detach.
+ *   hhfm_pairrank_fwd_bwd / _st then run, on the caller's stream: the pre-sum of S, the grouped training kernel, the
+ *     expansion of G into gV (fixed summation order) and the clearing of G.  The plan is used when M, K, n_ctx + n_time,
+ *     stride and the current device match it, every pool mode is HHFM_POOL_SUM, n_neg == 10, K in {32, 64, 128},
+ *     deterministic == 0 and no touched-row tracking, positive / negative outputs or single-touch plan is requested,
+ *     and the large-table (staged) kernel does not run; otherwise the call is the ungrouped one.  A sample whose member
+ *     id lies outside the planned range pools and scatters that group's member rows individually (hot-row plan / gV).
+ *     Member rows should not be hot rows: nothing but those fallback samples should reduce into them during the pass.
+ *     HHFM_POOL_GROUPS=0 ignores every plan.
+ *   hhfm_pool_groups_detach removes the plan (no-op unless V and handle match).
+ *   hhfm_pool_groups_tables returns the plan's S, G and their row count. */
+int hhfm_pool_groups_attach(const float* V, int64_t M, int64_t K, int32_t n_pool, int64_t stride, const int32_t* col_group,
+                            const int32_t* col_lo, const int32_t* col_card, int64_t* handle);
+int hhfm_pool_groups_detach(const float* V, int64_t handle);
+int hhfm_pool_groups_tables(const float* V, float** S, float** G, int64_t* rows);
+
 /* Backward only, for torch.autograd: dpos [B], dneg [B,n_neg] (nullable) given by the caller. */
 int hhfm_pairrank_bwd(const int32_t* idx, int64_t B, int64_t stride, int32_t n_ctx, int32_t n_time, int32_t n_neg,
                       int32_t pool_ctx, int32_t pool_time, int32_t pool_stack, const float* V, int64_t M, int64_t K,
