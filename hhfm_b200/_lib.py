@@ -32,6 +32,9 @@ SIGNATURES = {
     "hhfm_afm_fwd": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, vp, vp],
     "hhfm_afm_fwd_bwd_sqloss": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                 vp, vp, i32, vp, vp, vp, vp, vp, i32, i32, vp],
+    "hhfm_afm_fwd_bwd_sqloss_dropout": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp,
+                                        vp, vp, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, f32, f32, C.c_uint64, i64, vp],
+    "hhfm_afm_fwd_attn": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, i32, vp, vp],
     "hhfm_dfm_fwd": [vp, i64, i64, vp, vp, i64, i64, vp, i32, vp, vp, vp, vp],
     "hhfm_dfm_fwd_bwd_sqloss": [vp, i64, i64, vp, vp, i64, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32,
                                 vp],

@@ -19,18 +19,21 @@
 
 namespace hhfm {
 
-__host__ __device__ inline size_t afm_per_warp_floats(int F, int K, int A, int P) {
-  return 2 * (size_t)F * K + (size_t)P * A + (size_t)((2 * P + 3) / 4 * 4);
+// drop: the DROP instantiations keep the sample's attention-dropout factors m_p in one more row of P floats
+__host__ __device__ inline size_t afm_per_warp_floats(int F, int K, int A, int P, bool drop = false) {
+  return 2 * (size_t)F * K + (size_t)P * A + (size_t)((2 * P + 3) / 4 * 4) + (drop ? (size_t)((P + 3) / 4 * 4) : 0);
 }
 
-__host__ __device__ inline size_t afm_smem_floats(int NW, int F, int K, int A, int P) {
-  // sW[K][A+1] + sp[A] + sb[A] + swp[K] + NW * (sE[F][K] + sDE[F][K] + sZ[P][A] + sS[P] + sD[P] (padded)) + valid flags
-  return (size_t)K * (A + 1) + 2 * (size_t)A + K + (size_t)NW * afm_per_warp_floats(F, K, A, P) + 32;
+__host__ __device__ inline size_t afm_smem_floats(int NW, int F, int K, int A, int P, bool drop = false) {
+  // sW[K][A+1] + sp[A] + sb[A] + swp[K] + NW * (sE[F][K] + sDE[F][K] + sZ[P][A] + sS[P] + sD[P] (padded) [+ sM[P]]) + valid flags
+  return (size_t)K * (A + 1) + 2 * (size_t)A + K + (size_t)NW * afm_per_warp_floats(F, K, A, P, drop) + 32;
 }
 
 constexpr int PB = 8;       // pairs per register-blocked sweep of the two matrix products
 
-template <int TK, int TA, int NW, bool TRAIN>
+// DROP: training dropout (AFM.py:126,134).  a_p m_p replaces a_p in the pooled sum, w~ = prediction_W * n replaces
+// prediction_W, d prediction_W += g n afm, and the softmax backward becomes ds_p = a_p (m_p d a_p - sum_q a_q m_q d a_q).
+template <int TK, int TA, int NW, bool TRAIN, bool DROP = false>
 __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
   extern __shared__ __align__(16) float smem[];
   __shared__ float scratch[32];
@@ -41,7 +44,7 @@ __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
   float* sb = sp + A;                     // [A]
   float* swp = sb + A;                    // [K]
   float* warp_base = swp + K;
-  const size_t per_warp = afm_per_warp_floats(F, K, A, P);
+  const size_t per_warp = afm_per_warp_floats(F, K, A, P, DROP);
   int* sValid = reinterpret_cast<int*>(warp_base + (size_t)NW * per_warp);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* sE = warp_base + warp * per_warp;   // [F][K]
@@ -49,6 +52,8 @@ __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
   float* sZ = sDE + (size_t)F * K;           // [P][A]  Z, later dZ
   float* sS = sZ + (size_t)P * A;            // [P]     s, later a
   float* sD = sS + P;                        // [P]     d a, later d s
+  float* sM = sS + (2 * P + 3) / 4 * 4;      // [P]     m_p (DROP)
+  const uint64_t vseed = DROP ? splitmix64(a.drop_seed) : 0;
 
   for (int i = threadIdx.x; i < K * A; i += blockDim.x) sW[(i / A) * AS + (i % A)] = __ldg(a.W + i);
   for (int i = threadIdx.x; i < A; i += blockDim.x) { sp[i] = __ldg(a.pvec + i); sb[i] = __ldg(a.batt + i); }
@@ -158,14 +163,20 @@ __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
       for (int p = lane; p < P; p += 32) { const float e = expf(sS[p] - mx); sS[p] = e; den += e; }
       den = warp_sum(den);
       __syncwarp();
-      for (int p = lane; p < P; p += 32) sS[p] = sS[p] / den;
+      for (int p = lane; p < P; p += 32) {
+        sS[p] = sS[p] / den;
+        if (DROP) sM[p] = afm_mask_att(a, s, p) / a.keep_att;
+      }
       __syncwarp();
+      float nv[TK];                                               // n_k of the lane's columns (DROP)
+#pragma unroll
+      for (int t = 0; t < TK; t++) nv[t] = DROP ? afm_mask_vec(a, vseed, s, lane + 32 * t) / a.keep_vec : 1.f;
       // ---- afm = sum_p a_p P_p (lanes over k), out ----
       float afm[TK];
 #pragma unroll
       for (int t = 0; t < TK; t++) afm[t] = 0.f;
       for (int p = 0; p < P; p++) {
-        const float ap = sS[p];
+        const float ap = DROP ? sS[p] * sM[p] : sS[p];
         const float* xi = sE + sPairI[p] * K; const float* xj = sE + sPairJ[p] * K;
 #pragma unroll
         for (int t = 0; t < TK; t++) {
@@ -175,7 +186,7 @@ __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
       }
       float part = 0.f;
 #pragma unroll
-      for (int t = 0; t < TK; t++) { const int k = lane + 32 * t; if (k < K) part = fmaf(afm[t], swp[k], part); }
+      for (int t = 0; t < TK; t++) { const int k = lane + 32 * t; if (k < K) part = fmaf(afm[t], DROP ? swp[k] * nv[t] : swp[k], part); }
       const float bil = warp_sum(part);
       const float out = (bil + bsum) + b0;                       // AFM.py:142 add_n
       if (a.out && lane == 0) a.out[s] = out;
@@ -185,13 +196,13 @@ __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
         const float diff = y - out;
         const float g = -diff;
         if (lane == 0) { loss_acc += 0.5f * diff * diff; g0_acc += g; }
-        // d afm = g w_pred ; d w_pred += g afm
+        // d afm = g w_pred ; d w_pred += g afm   (DROP: w~ = w_pred n, d w_pred += g n afm)
         float dafm[TK];
 #pragma unroll
         for (int t = 0; t < TK; t++) {
           const int k = lane + 32 * t;
-          dafm[t] = (k < K) ? g * swp[k] : 0.f;
-          gwp_acc[t] = fmaf(g, afm[t], gwp_acc[t]);
+          dafm[t] = (k < K) ? g * (DROP ? swp[k] * nv[t] : swp[k]) : 0.f;
+          gwp_acc[t] = fmaf(g, DROP ? afm[t] * nv[t] : afm[t], gwp_acc[t]);
         }
         // d a_p = P_p . d afm ; softmax backward
         float dot = 0.f;
@@ -202,10 +213,10 @@ __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
           for (int t = 0; t < TK; t++) { const int k = lane + 32 * t; if (k < K) v = fmaf(xi[k] * xj[k], dafm[t], v); }
           v = warp_sum(v);
           if (lane == 0) sD[p] = v;
-          dot = fmaf(sS[p], v, dot);
+          dot = fmaf(DROP ? sS[p] * sM[p] : sS[p], v, dot);
         }
         __syncwarp();
-        for (int p = lane; p < P; p += 32) sD[p] = sS[p] * (sD[p] - dot);       // d s_p
+        for (int p = lane; p < P; p += 32) sD[p] = sS[p] * ((DROP ? sM[p] * sD[p] : sD[p]) - dot);       // d s_p
         __syncwarp();
         // d Z_p = d s_p p (Z_p > 0) (overwrites Z) ; d p += d s_p relu(Z_p) ; d b += d Z_p
         for (int p = 0; p < P; p++) {
@@ -230,7 +241,7 @@ __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
           float dp[PB][TK];
 #pragma unroll
           for (int q = 0; q < PB; q++) {
-            const float ap = (p0 + q < P) ? sS[p0 + q] : 0.f;
+            const float ap = (p0 + q < P) ? (DROP ? sS[p0 + q] * sM[p0 + q] : sS[p0 + q]) : 0.f;
 #pragma unroll
             for (int t = 0; t < TK; t++) dp[q][t] = ap * dafm[t];
           }
@@ -356,11 +367,11 @@ __global__ void __launch_bounds__(NW * 32) afm_kernel(const AfmArgs a) {
 // fit next to W and W^T.
 // ---------------------------------------------------------------------------------------------------------------
 __host__ __device__ inline int afm2_p4(int P) { return (P + 3) / 4 * 4; }
-__host__ __device__ inline size_t afm2_per_warp_floats(int F, int KD, int P) {
-  return (size_t)F * KD + KD + 2 * (size_t)afm2_p4(P) + (size_t)(F + P) * (KD + 4);   // every term a multiple of 4
+__host__ __device__ inline size_t afm2_per_warp_floats(int F, int KD, int P, bool drop = false) {
+  return (size_t)F * KD + KD + (drop ? 3 : 2) * (size_t)afm2_p4(P) + (size_t)(F + P) * (KD + 4);   // every term a multiple of 4
 }
-__host__ __device__ inline size_t afm2_smem_floats(int NW, int F, int KD, int P) {
-  return 2 * (size_t)KD * KD + 3 * (size_t)KD + (size_t)NW * afm2_per_warp_floats(F, KD, P) + 32;
+__host__ __device__ inline size_t afm2_smem_floats(int NW, int F, int KD, int P, bool drop = false) {
+  return 2 * (size_t)KD * KD + 3 * (size_t)KD + (size_t)NW * afm2_per_warp_floats(F, KD, P, drop) + 32;
 }
 
 // acc[r][c] += sum_k x_rk * Wc[k*KD + c], c in [0, NC), r in [0, NR), with x_rk = u_r[k] * v_r[k] (PROD) or u_r[k].
@@ -431,9 +442,11 @@ __device__ __forceinline__ void afm2_logits(const float* sE, const unsigned char
   }
 }
 
-// dP_p = a_p d_afm + dZ_p W^T, written over dZ_p (both lanes of a row finish reading it before either writes)
-template <int KD, int NR>
-__device__ __forceinline__ void afm2_dpairs(float* sZ, const float* sWT, const float* sdafm, const float* sS, int P, int lane) {
+// dP_p = a_p d_afm + dZ_p W^T, written over dZ_p (both lanes of a row finish reading it before either writes);
+// DROP: a_p m_p d_afm, m_p from sM
+template <int KD, int NR, bool DROP = false>
+__device__ __forceinline__ void afm2_dpairs(float* sZ, const float* sWT, const float* sdafm, const float* sS, const float* sM, int P,
+                                            int lane) {
   constexpr int NC = KD / 2, RS = KD + 4;
   const int c0 = (lane >> 4) * NC, l = lane & 15;
   float acc[NR][NC];
@@ -441,7 +454,7 @@ __device__ __forceinline__ void afm2_dpairs(float* sZ, const float* sWT, const f
 #pragma unroll
   for (int r = 0; r < NR; r++) {
     const int p = l + 16 * r;
-    const float ap = p < P ? sS[p] : 0.f;
+    const float ap = p < P ? (DROP ? sS[p] * sM[p] : sS[p]) : 0.f;
     u[r] = sZ + (p < P ? p : 0) * RS;
 #pragma unroll
     for (int c = 0; c < NC; c++) acc[r][c] = ap * sdafm[c0 + c];
@@ -459,7 +472,8 @@ __device__ __forceinline__ void afm2_dpairs(float* sZ, const float* sWT, const f
   }
 }
 
-template <int KD, int NW, int NR, bool TRAIN>
+// DROP: training dropout, as in afm_kernel
+template <int KD, int NW, int NR, bool TRAIN, bool DROP = false>
 __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
   extern __shared__ __align__(16) float smem[];
   __shared__ float scratch[32];
@@ -476,16 +490,18 @@ __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
   float* sb = sp + KD;                       // [KD]
   float* swp = sb + KD;                      // [KD]
   float* warp_base = swp + KD;
-  const size_t per_warp = afm2_per_warp_floats(F, KD, P);
+  const size_t per_warp = afm2_per_warp_floats(F, KD, P, DROP);
   int* sValid = reinterpret_cast<int*>(warp_base + (size_t)NW * per_warp);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* sDE = warp_base + warp * per_warp;  // [F][KD]
   float* sdafm = sDE + (size_t)F * KD;       // [KD]
   float* sS = sdafm + KD;                    // [P] s, later a
   float* sD = sS + P4;                       // [P] d a, later d s
-  float* sE = sD + P4;                       // [F][RS]
+  float* sM = sD + P4;                       // [P] m_p (DROP only)
+  float* sE = sM + (DROP ? P4 : 0);          // [F][RS]
   float* sZ = sE + (size_t)F * RS;           // [P][RS]  Z, then dZ, then dP
-  const size_t offE = (size_t)F * KD + KD + 2 * (size_t)P4;
+  const size_t offE = (size_t)F * KD + KD + (DROP ? 3 : 2) * (size_t)P4;
+  const uint64_t vseed = DROP ? splitmix64(a.drop_seed) : 0;
 
   for (int i = threadIdx.x; i < KD * KD; i += blockDim.x) {
     const float w = __ldg(a.W + i);
@@ -541,8 +557,14 @@ __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
       for (int p = lane; p < P; p += 32) { const float e = expf(sS[p] - mx); sS[p] = e; den += e; }
       den = warp_sum(den);
       __syncwarp();
-      for (int p = lane; p < P; p += 32) sS[p] = sS[p] / den;
+      for (int p = lane; p < P; p += 32) {
+        sS[p] = sS[p] / den;
+        if (DROP) sM[p] = afm_mask_att(a, s, p) / a.keep_att;
+      }
       __syncwarp();
+      float nv[TD];                                               // n_k of the lane's columns (DROP)
+#pragma unroll
+      for (int t = 0; t < TD; t++) nv[t] = DROP ? afm_mask_vec(a, vseed, s, lane + 32 * t) / a.keep_vec : 1.f;
       // ---- afm = sum_p a_p E_i E_j (lanes over k), out ----
       float afm[TD];
 #pragma unroll
@@ -554,7 +576,7 @@ __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
 #pragma unroll
           for (int t = 0; t < TD; t++) { const int k = lane + 32 * t; ei[t] = (k < KD) ? sE[i * RS + k] : 0.f; in[t] = 0.f; }
           for (int j = i + 1; j < F; j++, p++) {
-            const float ap = sS[p];
+            const float ap = DROP ? sS[p] * sM[p] : sS[p];
 #pragma unroll
             for (int t = 0; t < TD; t++) { const int k = lane + 32 * t; if (k < KD) in[t] = fmaf(ap, sE[j * RS + k], in[t]); }
           }
@@ -564,7 +586,7 @@ __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
       }
       float part = 0.f;
 #pragma unroll
-      for (int t = 0; t < TD; t++) { const int k = lane + 32 * t; if (k < KD) part = fmaf(afm[t], swp[k], part); }
+      for (int t = 0; t < TD; t++) { const int k = lane + 32 * t; if (k < KD) part = fmaf(afm[t], DROP ? swp[k] * nv[t] : swp[k], part); }
       const float bil = warp_sum(part);
       const float out = (bil + bsum) + b0;                       // AFM.py:142 add_n
       if (a.out && lane == 0) a.out[s] = out;
@@ -577,7 +599,10 @@ __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
 #pragma unroll
         for (int t = 0; t < TD; t++) {
           const int k = lane + 32 * t;
-          if (k < KD) { sdafm[k] = g * swp[k]; gwp_acc[t] = fmaf(g, afm[t], gwp_acc[t]); }
+          if (k < KD) {
+            sdafm[k] = g * (DROP ? swp[k] * nv[t] : swp[k]);
+            gwp_acc[t] = fmaf(g, DROP ? afm[t] * nv[t] : afm[t], gwp_acc[t]);
+          }
         }
         __syncwarp();
         // ---- d a_p = (E_i E_j) . d afm (lane = pair), softmax backward ----
@@ -592,11 +617,11 @@ __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
             v = fmaf(x.x * y4.x, d.x, v); v = fmaf(x.y * y4.y, d.y, v); v = fmaf(x.z * y4.z, d.z, v); v = fmaf(x.w * y4.w, d.w, v);
           }
           sD[p] = v;
-          dotp = fmaf(sS[p], v, dotp);
+          dotp = fmaf(DROP ? sS[p] * sM[p] : sS[p], v, dotp);
         }
         const float dot = warp_sum(dotp);
         __syncwarp();
-        for (int p = lane; p < P; p += 32) sD[p] = sS[p] * (sD[p] - dot);       // d s_p
+        for (int p = lane; p < P; p += 32) sD[p] = sS[p] * ((DROP ? sM[p] * sD[p] : sD[p]) - dot);       // d s_p
         __syncwarp();
         // ---- d Z_p = d s_p p (Z_p > 0) (over Z) ; d p += d s_p relu(Z_p) ; d b += d Z_p  (lanes over a) ----
         for (int p = 0; p < P; p++) {
@@ -650,7 +675,7 @@ __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
       if (valid) {
         const int32_t* rec = a.idx + s * F;
         // ---- d P_p = a_p d afm + d Z_p W^T, in place ----
-        afm2_dpairs<KD, NR>(sZ, sWT, sdafm, sS, P, lane);
+        afm2_dpairs<KD, NR, DROP>(sZ, sWT, sdafm, sS, sM, P, lane);
         __syncwarp();
         // ---- d E_f = sum_{g != f} dP_{fg} * E_g  (lanes over k, registers; no read-modify-write through shared memory) ----
         for (int f = 0; f < F; f++) {
@@ -707,11 +732,11 @@ __global__ void __launch_bounds__(NW * 32, 1) afm2_kernel(const AfmArgs a) {
   }
 }
 
-template <int KD, int NW, int NR, bool TRAIN>
+template <int KD, int NW, int NR, bool TRAIN, bool DROP>
 static int launch_afm2(const AfmArgs& a, cudaStream_t st) {
-  const size_t smem = afm2_smem_floats(NW, a.F, KD, a.P) * sizeof(float);
+  const size_t smem = afm2_smem_floats(NW, a.F, KD, a.P, DROP) * sizeof(float);
   if (smem > 220 * 1024) return 1;
-  auto kern = afm2_kernel<KD, NW, NR, TRAIN>;
+  auto kern = afm2_kernel<KD, NW, NR, TRAIN, DROP>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
     set_error("afm2_kernel: cannot reserve %zu bytes of shared memory", smem);
     return HHFM_ERR_LAUNCH;
@@ -727,17 +752,17 @@ static int launch_afm2(const AfmArgs& a, cudaStream_t st) {
   return check_launch("afm2_kernel");
 }
 
-template <int KD, int NR, bool TRAIN>
+template <int KD, int NR, bool TRAIN, bool DROP>
 static int launch_afm2_warps(const AfmArgs& a, cudaStream_t st) {
   if constexpr (KD >= 32) {
-    const int rc = launch_afm2<KD, 8, NR, TRAIN>(a, st);
+    const int rc = launch_afm2<KD, 8, NR, TRAIN, DROP>(a, st);
     if (rc != 1) return rc;
   }
-  return launch_afm2<KD, 4, NR, TRAIN>(a, st);
+  return launch_afm2<KD, 4, NR, TRAIN, DROP>(a, st);
 }
 
 // returns 1 when the shape is not covered (the caller then uses afm_kernel)
-template <bool TRAIN>
+template <bool TRAIN, bool DROP>
 static int dispatch_afm2(const AfmArgs& a, cudaStream_t st) {
   const char* e = getenv("HHFM_AFM_V1");           // 1 = force the first layout (A/B measurements, tests of both kernels)
   if (e && e[0] == '1') return 1;
@@ -746,9 +771,9 @@ static int dispatch_afm2(const AfmArgs& a, cudaStream_t st) {
   if (nr > 3) return 1;
 #define HHFM_AFM2_CASE(KD_)                                                       \
   if (a.K == KD_) {                                                               \
-    if (nr == 1) return launch_afm2_warps<KD_, 1, TRAIN>(a, st);                  \
-    if (nr == 2) return launch_afm2_warps<KD_, 2, TRAIN>(a, st);                  \
-    return launch_afm2_warps<KD_, 3, TRAIN>(a, st);                               \
+    if (nr == 1) return launch_afm2_warps<KD_, 1, TRAIN, DROP>(a, st);            \
+    if (nr == 2) return launch_afm2_warps<KD_, 2, TRAIN, DROP>(a, st);            \
+    return launch_afm2_warps<KD_, 3, TRAIN, DROP>(a, st);                         \
   }
   HHFM_AFM2_CASE(64)
   HHFM_AFM2_CASE(32)
@@ -757,11 +782,11 @@ static int dispatch_afm2(const AfmArgs& a, cudaStream_t st) {
   return 1;
 }
 
-template <int TK, int TA, int NW, bool TRAIN>
+template <int TK, int TA, int NW, bool TRAIN, bool DROP>
 static int launch_afm(const AfmArgs& a, cudaStream_t st) {
-  const size_t smem = afm_smem_floats(NW, a.F, a.K, a.A, a.P) * sizeof(float);
+  const size_t smem = afm_smem_floats(NW, a.F, a.K, a.A, a.P, DROP) * sizeof(float);
   if (smem > 220 * 1024) return 1;
-  auto kern = afm_kernel<TK, TA, NW, TRAIN>;
+  auto kern = afm_kernel<TK, TA, NW, TRAIN, DROP>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
     set_error("afm_kernel: cannot reserve %zu bytes of shared memory", smem);
     return HHFM_ERR_LAUNCH;
@@ -777,17 +802,18 @@ static int launch_afm(const AfmArgs& a, cudaStream_t st) {
   return check_launch("afm_kernel");
 }
 
-template <bool TRAIN>
+// DROP: the training-dropout instantiations (TRAIN only)
+template <bool TRAIN, bool DROP = false>
 static int dispatch_afm(const AfmArgs& a, cudaStream_t st) {
   {
-    const int rc2 = dispatch_afm2<TRAIN>(a, st);
+    const int rc2 = dispatch_afm2<TRAIN, DROP>(a, st);
     if (rc2 != 1) return rc2;
   }
   // largest warp count whose shared-memory footprint fits; K % NW == 0 and K/NW % 4 == 0 are needed by the dW sweep
   const int tk = (a.K + 31) / 32, ta = (a.A + 31) / 32;
   int rc = 1;
 #define TRY(TKV, TAV, NWV)                                                      \
-  if (rc == 1 && tk == TKV && ta == TAV && a.K % (NWV * 4) == 0) rc = launch_afm<TKV, TAV, NWV, TRAIN>(a, st);
+  if (rc == 1 && tk == TKV && ta == TAV && a.K % (NWV * 4) == 0) rc = launch_afm<TKV, TAV, NWV, TRAIN, DROP>(a, st);
   TRY(1, 1, 4) TRY(1, 1, 2) TRY(2, 2, 4) TRY(2, 2, 2) TRY(4, 4, 4) TRY(4, 4, 2) TRY(4, 4, 1)
 #undef TRY
   if (rc == 1) {
@@ -796,6 +822,93 @@ static int dispatch_afm(const AfmArgs& a, cudaStream_t st) {
     return HHFM_ERR_UNSUPPORTED;
   }
   return rc;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// attention = 0 (AFM.py:132): afm = sum_p P_p = 0.5 (S^2 - sum_f E_f^2) with S = sum_f E_f, out = (afm n) . prediction_W
+// + sum_f bias[x_f] + b0 -- FM's interaction weighted by w~ = prediction_W n (n = the pooled-vector dropout factors, 1 outside
+// training).  No attention net, so no shared memory: one warp per sample, lane c owns the float4 chunk c of a row (K <= 128).
+// Training: dE_f = g w~ (S - E_f) into the gradient rows (vector reductions, hot-row replicas, touched rows as in afm_kernel),
+// d prediction_W += g n afm in registers, one atomic per column at the end.
+// ---------------------------------------------------------------------------------------------------------------
+template <bool TRAIN>
+__global__ void __launch_bounds__(kBlock) afm_sum_kernel(const AfmArgs a) {
+  __shared__ float scratch[32];
+  constexpr int NW = kBlock / 32;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int F = a.F, K = a.K;
+  const bool on = lane < (K >> 2);
+  const bool drop = TRAIN && a.keep_vec < 1.f;
+  const uint64_t vseed = splitmix64(a.drop_seed);
+  const float b0 = a.b0 ? __ldg(a.b0) : 0.f;
+  const float4 wp = on ? __ldg(reinterpret_cast<const float4*>(a.wpred) + lane) : f4_zero();
+  const int rep = a.hot.slot ? (int)(((int64_t)blockIdx.x * NW + warp) % a.hot.n_rep) : 0;
+  float4 gwp_acc = f4_zero();
+  float loss_acc = 0.f, g0_acc = 0.f;
+  for (int64_t s = (int64_t)blockIdx.x * NW + warp; s < a.B; s += (int64_t)gridDim.x * NW) {
+    const int32_t* rec = a.idx + s * F;
+    float4 S = f4_zero(), Q = f4_zero();
+    float bsum = 0.f;
+    for (int f = 0; f < F; f++) {
+      const int id = __ldg(rec + f);
+      if (on) {
+        const float4 e = __ldg(reinterpret_cast<const float4*>(a.V + (size_t)id * K) + lane);
+        S = f4_add(S, e);
+        Q = f4_add(Q, f4_mul(e, e));
+      }
+      if (a.bias) bsum += __ldg(a.bias + id);
+    }
+    float4 n = make_float4(1.f, 1.f, 1.f, 1.f);
+    if (drop && on)
+      n = make_float4(afm_mask_vec(a, vseed, s, 4 * lane) / a.keep_vec, afm_mask_vec(a, vseed, s, 4 * lane + 1) / a.keep_vec,
+                      afm_mask_vec(a, vseed, s, 4 * lane + 2) / a.keep_vec, afm_mask_vec(a, vseed, s, 4 * lane + 3) / a.keep_vec);
+    const float4 afm = f4_scale(f4_sub(f4_mul(S, S), Q), 0.5f);
+    const float4 wt = f4_mul(wp, n);                                    // w~ (zero on the lanes past K)
+    const float out = (warp_sum(f4_dot(afm, wt)) + bsum) + b0;
+    if (a.out && lane == 0) a.out[s] = out;
+    if (TRAIN) {
+      const float diff = __ldg(a.labels + s) - out;
+      const float g = -diff;
+      if (lane == 0) { loss_acc += 0.5f * diff * diff; g0_acc += g; }
+      gwp_acc = f4_fma(f4_mul(afm, n), g, gwp_acc);
+      const float4 dt = f4_scale(wt, g);
+      for (int f = 0; f < F; f++) {
+        const int id = __ldg(rec + f);
+        if (on) {
+          float* dst = a.gV + (size_t)id * K;
+          if (a.hot.slot != nullptr) {
+            const int hs = __ldg(a.hot.slot + id);
+            if (hs >= 0) dst = a.hot.ghot + ((size_t)rep * a.hot.n_hot + hs) * K;
+          }
+          const float4 e = __ldg(reinterpret_cast<const float4*>(a.V + (size_t)id * K) + lane);
+          red_add_v4(dst + 4 * lane, f4_mul(dt, f4_sub(S, e)));
+        }
+        if (lane == 0) {
+          if (a.gbias) scatter_bias(a.gbias, a.hot, rep, id, g);
+          touch_row(a.touch_stamp, a.stamp, a.touched_rows, a.touched_count, id);
+        }
+      }
+    }
+  }
+  if (TRAIN) {
+    if (on) {
+      atomicAdd(a.gwpred + 4 * lane, gwp_acc.x); atomicAdd(a.gwpred + 4 * lane + 1, gwp_acc.y);
+      atomicAdd(a.gwpred + 4 * lane + 2, gwp_acc.z); atomicAdd(a.gwpred + 4 * lane + 3, gwp_acc.w);
+    }
+    const float bl = block_sum(loss_acc, scratch);
+    write_partial(a.loss_partials, bl);
+    const float bg = block_sum(g0_acc, scratch);
+    if (threadIdx.x == 0 && a.gb0 && bg != 0.f) atomicAdd(a.gb0, bg);
+  }
+}
+
+template <bool TRAIN>
+static int launch_afm_sum(const AfmArgs& a, cudaStream_t st) {
+  int occ = 1;
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, afm_sum_kernel<TRAIN>, kBlock, 0);
+  if (occ < 1) occ = 1;
+  afm_sum_kernel<TRAIN><<<grid_for(a.B, kBlock / 32, occ), kBlock, 0, st>>>(a);
+  return check_launch("afm_sum_kernel");
 }
 
 static int check_afm(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* W, const float* batt,
@@ -817,6 +930,24 @@ static AfmArgs make_afm(const int32_t* idx, int64_t B, int64_t F, const float* V
   return a;
 }
 
+static int make_afm_train(AfmArgs& a, const int32_t* idx, int64_t B, int64_t F, const float* V, const float* bias, const float* b0,
+                          const float* W, const float* batt, const float* pvec, const float* wpred, int64_t M, int64_t K, int64_t A,
+                          const float* labels, float* out, float* gV, float* gbias, float* gb0, float* gW, float* gbatt, float* gp,
+                          float* gwpred, float* loss_partials, int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows,
+                          int32_t* touched_count, const int32_t* hot_slot, float* ghot, float* ghot_bias, int32_t n_rep, int32_t n_hot) {
+  int rc = check_afm(idx, B, F, V, W, batt, pvec, wpred, M, K, A);
+  if (rc) return rc;
+  HHFM_REQUIRE(B > 0 && labels && gV && gW && gbatt && gp && gwpred && loss_partials, "afm_fwd_bwd_sqloss: NULL argument");
+  HHFM_REQUIRE(!touch_stamp || (touched_rows && touched_count), "afm_fwd_bwd_sqloss: touch_stamp needs touched_rows/count");
+  HHFM_REQUIRE(!hot_slot || (ghot && n_rep >= 1 && n_hot >= 1), "afm_fwd_bwd_sqloss: hot_slot needs ghot, n_rep, n_hot");
+  a = make_afm(idx, B, F, V, bias, b0, W, batt, pvec, wpred, K, A);
+  a.labels = labels; a.out = out; a.gV = gV; a.gbias = gbias; a.gb0 = gb0; a.gW = gW; a.gbatt = gbatt; a.gp = gp;
+  a.gwpred = gwpred; a.loss_partials = loss_partials; a.touch_stamp = touch_stamp; a.stamp = stamp;
+  a.touched_rows = touched_rows; a.touched_count = touched_count;
+  a.hot = HotPlan{hot_slot, ghot, ghot_bias, n_rep, n_hot};
+  return HHFM_OK;
+}
+
 }  // namespace hhfm
 
 using namespace hhfm;
@@ -833,6 +964,21 @@ extern "C" int hhfm_afm_fwd(const int32_t* idx, int64_t B, int64_t F, const floa
   return dispatch_afm<false>(a, (cudaStream_t)stream);
 }
 
+extern "C" int hhfm_afm_fwd_attn(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* bias, const float* b0,
+                                 const float* W, const float* batt, const float* pvec, const float* wpred, int64_t M, int64_t K,
+                                 int64_t A, int32_t attention, float* out, hhfm_stream_t stream) {
+  HHFM_REQUIRE(attention == 0 || attention == 1, "afm_fwd_attn: attention=%d must be 0 or 1", (int)attention);
+  if (attention == 1) return hhfm_afm_fwd(idx, B, F, V, bias, b0, W, batt, pvec, wpred, M, K, A, out, stream);
+  int rc = check_afm(idx, B, F, V, W, batt, pvec, wpred, M, K, A);
+  if (rc) return rc;
+  HHFM_REQUIRE(out != nullptr, "afm_fwd_attn: out is NULL");
+  HHFM_REQUIRE(((uintptr_t)wpred & 15) == 0, "afm: prediction_W must be 16-byte aligned");
+  if (B == 0) return HHFM_OK;
+  AfmArgs a = make_afm(idx, B, F, V, bias, b0, W, batt, pvec, wpred, K, A);
+  a.out = out;
+  return launch_afm_sum<false>(a, (cudaStream_t)stream);
+}
+
 extern "C" int hhfm_afm_fwd_bwd_sqloss(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* bias,
                                        const float* b0, const float* W, const float* batt, const float* pvec,
                                        const float* wpred, int64_t M, int64_t K, int64_t A, const float* labels, float* out,
@@ -840,19 +986,50 @@ extern "C" int hhfm_afm_fwd_bwd_sqloss(const int32_t* idx, int64_t B, int64_t F,
                                        float* loss_partials, int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows,
                                        int32_t* touched_count, const int32_t* hot_slot, float* ghot, float* ghot_bias,
                                        int32_t n_rep, int32_t n_hot, hhfm_stream_t stream) {
-  int rc = check_afm(idx, B, F, V, W, batt, pvec, wpred, M, K, A);
+  AfmArgs a;
+  int rc = make_afm_train(a, idx, B, F, V, bias, b0, W, batt, pvec, wpred, M, K, A, labels, out, gV, gbias, gb0, gW, gbatt, gp,
+                          gwpred, loss_partials, touch_stamp, stamp, touched_rows, touched_count, hot_slot, ghot, ghot_bias, n_rep,
+                          n_hot);
   if (rc) return rc;
-  HHFM_REQUIRE(B > 0 && labels && gV && gW && gbatt && gp && gwpred && loss_partials, "afm_fwd_bwd_sqloss: NULL argument");
-  HHFM_REQUIRE(!touch_stamp || (touched_rows && touched_count), "afm_fwd_bwd_sqloss: touch_stamp needs touched_rows/count");
-  HHFM_REQUIRE(!hot_slot || (ghot && n_rep >= 1 && n_hot >= 1), "afm_fwd_bwd_sqloss: hot_slot needs ghot, n_rep, n_hot");
-  AfmArgs a = make_afm(idx, B, F, V, bias, b0, W, batt, pvec, wpred, K, A);
-  a.labels = labels; a.out = out; a.gV = gV; a.gbias = gbias; a.gb0 = gb0; a.gW = gW; a.gbatt = gbatt; a.gp = gp;
-  a.gwpred = gwpred; a.loss_partials = loss_partials; a.touch_stamp = touch_stamp; a.stamp = stamp;
-  a.touched_rows = touched_rows; a.touched_count = touched_count;
-  a.hot = HotPlan{hot_slot, ghot, ghot_bias, n_rep, n_hot};
   {
     const int frc = dispatch_afm_fused_tc(a, M, (cudaStream_t)stream);      // K = A = 64, F <= 11: one tcgen05 kernel
     if (frc != 1) return frc;
   }
   return dispatch_afm<true>(a, (cudaStream_t)stream);
+}
+
+extern "C" int hhfm_afm_fwd_bwd_sqloss_dropout(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* bias,
+                                               const float* b0, const float* W, const float* batt, const float* pvec,
+                                               const float* wpred, int64_t M, int64_t K, int64_t A, const float* labels,
+                                               float* out, float* gV, float* gbias, float* gb0, float* gW, float* gbatt, float* gp,
+                                               float* gwpred, float* loss_partials, int32_t* touch_stamp, int32_t stamp,
+                                               int32_t* touched_rows, int32_t* touched_count, const int32_t* hot_slot,
+                                               float* ghot, float* ghot_bias, int32_t n_rep, int32_t n_hot, int32_t attention,
+                                               float keep_att, float keep_vec, uint64_t drop_seed, int64_t sample_base,
+                                               hhfm_stream_t stream) {
+  HHFM_REQUIRE(attention == 0 || attention == 1, "afm_fwd_bwd_sqloss_dropout: attention=%d must be 0 or 1", (int)attention);
+  HHFM_REQUIRE(keep_att > 0.f && keep_att <= 1.f && keep_vec > 0.f && keep_vec <= 1.f,
+               "afm_fwd_bwd_sqloss_dropout: dropout keep [%g, %g] must be in (0, 1]", (double)keep_att, (double)keep_vec);
+  HHFM_REQUIRE(sample_base >= 0, "afm_fwd_bwd_sqloss_dropout: sample_base=%lld must be >= 0", (long long)sample_base);
+  const bool drop = keep_att < 1.f || keep_vec < 1.f;
+  if (attention == 1 && !drop)                            // keep = [1, 1]: the kernels of hhfm_afm_fwd_bwd_sqloss, unchanged
+    return hhfm_afm_fwd_bwd_sqloss(idx, B, F, V, bias, b0, W, batt, pvec, wpred, M, K, A, labels, out, gV, gbias, gb0, gW, gbatt, gp,
+                                   gwpred, loss_partials, touch_stamp, stamp, touched_rows, touched_count, hot_slot, ghot, ghot_bias,
+                                   n_rep, n_hot, stream);
+  AfmArgs a;
+  int rc = make_afm_train(a, idx, B, F, V, bias, b0, W, batt, pvec, wpred, M, K, A, labels, out, gV, gbias, gb0, gW, gbatt, gp,
+                          gwpred, loss_partials, touch_stamp, stamp, touched_rows, touched_count, hot_slot, ghot, ghot_bias, n_rep,
+                          n_hot);
+  if (rc) return rc;
+  a.keep_att = keep_att; a.keep_vec = keep_vec; a.drop_seed = drop_seed; a.sample_base = sample_base;
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (attention == 0) {
+    HHFM_REQUIRE(((uintptr_t)wpred & 15) == 0, "afm: prediction_W must be 16-byte aligned");
+    return launch_afm_sum<true>(a, st);
+  }
+  {
+    const int frc = dispatch_afm_fused_tc(a, M, st, true);
+    if (frc != 1) return frc;
+  }
+  return dispatch_afm<true, true>(a, st);
 }

@@ -33,9 +33,24 @@ struct AfmArgs {
   int32_t* touched_rows;
   int32_t* touched_count;
   HotPlan hot;
+  // training dropout (AFM.py:126,134), read by the DROP instantiations and the attention=0 kernel only:
+  // m_p = mask(seed, s, p) / keep_att on the attention weights, n_k = mask(splitmix64(seed), s, k) / keep_vec on the
+  // pooled vector, s = sample_base + row (the row's index in the global batch under data parallelism)
+  float keep_att, keep_vec;
+  uint64_t drop_seed;
+  int64_t sample_base;
 };
 
+// 0/1 masks of the two AFM dropout streams (oracle: afm_dropout_masks)
+__device__ __forceinline__ float afm_mask_att(const AfmArgs& a, int64_t s, int p) {
+  return dropout_keep01(a.drop_seed, a.sample_base + s, p, a.keep_att);
+}
+__device__ __forceinline__ float afm_mask_vec(const AfmArgs& a, uint64_t vseed, int64_t s, int k) {
+  return dropout_keep01(vseed, a.sample_base + s, k, a.keep_vec);
+}
+
 // afm_fused_tc.cu: returns 1 when the shape is not covered (the caller falls back to the SIMT kernels), else an HHFM_* code.
-int dispatch_afm_fused_tc(const AfmArgs& a, int64_t M, cudaStream_t st);
+// drop: the DROP instantiation (keep < 1 on either stream).
+int dispatch_afm_fused_tc(const AfmArgs& a, int64_t M, cudaStream_t st, bool drop = false);
 
 }  // namespace hhfm

@@ -76,6 +76,8 @@ struct Misc {
   unsigned char pidx[kMaxF][kMaxF + 1];
   uint64_t bar1, bar2, bar3;    // GEMM 1 | GEMM 2 | GEMM 3 complete
   uint32_t tmem;
+  uint32_t abits[2][2][2];        // DROP: [tile parity][slot][pair / 32] attention-dropout keep bits
+  float nvec[2][2][KD];           // DROP: [tile parity][slot][column] pooled-vector dropout factors n_k (0 or 1 / keep)
 };
 static_assert(sizeof(Misc) <= kMiscBytes, "Misc does not fit its shared-memory slot");
 
@@ -173,7 +175,12 @@ __device__ __forceinline__ float finish8(float (&acc)[8], int lane) {
 }
 
 // NQ column groups: thread = (operand row, group of CW = 64 / NQ columns); 128 * NQ threads
-template <int NQ>
+// DROP: training dropout (AFM.py:126,134).  The masks of a tile's two samples are drawn two tiles ahead, during the embedding
+// scatter (where warps 10..15 have no items), one hash per lane of the last 8 warps, into Misc: the pair keep bits (one ballot
+// per 32 pairs) and the column factors n_k.  With m_p (pairs) and n_k (columns): u_p is built
+// with w~ = prediction_W n, the softmax uses od = sum a_p m_p u_p, c_r = g a_p m_p and ds = g a_p (m_p u_p - od), the direct
+// term of dP is c_r w~ and the d prediction_W fold is scaled by n.  Everything downstream of ds is unchanged.
+template <int NQ, bool DROP>
 __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs a, const int64_t n_tiles) {
   constexpr int CW = KD / NQ;
   constexpr int kThreads = 128 * NQ;
@@ -303,6 +310,25 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
       pr[i] = m * (x.x * y.x); pr[i + 1] = m * (x.y * y.y); pr[i + 2] = m * (x.z * y.z); pr[i + 3] = m * (x.w * y.w);
     }
   };
+  // DROP: the masks of the tile `tile` (two samples) -> abits / nvec [pr]; warp-uniform, called by every thread
+  auto stage_masks = [&](int64_t tile, int pr) {
+    constexpr int w0 = kThreads / 32 - 8;
+    if constexpr (DROP) if (warp >= w0) {
+      const int w8 = warp - w0, sl = (w8 >> 1) & 1, wd = w8 & 1;
+      const int64_t smp2 = 2 * tile + sl;
+      if (w8 < 4) {
+        mi.nvec[pr][sl][32 * wd + lane] = afm_mask_vec(a, splitmix64(a.drop_seed), smp2, 32 * wd + lane) / a.keep_vec;
+      } else {
+        const uint32_t bits = __ballot_sync(0xffffffffu, afm_mask_att(a, smp2, 32 * wd + lane) != 0.f);
+        if (lane == 0) mi.abits[pr][sl][wd] = bits;
+      }
+    }
+  };
+  // w~_i = prediction_W n_i of this thread's column i in the tile of parity pr
+  auto wtilde = [&](int pr, int i) {
+    if constexpr (DROP) return mi.wpred[c0 + i] * mi.nvec[pr][ss][c0 + i];
+    else return mi.wpred[c0 + i];
+  };
   // P rows of a tile -> TMEM (x and lo): the A operand of GEMM 1
   auto build_p_tmem = [&](const float* Es, int par) {
     float pr[CW];
@@ -312,7 +338,7 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
 #pragma unroll
     for (int i = 0; i < CW; i++) {
       rx[i] = __float_as_uint(pr[i]); rl[i] = __float_as_uint(lo_part(pr[i]));
-      up = fmaf(mi.wpred[c0 + i], pr[i], up);                           // u_p = prediction_W . P_p (AFM.py:138-139, per pair)
+      up = fmaf(wtilde(par, i), pr[i], up);                              // u_p = prediction_W . P_p (AFM.py:138-139, per pair)
     }
     mi.u_part[par][cg][row] = up;
     tmem_st(t_lane + cPX + c0, rx);
@@ -338,6 +364,10 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
   {
     const int id0 = load_id(blockIdx.x), id1 = load_id((int64_t)blockIdx.x + g_tiles);
     if (bt >= 0 && bt < 2 * F) { mi.ids[0][bt / F][bt % F] = id0; mi.ids[1][bt / F][bt % F] = id1; }
+    if constexpr (DROP) {
+      stage_masks(blockIdx.x, 0);
+      stage_masks((int64_t)blockIdx.x + g_tiles, 1);
+    }
     if (tid < 2 * (kMaxF + 1)) {
       const int s2 = tid / (kMaxF + 1), f = tid % (kMaxF + 1);
 #pragma unroll
@@ -420,6 +450,13 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
       const float e_lo = v_lo ? expf(s_lo - mx) : 0.f, e_hi = v_hi ? expf(s_hi - mx) : 0.f;   // AFM.py:125 softmax over the pairs
+      float m_lo = 1.f, m_hi = 1.f;                           // m_p of the pairs lane and lane + 32 (DROP)
+      if constexpr (DROP) {
+        const float m_on = 1.f / a.keep_att;
+        m_lo = ((mi.abits[par][ss][0] >> lane) & 1u) ? m_on : 0.f;
+        m_hi = ((mi.abits[par][ss][1] >> lane) & 1u) ? m_on : 0.f;
+        u_lo *= m_lo; u_hi *= m_hi;                           // m_p u_p
+      }
       float d0 = e_lo, d1 = e_hi, n0 = e_lo * u_lo, n1 = e_hi * u_hi;
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) {
@@ -429,7 +466,7 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
       const float den = d0 + d1;
       const float od = (n0 + n1) / den;                       // sum_p a_p (prediction_W . P_p) = prediction_W . afm, AFM.py:130-139
       const float att = ((pp < 32) ? e_lo : e_hi) / den;
-      const float u_r = (pp < 32) ? u_lo : u_hi;
+      const float u_r = (pp < 32) ? u_lo : u_hi;            // DROP: m_p u_p
       float g = 0.f;
       if (smp < a.B) {
         const float out = (od + mi.bsum[ss]) + b0;            // AFM.py:142
@@ -442,8 +479,13 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
         }
       }
       if (pp == 0 && cg == 0) mi.g[ss] = g;
-      c_r = g * att;                                          // d afm . P_p = g * u_p; softmax backward: ds = a (da - sum a da)
-      ds = c_r * (u_r - od);
+      if constexpr (DROP) {                                   // d a_p = g m_p u_p; ds = a (da - sum a da)
+        c_r = (g * att) * ((pp < 32) ? m_lo : m_hi);
+        ds = (g * att) * (u_r - od);
+      } else {
+        c_r = g * att;                                        // d afm . P_p = g * u_p; softmax backward: ds = a (da - sum a da)
+        ds = c_r * (u_r - od);
+      }
     }
     // dZ = ds * p * relu'(Z + b) -> TMEM (A of GEMM 2) and the K-major dZT tiles (B of GEMM 3)
     float dz[CW], hp[CW];
@@ -505,6 +547,10 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
     fold8<CW>(dz, gb8, lane);
     fold8<CW>(hp, gp8, lane);
     pair_products(Es, dz, c_r);
+    if constexpr (DROP) {
+#pragma unroll
+      for (int i = 0; i < CW; i++) dz[i] *= mi.nvec[par][ss][c0 + i];
+    }
     fold8<CW>(dz, gw8, lane);
     if (has_next) build_p_tmem(EsBuf + nb * (kEBytes / 4), par ^ 1);
     mbar_wait(&mi.bar2, ph2, nullptr);      // GEMM 2
@@ -516,7 +562,7 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
       uint32_t r[CW];
       tmem_ld(t_lane + cDP + c0, r);
 #pragma unroll
-      for (int i = 0; i < CW; i++) r[i] = __float_as_uint(fmaf(c_r, mi.wpred[c0 + i], __uint_as_float(r[i])));
+      for (int i = 0; i < CW; i++) r[i] = __float_as_uint(fmaf(c_r, wtilde(par, i), __uint_as_float(r[i])));
       mbar_wait(&mi.bar3, ph2, nullptr);    // GEMM 3
       ph2 ^= 1;
       tc_fence_after();
@@ -532,6 +578,9 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
     tc_fence_before();
     __syncthreads();
     if (tid == kIssuer1 && has_next) { tc_fence_after(); issue_gemm1(); }      // GEMM 1 of the next tile runs behind the scatter below
+    // the masks of tile t + 2 into parity par: its last reader (this tile's epilogue 2) is behind the barrier above, its first
+    // reader (the P rows of tile t + 2, built in the next tile) behind the next tile's barrier (1)
+    if constexpr (DROP) stage_masks(t + 2 * g_tiles, par);
     // dE_f = sum_{j != f} dP_(f,j) * E_j ; one vector reduction per 16 bytes of the gradient row
     for (int i = tid; i < 2 * F * (KD / 4); i += kThreads) {
       int s2, f, c;
@@ -600,26 +649,37 @@ __global__ void __launch_bounds__(128 * NQ, 1) afm_fused_tc_kernel(const AfmArgs
 
 }  // namespace aft
 
-int dispatch_afm_fused_tc(const AfmArgs& a, int64_t M, cudaStream_t st) {
-  if (a.K != aft::KD || a.A != aft::KD || a.F > aft::kMaxF || a.F < 2 || a.P > aft::kSlot) return 1;
-  const char* env = getenv("HHFM_AFM_TC");               // 0 = fp32 CUDA-core kernels (A/B runs, tests of both paths)
-  if (env && env[0] == '0') return 1;
+template <bool DROP>
+static bool configure_fused_tc() {
   static bool configured = false;
   if (!configured) {
-    if (cudaFuncSetAttribute(aft::afm_fused_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)aft::kSmemBytes) != cudaSuccess ||
-        cudaFuncSetAttribute(aft::afm_fused_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)aft::kSmemBytes) != cudaSuccess) {
+    if (cudaFuncSetAttribute(aft::afm_fused_tc_kernel<4, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)aft::kSmemBytes) != cudaSuccess ||
+        cudaFuncSetAttribute(aft::afm_fused_tc_kernel<2, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)aft::kSmemBytes) != cudaSuccess) {
       cudaGetLastError();
-      return 1;
+      return false;
     }
     configured = true;
   }
+  return true;
+}
+
+int dispatch_afm_fused_tc(const AfmArgs& a, int64_t M, cudaStream_t st, bool drop) {
+  if (a.K != aft::KD || a.A != aft::KD || a.F > aft::kMaxF || a.F < 2 || a.P > aft::kSlot) return 1;
+  const char* env = getenv("HHFM_AFM_TC");               // 0 = fp32 CUDA-core kernels (A/B runs, tests of both paths)
+  if (env && env[0] == '0') return 1;
+  if (!(drop ? configure_fused_tc<true>() : configure_fused_tc<false>())) return 1;
   const int groups = (env && env[0] == '2') ? 2 : 4;      // column groups per row: 4 = 16 warps (default), HHFM_AFM_TC=2: 8 warps
   const int64_t n_tiles = (a.B + 1) / 2;
   int grid = sm_count();
   if (grid > kPartials) grid = kPartials;
   if ((int64_t)grid > n_tiles) grid = (int)n_tiles;
-  if (groups == 4) aft::afm_fused_tc_kernel<4><<<grid, 512, aft::kSmemBytes, st>>>(a, n_tiles);
-  else aft::afm_fused_tc_kernel<2><<<grid, 256, aft::kSmemBytes, st>>>(a, n_tiles);
+  if (drop) {
+    if (groups == 4) aft::afm_fused_tc_kernel<4, true><<<grid, 512, aft::kSmemBytes, st>>>(a, n_tiles);
+    else aft::afm_fused_tc_kernel<2, true><<<grid, 256, aft::kSmemBytes, st>>>(a, n_tiles);
+  } else {
+    if (groups == 4) aft::afm_fused_tc_kernel<4, false><<<grid, 512, aft::kSmemBytes, st>>>(a, n_tiles);
+    else aft::afm_fused_tc_kernel<2, false><<<grid, 256, aft::kSmemBytes, st>>>(a, n_tiles);
+  }
   int rc = check_launch("afm_fused_tc_kernel");
   if (rc != HHFM_OK) return rc;
   if (a.touch_stamp != nullptr) rc = launch_touched_compact(a.touch_stamp, a.stamp, M, a.touched_rows, a.touched_count, st);

@@ -133,9 +133,12 @@ class _Base:
         keep = float(getattr(self, "keep", 1.0))
         if keep >= 1.0:
             return 1.0, 0
+        return keep, self._drop_seed()
+
+    def _drop_seed(self):
         seed = (int(getattr(self, "random_seed", 2016)) * 0x9E3779B97F4A7C15 + self._opt.t) & 0xFFFFFFFFFFFFFFFF
         self._last_drop_seed = seed
-        return keep, seed
+        return seed
 
     # ---- single-touch rows (include/hhfm_sm100.h K14) ---------------------------------------------------------------
     def _single_touch(self, ids_dev, n_cols, with_bias, keep=1.0):
@@ -984,10 +987,10 @@ class AFM(FM):
         self._init_graph()
 
     def _init_graph(self):
-        if not self.attention:
-            raise NotImplementedError("attention=0 (AFM.py:132) is not on the accelerated path; the reference default is 1")
-        if any(float(k) != 1.0 for k in self.keep):
-            raise NotImplementedError("dropout keep<1 (AFM.py:126,134) is not on the accelerated path; default is [1,1]")
+        self.keep = [float(k) for k in self.keep]
+        if len(self.keep) != 2 or not all(0.0 < k <= 1.0 for k in self.keep):
+            raise ValueError("keep must be two values in (0, 1] (attention weights, pooled vector)")
+        self.attention = 1 if self.attention else 0
         self.train_features = Handle("train_features_afm")
         self.train_labels = Handle("train_labels_afm")
         self.dropout_keep = Handle("dropout_keep_afm")
@@ -1030,12 +1033,33 @@ class AFM(FM):
         return self._predict_dev(idx)
 
     def _predict_dev(self, idx):
+        """The forward with keep = [1, 1] (the reference evaluates without dropout)."""
         B, F = idx.shape
         out = torch.empty(B, dtype=torch.float32, device=self.device)
         W, batt, pv, wp = self._small()
-        _lib.call("hhfm_afm_fwd", ptr(idx), B, F, ptr(self.weights["feature_embeddings"]), ptr(self.weights["feature_bias"]),
-                  ptr(self._b0), W, batt, pv, wp, self._M, self._K, self._A, ptr(out), cur_stream())
+        _lib.call("hhfm_afm_fwd_attn", ptr(idx), B, F, ptr(self.weights["feature_embeddings"]), ptr(self.weights["feature_bias"]),
+                  ptr(self._b0), W, batt, pv, wp, self._M, self._K, self._A, self.attention, ptr(out), cur_stream())
         return out
+
+    def _drop_args(self):
+        """(keep_att, keep_vec, seed) of this step's dropout masks (AFM.py:126,134; training only).  The seed follows the
+        scheme of FM / MF: a pure function of (random_seed, step)."""
+        k0, k1 = self.keep
+        if k0 >= 1.0 and k1 >= 1.0:
+            return 1.0, 1.0, 0
+        return k0, k1, self._drop_seed()
+
+    def _sample_base(self, B):
+        """Index of this rank's first row in the global batch, so that every rank draws the masks of its own rows: the
+        ranks' batch sizes are exchanged (rank order) under data parallelism, 0 on one GPU."""
+        if self._dp_group is None:
+            return 0
+        import torch.distributed as dist
+        ws = dist.get_world_size(self._dp_group)
+        sizes = [torch.zeros(1, dtype=torch.int64, device=self.device) for _ in range(ws)]
+        dist.all_gather(sizes, torch.tensor([B], dtype=torch.int64, device=self.device), group=self._dp_group)
+        rank = dist.get_rank(self._dp_group)
+        return int(sum(int(t.item()) for t in sizes[:rank]))
 
     def partial_fit(self, data):
         """AFM.py:205-208.  V and feature_bias receive IndexedSlices (only touched rows move); attention_W carries the
@@ -1056,21 +1080,30 @@ class AFM(FM):
                   ptr(self._gbatt), ptr(self._gp), ptr(self._gwp), ptr(self._loss_partials), ts, stamp, tr, tc,
                   *(hot.args(True) if hot else NO_HOT_BIAS))
         # K == A == 64, F <= 11: one fused tcgen05 kernel (csrc/afm_fused_tc.cu); other shapes: fp32 CUDA-core kernels
-        _lib.call("hhfm_afm_fwd_bwd_sqloss", *common, cur_stream())
+        k0, k1, dseed = self._drop_args()
+        att = self.attention
+        if att and k0 >= 1.0 and k1 >= 1.0:
+            _lib.call("hhfm_afm_fwd_bwd_sqloss", *common, cur_stream())
+        else:
+            base = self._sample_base(B) if dseed else 0
+            _lib.call("hhfm_afm_fwd_bwd_sqloss_dropout", *common, att, k0, k1, dseed, base, cur_stream())
+        # attention=0: attention_W / b / p are not part of the graph (no gradient, no update, no regulariser: AFM.py:132)
+        dense = (self._gW, self._gbatt, self._gp, self._gwp) if att else (self._gwp,)
         if hot:
             hot.fold(self._gV, self._gb)
         if self._dp_group is not None:
             import torch.distributed as dist
             self._allreduce_grads()
-            for g in (self._gW, self._gbatt, self._gp, self._gwp):
+            for g in dense:
                 dist.all_reduce(g, group=self._dp_group)
         self._apply_table(sparse_ok=True)                       # lamda on V is 0: rows (or the dense equivalent under DP)
         self._apply_bias()
-        lam = float(self.lamda_attention)
+        lam = float(self.lamda_attention) if att else 0.0
         o = self._opt
-        o.apply_dense("attention_W", self.weights["attention_W"], self._gW, lam, self._sq_partials if lam > 0 else None)
-        o.apply_dense("attention_b", self.weights["attention_b"], self._gbatt, 0.0, None)
-        o.apply_dense("attention_p", self.weights["attention_p"], self._gp, 0.0, None)
+        if att:
+            o.apply_dense("attention_W", self.weights["attention_W"], self._gW, lam, self._sq_partials if lam > 0 else None)
+            o.apply_dense("attention_b", self.weights["attention_b"], self._gbatt, 0.0, None)
+            o.apply_dense("attention_p", self.weights["attention_p"], self._gp, 0.0, None)
         o.apply_dense("prediction", self.weights["prediction"], self._gwp, 0.0, None)
         self._enqueue_loss(lam > 0, 0.5 * lam)
 
@@ -1078,15 +1111,16 @@ class AFM(FM):
         """AFM.topk (AFM.py:209-246) scores every item for each context row.  The reference restates `out` with an
         un-normalised exp attention and drops the per-row constants, which is rank-equivalent to scoring the full model.
         Covered shapes (K == A in {16, 32, 64}) go through the item-separable scorer (csrc/afm_topn.cu: the context-only
-        pairs once per row, the F-1 item pairs per (row, item)); other shapes send every (row, item) pair through the
-        forward kernel.  Either way the exact selector (lowest-index ties) makes the lists."""
+        pairs once per row, the F-1 item pairs per (row, item)); other shapes, and attention=0, send every (row, item) pair
+        through the model's forward kernel.  Either way the exact selector (lowest-index ties) makes the lists."""
         A = np.asarray(A)
         A_dev, stride = self._topn.upload_rows(A, self._M)
         C_rows, F = A.shape
         N = self.n_item
         K, Adim = int(self.hidden_factor[1]), int(self._A)
         out_ids = torch.empty(C_rows, tp, dtype=torch.int32, device=self.device)
-        separable = bool(_lib.load().hhfm_afm_topn_supported(F, K, Adim)) and os.environ.get("HHFM_AFM_TOPN_SEPARABLE", "1") != "0"
+        separable = bool(_lib.load().hhfm_afm_topn_supported(F, K, Adim)) and os.environ.get("HHFM_AFM_TOPN_SEPARABLE", "1") != "0" \
+            and self.attention == 1
         w = self.weights
         if separable:
             chunk = max(1, min(65535, (1 << 26) // max(N, 1)))

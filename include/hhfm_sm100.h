@@ -191,6 +191,27 @@ int hhfm_afm_fwd_bwd_sqloss(const int32_t* idx, int64_t B, int64_t F, const floa
                             const int32_t* hot_slot, float* ghot, float* ghot_bias, int32_t n_rep, int32_t n_hot,
                             hhfm_stream_t stream);
 
+/* Training dropout and the attention=0 variant (AFM.py:126,132,134).  The arguments of hhfm_afm_fwd_bwd_sqloss, then:
+ *   attention   1: the attention net as above;  0: afm = sum_p P_p = 0.5 (S^2 - sum_f E_f^2) (no attention net; gW, gbatt, gp
+ *               are not written)
+ *   keep_att, keep_vec   tf.nn.dropout keep probabilities in (0, 1] of the attention weights (per sample and pair; unused
+ *               when attention = 0) and of the pooled vector (per sample and column): a_p -> a_p m_p / keep_att and
+ *               afm -> afm n / keep_vec with 0/1 masks m = mask(drop_seed, s, p), n = mask(splitmix64(drop_seed), s, k)
+ *   sample_base the index of row 0 in the global batch (data parallelism: every rank draws the masks of its own rows), >= 0
+ * keep = [1, 1] with attention = 1 runs the kernels of hhfm_afm_fwd_bwd_sqloss unchanged.  hhfm_afm_fwd_attn is the
+ * forward (no dropout: the reference evaluates with keep = [1, 1]) for either value of `attention`. */
+int hhfm_afm_fwd_bwd_sqloss_dropout(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* bias,
+                                    const float* b0, const float* W, const float* batt, const float* pvec, const float* wpred,
+                                    int64_t M, int64_t K, int64_t A, const float* labels, float* out, float* gV, float* gbias,
+                                    float* gb0, float* gW, float* gbatt, float* gp, float* gwpred, float* loss_partials,
+                                    int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows, int32_t* touched_count,
+                                    const int32_t* hot_slot, float* ghot, float* ghot_bias, int32_t n_rep, int32_t n_hot,
+                                    int32_t attention, float keep_att, float keep_vec, uint64_t drop_seed, int64_t sample_base,
+                                    hhfm_stream_t stream);
+int hhfm_afm_fwd_attn(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* bias, const float* b0,
+                      const float* W, const float* batt, const float* pvec, const float* wpred, int64_t M, int64_t K,
+                      int64_t A, int32_t attention, float* out, hhfm_stream_t stream);
+
 /* The training pass of K == A == 64, F <= 11 runs as ONE tcgen05 kernel (afm_fused_tc.cu: the three matrix products P W,
  * dZ W^T, P^T dZ as 3xTF32 split products with the operands built in shared memory and the logits / dP in TMEM);
  * hhfm_afm_fwd_bwd_sqloss selects it by shape, HHFM_AFM_TC=0 forces the fp32 CUDA-core kernels. */
