@@ -413,12 +413,25 @@ __global__ void __launch_bounds__(kBlock, 2) pairrank_sum_train_kernel(const PrA
 #pragma unroll
     for (int j = 0; j <= NNEG; j++) p[j] = group_sum<LPS>(p[j]);
 
+    // KEEP: the first negative that reaches the max stays in registers (row and id), so the backward pass does not load it
+    // again -- one dependent L2 round trip less per sample.  It costs registers: with NP > 0 the kernel stays within the 128
+    // of two CTAs per SM (at most 128 in -Xptxas -v), but without context (NP = 0, BPR) it would go from about 80 registers
+    // (three CTAs per SM) to about 118 (two), and the lost residency costs more than the load (on a B200, models.bpr_c4:
+    // 0.697 -> 0.870 ms per step with KEEP), so NP = 0 loads the row again.
+    constexpr bool KEEP = NP > 0;
     float m = p[1];
     unsigned tie = 1u;
+    float4 vmax = e[2 + NS];
+    int idmax = idx[2 + NP];
 #pragma unroll
     for (int j = 1; j < NNEG; j++) {
-      if (p[1 + j] > m) { m = p[1 + j]; tie = 1u << j; }
-      else if (p[1 + j] == m) tie |= 1u << j;
+      if (p[1 + j] > m) {
+        m = p[1 + j];
+        tie = 1u << j;
+        if (KEEP) { vmax = e[2 + NS + j]; idmax = idx[2 + NP + j]; }
+      } else if (p[1 + j] == m) {
+        tie |= 1u << j;
+      }
     }
     if (valid) {
       const float x = p[0] - m;
@@ -430,6 +443,11 @@ __global__ void __launch_bounds__(kBlock, 2) pairrank_sum_train_kernel(const PrA
       scatter(idx[1], f4_scale(hyb, gp));
       const float4 tn = f4_scale(hyb, gn);
       unsigned w = tie;
+      if (KEEP) {                           // further tied negatives (rare) are loaded again, in the same order
+        dh = f4_fma(vmax, gn, dh);
+        scatter(idmax, tn);
+        w &= w - 1u;
+      }
       while (w) {
         const int j = __ffs((int)w) - 1;
         w &= w - 1;
