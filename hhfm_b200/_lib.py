@@ -27,6 +27,10 @@ SIGNATURES = {
                                        vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64, vp],
     "hhfm_fm_fwd_bwd_sqloss_st": [vp, vp, vp, i64, i64, vp, vp, vp, i64, i64, i32, vp, vp, vp, vp, vp, vp, vp, i32, vp,
                                   vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64, vp, vp],
+    "hhfm_fm_bn_fwd_bwd_sqloss": [vp, vp, vp, i64, i64, vp, vp, vp, i64, i64, i32, vp, vp, vp, vp, vp, vp, vp, i32, vp,
+                                  vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64, vp, vp, vp, vp, vp, vp, f32, f32, vp, i64,
+                                  vp],
+    "hhfm_fm_bn_fwd": [vp, i64, i64, vp, vp, vp, i64, i64, vp, vp, vp, vp, f32, vp, vp],
     "hhfm_count_refs": [vp, i64, i64, i64, i64, vp, vp],
     "hhfm_fm_bwd": [vp, vp, vp, i64, i64, vp, i64, i64, i32, vp, vp, vp, vp, i32, vp],
     "hhfm_afm_fwd": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, vp, vp],
@@ -100,6 +104,7 @@ INT64_FUNCS = {
     "hhfm_dfm_param_count": [i64, i64, i32, vp],
     "hhfm_dfm_reg_count": [i64, i64, i32, vp],
     "hhfm_workspace_bytes_dfm": [i64, i64, i64, i32, vp],
+    "hhfm_workspace_bytes_fm_bn": [i64, i64],
 }
 OPTIONAL = {}   # symbols added by later kernels are appended by their modules via `declare`
 

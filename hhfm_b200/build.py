@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libhhfm_sm100.so")
 OBJ = os.path.join(HERE, "build")
-SOURCES = ["host.cu", "fm.cu", "pairrank.cu", "opt.cu", "topn.cu", "afm.cu", "afm_fused_tc.cu", "afm_topn.cu", "cars2.cu", "dfm.cu", "dfm_tc.cu", "p2p.cu", "sampler.cu", "topn_tc.cu", "wd.cu"]
+SOURCES = ["host.cu", "fm.cu", "fm_bn.cu", "pairrank.cu", "opt.cu", "topn.cu", "afm.cu", "afm_fused_tc.cu", "afm_topn.cu", "cars2.cu", "dfm.cu", "dfm_tc.cu", "p2p.cu", "sampler.cu", "topn_tc.cu", "wd.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "--expt-relaxed-constexpr"]

@@ -589,6 +589,8 @@ class FM(_Base):
     _supports_sparse_dp = True
 
     interaction = 0
+    _bn = False
+    BN_EPS, BN_DECAY = 1e-3, 0.9          # batch_norm_layer: decay=0.9, epsilon left at the tf.contrib.layers.batch_norm default
 
     def __init__(self, valid_dimension, features_M, n_user, n_item, hidden_factor, learning_rate, lamda_bilinear, keep,
                  optimizer_type, batch_norm, verbose, random_seed=2016):
@@ -608,8 +610,6 @@ class FM(_Base):
         self._init_graph()
 
     def _init_graph(self):
-        if self.batch_norm:
-            raise NotImplementedError("batch_norm=1 (FM.py:111-112) is not on the accelerated path; default is 0")
         if not (0.0 < float(self.keep) <= 1.0):
             raise ValueError("keep must be in (0, 1]")
         self.train_features = Handle("train_features_fm")    # FM.py:89-92
@@ -623,6 +623,26 @@ class FM(_Base):
                     self.learning_rate, 0.1, self.lamda_bilinear)
         self._b0 = torch.zeros(1, dtype=torch.float32, device=self.device)
         self.weights["bias"] = self._b0.view(())                                   # FM.py:157
+        self._bn = bool(self.batch_norm)
+        if self._bn:
+            # FM.py:111-112 batch_norm_layer(scope='bn_fm'): scale gamma = 1, offset beta = 0, moving mean 0, moving variance 1
+            K, dev = self._K, self.device
+            self.weights["bn_fm/gamma"] = torch.ones(K, dtype=torch.float32, device=dev)
+            self.weights["bn_fm/beta"] = torch.zeros(K, dtype=torch.float32, device=dev)
+            self.weights["bn_fm/moving_mean"] = torch.zeros(K, dtype=torch.float32, device=dev)
+            self.weights["bn_fm/moving_variance"] = torch.ones(K, dtype=torch.float32, device=dev)
+            self._g_bn = torch.zeros(2, K, dtype=torch.float32, device=dev)         # d gamma, d beta
+            self._bn_ws = None
+
+    def enable_data_parallel(self, *args, **kwargs):
+        if self._bn:
+            raise NotImplementedError("batch_norm=1 under data parallelism: per-rank batch statistics are not the single-GPU "
+                                      "step, and global statistics need two more collectives per step")
+        return super().enable_data_parallel(*args, **kwargs)
+
+    def _bn_args(self):
+        w = self.weights
+        return (ptr(w["bn_fm/gamma"]), ptr(w["bn_fm/beta"]), ptr(w["bn_fm/moving_mean"]), ptr(w["bn_fm/moving_variance"]))
 
     # -- forward only: `sess.run(model.out, ...)` of evaluate_AUC (FM.py:313-319) --
     def score_device(self, idx):
@@ -630,6 +650,10 @@ class FM(_Base):
         self.flush()
         B, F = idx.shape
         out = torch.empty(B, dtype=torch.float32, device=self.device)
+        if self._bn:                  # train_phase=False: the moving statistics (FM.py:111, is_training=train_phase)
+            _lib.call("hhfm_fm_bn_fwd", ptr(idx), B, F, ptr(self.weights["feature_embeddings"]), ptr(self.weights["feature_bias"]),
+                      ptr(self._b0), self._M, self._K, *self._bn_args(), self.BN_EPS, ptr(out), cur_stream())
+            return out
         _lib.call("hhfm_fm_fwd", None, ptr(idx), None, B, F, ptr(self.weights["feature_embeddings"]),
                   ptr(self.weights.get("feature_bias")), ptr(self._b0), self._M, self._K, self.interaction, ptr(out),
                   cur_stream())
@@ -657,12 +681,32 @@ class FM(_Base):
         ts, stamp, tr, tc = self._touch_args(extra=self._opt.kind == "momentum")
         hot = self._hot_plan(idx, True)
         keep, dseed = self._drop_args()
+        if self._bn:
+            self._fit_bn(idx, y, ts, stamp, tr, tc, hot, keep, dseed)
+            return
         plan = self._single_touch(idx, F, True, keep) if ts is not None else None
         _lib.call("hhfm_fm_fwd_bwd_sqloss_st", None, ptr(idx), None, B, F, ptr(V), ptr(bias), ptr(self._b0), self._M,
                   self._K, self.interaction, ptr(y), None, ptr(self._gV), ptr(self._gb), ptr(self._gb0),
                   ptr(self._loss_partials), ts, stamp, tr, tc, *(hot.args(True) if hot else NO_HOT_BIAS),
                   1 if self.deterministic else 0, keep, dseed, C.addressof(plan) if plan is not None else None, cur_stream())
         self._finish_step(hot, True, self._apply_bias if bias is not None else None)
+
+    def _fit_bn(self, idx, y, ts, stamp, tr, tc, hot, keep, dseed):
+        """The step with batch normalisation (csrc/fm_bn.cu): V, feature_bias and the scalar bias go through the usual tail;
+        gamma and beta are dense variables without L2, stepped after it.  Single-touch rows (K14) stay off."""
+        B, F = idx.shape
+        nbytes = int(_lib.load().hhfm_workspace_bytes_fm_bn(B, self._K))
+        if self._bn_ws is None or self._bn_ws.numel() < nbytes:
+            self._bn_ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        V = self.weights["feature_embeddings"]
+        _lib.call("hhfm_fm_bn_fwd_bwd_sqloss", None, ptr(idx), None, B, F, ptr(V), ptr(self.weights["feature_bias"]), ptr(self._b0),
+                  self._M, self._K, 0, ptr(y), None, ptr(self._gV), ptr(self._gb), ptr(self._gb0), ptr(self._loss_partials),
+                  ts, stamp, tr, tc, *(hot.args(True) if hot else NO_HOT_BIAS), 1 if self.deterministic else 0, keep, dseed,
+                  *self._bn_args(), ptr(self._g_bn[0]), ptr(self._g_bn[1]), self.BN_EPS, self.BN_DECAY, ptr(self._bn_ws),
+                  self._bn_ws.numel(), cur_stream())
+        self._finish_step(hot, True, self._apply_bias)
+        self._opt.apply_dense("bn_fm/gamma", self.weights["bn_fm/gamma"], self._g_bn[0], 0.0, None)
+        self._opt.apply_dense("bn_fm/beta", self.weights["bn_fm/beta"], self._g_bn[1], 0.0, None)
 
     def _fused_segments(self):
         n_v, n_b, _ = self._arena_layout

@@ -139,6 +139,33 @@ int hhfm_fm_fwd_bwd_sqloss_dropout(const int32_t* row_ptr, const int32_t* col, c
                            int32_t* touched_count, const int32_t* hot_slot, float* ghot, float* ghot_bias,
                            int32_t n_rep, int32_t n_hot, int32_t deterministic, float keep, uint64_t drop_seed, hhfm_stream_t stream);
 
+/* FM training step with batch normalisation of the interaction vector (FM.py:111-112, batch_norm=1; tf.contrib.layers
+ * .batch_norm with center, scale, is_training=True), before the dropout of the call above:
+ *   x = 0.5 (S^2 - sum_f e_f^2), y = gamma (x - mu) / sqrt(var + eps) + beta, out = sum_k y / keep * m + sum_f b[x_f] + b0,
+ * mu and var (biased) over the batch per column.  In the same step moving_mean -= (1 - decay) (moving_mean - mu) and
+ * moving_var -= (1 - decay) (moving_var - var * B / max(B - 1, 1)).  dgamma / dbeta [K] are WRITTEN (not accumulated);
+ * gV, gbias, gb0, the loss partials, the hot replicas and the touched-row list as in hhfm_fm_fwd_bwd_sqloss.
+ * Fixed-width rows only (row_ptr = val = NULL) and interaction = 0; gamma, beta, moving_mean, moving_var 16-byte aligned.
+ * eps > 0 (the reference: 1e-3), decay in [0, 1) (0.9).  workspace: hhfm_workspace_bytes_fm_bn(B, K) bytes, caller-owned,
+ * 16-byte aligned.  Batch statistics, loss, dgamma, dbeta, gb0 and the moving statistics are fixed-order reductions
+ * (bit-identical from run to run); deterministic = 1 also makes the row scatter one warp in program order. */
+int hhfm_fm_bn_fwd_bwd_sqloss(const int32_t* row_ptr, const int32_t* col, const float* val, int64_t B, int64_t F,
+                              const float* V, const float* bias, const float* b0, int64_t M, int64_t K,
+                              int32_t interaction, const float* labels, float* out, float* gV, float* gbias, float* gb0,
+                              float* loss_partials, int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows,
+                              int32_t* touched_count, const int32_t* hot_slot, float* ghot, float* ghot_bias,
+                              int32_t n_rep, int32_t n_hot, int32_t deterministic, float keep, uint64_t drop_seed,
+                              const float* gamma, const float* beta, float* moving_mean, float* moving_var, float* dgamma,
+                              float* dbeta, float eps, float decay, void* workspace, int64_t workspace_bytes,
+                              hhfm_stream_t stream);
+/* Bytes of the workspace of hhfm_fm_bn_fwd_bwd_sqloss for a batch of B samples and K factors; -1 for bad sizes. */
+int64_t hhfm_workspace_bytes_fm_bn(int64_t B, int64_t K);
+/* The batch-normalised FM forward at evaluation (train_phase=False): the moving statistics, no dropout.
+ * out[s] = sum_k (gamma (x - moving_mean) / sqrt(moving_var + eps) + beta) + sum_f b[x_f] + b0, fixed-width rows. */
+int hhfm_fm_bn_fwd(const int32_t* col, int64_t B, int64_t F, const float* V, const float* bias, const float* b0, int64_t M,
+                   int64_t K, const float* gamma, const float* beta, const float* moving_mean, const float* moving_var,
+                   float eps, float* out, hhfm_stream_t stream);
+
 /* K14  single-touch rows.  At the scaled shapes (M = 10^7, SURVEY.md 8d) ~40 % of the rows a step touches are referenced by
  * exactly one sample.  hhfm_count_refs counts the references of a step's id matrix (ref_count[M] is cleared first, ids < 0
  * are padding); the *_st variants of the training passes then apply the optimizer step of a row with ref_count == 1 on the
