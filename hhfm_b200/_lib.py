@@ -25,13 +25,10 @@ SIGNATURES = {
                                vp, vp, vp, vp, i32, i32, i32, vp],
     "hhfm_fm_fwd_bwd_sqloss_dropout": [vp, vp, vp, i64, i64, vp, vp, vp, i64, i64, i32, vp, vp, vp, vp, vp, vp, vp, i32, vp,
                                        vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64, vp],
-    "hhfm_fm_fwd_bwd_sqloss_st": [vp, vp, vp, i64, i64, vp, vp, vp, i64, i64, i32, vp, vp, vp, vp, vp, vp, vp, i32, vp,
-                                  vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64, vp, vp],
     "hhfm_fm_bn_fwd_bwd_sqloss": [vp, vp, vp, i64, i64, vp, vp, vp, i64, i64, i32, vp, vp, vp, vp, vp, vp, vp, i32, vp,
                                   vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64, vp, vp, vp, vp, vp, vp, f32, f32, vp, i64,
                                   vp],
     "hhfm_fm_bn_fwd": [vp, i64, i64, vp, vp, vp, i64, i64, vp, vp, vp, vp, f32, vp, vp],
-    "hhfm_count_refs": [vp, i64, i64, i64, i64, vp, vp],
     "hhfm_fm_bwd": [vp, vp, vp, i64, i64, vp, i64, i64, i32, vp, vp, vp, vp, i32, vp],
     "hhfm_afm_fwd": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, vp, vp],
     "hhfm_afm_fwd_bwd_sqloss": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp,
@@ -54,8 +51,6 @@ SIGNATURES = {
     "hhfm_pairrank_fwd": [vp, i64, i64, i32, i32, i32, i32, i32, i32, vp, i64, i64, vp, vp, vp],
     "hhfm_pairrank_fwd_bwd": [vp, i64, i64, i32, i32, i32, i32, i32, i32, vp, i64, i64, vp, vp, vp, vp, vp, i32, vp,
                               vp, vp, vp, i32, i32, i32, vp],
-    "hhfm_pairrank_fwd_bwd_st": [vp, i64, i64, i32, i32, i32, i32, i32, i32, vp, i64, i64, vp, vp, vp, vp, vp, i32, vp,
-                                 vp, vp, vp, i32, i32, i32, vp, vp],
     "hhfm_pairrank_bwd": [vp, i64, i64, i32, i32, i32, i32, i32, i32, vp, i64, i64, vp, vp, vp, i32, vp],
     "hhfm_pool_groups_attach": [vp, i64, i64, i32, i64, vp, vp, vp, vp],
     "hhfm_pool_groups_detach": [vp, i64],

@@ -8,7 +8,6 @@
 #include <stdlib.h>
 
 #include "common.cuh"
-#include "opt_elem.cuh"
 #include "staged.cuh"
 
 namespace hhfm {
@@ -39,7 +38,6 @@ struct FmArgs {
   HotPlan hot;
   float keep;            // dropout keep probability of the interaction layer (FM.py:114, MF.py:87); 1 = off
   uint64_t drop_seed;
-  SingleTouch st1;       // in-place optimizer step of single-touch rows (staged kernel only); ref_count == nullptr: off
 };
 
 enum { FM_FWD = 0, FM_TRAIN = 1, FM_BWD = 2 };
@@ -375,11 +373,11 @@ static int dispatch_fm_fixed(const FmArgs& a, cudaStream_t st) {
 constexpr int kStagedWarps = 10;
 constexpr int kStagedMaxF = 16;
 
-// shared memory per warp: NS row stages [F][K] floats, then (NS+PD) id slots, NS bias slots, NS hot-slot slots, NS
-// reference-count slots of kStagedMaxF words each, then NS mbarriers.
+// shared memory per warp: NS row stages [F][K] floats, then (NS+PD) id slots, NS bias slots, NS hot-slot slots of
+// kStagedMaxF words each, then NS mbarriers.
 __host__ __device__ inline size_t staged_warp_bytes(int NS, int F, int K) {
   const int PD = NS - 1;
-  const size_t b = (size_t)NS * F * K * 4 + (size_t)((NS + PD) + 3 * NS) * kStagedMaxF * 4 + (size_t)NS * 8;
+  const size_t b = (size_t)NS * F * K * 4 + (size_t)((NS + PD) + 2 * NS) * kStagedMaxF * 4 + (size_t)NS * 8;
   return (b + 127) / 128 * 128;
 }
 
@@ -397,8 +395,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fm_train_staged_kernel(const FmArg
   int* idring = reinterpret_cast<int*>(base + (size_t)NS * F * K * 4);             // [RI][16]
   float* biasbuf = reinterpret_cast<float*>(idring + RI * kStagedMaxF);            // [NS][16]
   int* slotbuf = reinterpret_cast<int*>(biasbuf + NS * kStagedMaxF);               // [NS][16]
-  int* cntbuf = slotbuf + NS * kStagedMaxF;                                        // [NS][16]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(cntbuf + NS * kStagedMaxF);         // [NS]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(slotbuf + NS * kStagedMaxF);        // [NS]
   if (lane == 0) {
 #pragma unroll
     for (int i = 0; i < NS; i++) mbar_init1(bars + i);
@@ -417,10 +414,6 @@ __global__ void __launch_bounds__(NW * 32, 1) fm_train_staged_kernel(const FmArg
   const float b0 = a.b0 ? __ldg(a.b0) : 0.f;
   const int rep = a.hot.slot ? (int)(warp_g % a.hot.n_rep) : 0;
   float loss_acc = 0.f, g0_acc = 0.f;
-  PendingRows pend;
-  pend.n = 0;
-  int pb_id = -1;
-  float pb_w = 0.f, pb_acc = 0.f, pb_g = 0.f;
 
   for (int64_t t = 0; t < n + PD + NS - 1; t++) {
     // (A) ids of sample t
@@ -441,7 +434,6 @@ __global__ void __launch_bounds__(NW * 32, 1) fm_train_staged_kernel(const FmArg
         bulk_row(rows + ((size_t)st * F + lane) * K, a.V + (size_t)id * K, row_bytes, bars + st);
         if (a.bias) ldgsts4(biasbuf + st * kStagedMaxF + lane, a.bias + id);
         if (a.hot.slot) ldgsts4(slotbuf + st * kStagedMaxF + lane, a.hot.slot + id);
-        if (a.st1.ref_count) ldgsts4(cntbuf + st * kStagedMaxF + lane, a.st1.ref_count + id);
       }
     }
     ldgsts_commit();
@@ -453,44 +445,6 @@ __global__ void __launch_bounds__(NW * 32, 1) fm_train_staged_kernel(const FmArg
       mbar_wait_parity(bars + st, (uint32_t)((c / NS) & 1));
       const float4* r4 = reinterpret_cast<const float4*>(rows + (size_t)st * F * K);
       const int* ids = idring + (c % RI) * kStagedMaxF;
-      // single-touch rows (K14): first the pending in-place steps of the previous sample (their accumulator loads have
-      // landed by now), then this sample's rows -- at most kSingleTouchCap -- whose accumulator loads go out here
-      unsigned smask = 0u;
-      if (a.st1.ref_count) {
-        pending_flush(a.st1, pend, K, kv, lane);
-        if (pb_id >= 0) {
-          const OptP p{a.st1.lr, 0.f, 0.f, 0.f, 0.f};
-          float dummy = 0.f;
-          if (a.st1.kind == HHFM_OPT_ADAGRAD) {
-            opt_elem<HHFM_OPT_ADAGRAD>(pb_w, pb_acc, dummy, pb_g, p);
-            a.st1.bias_acc[pb_id] = pb_acc;
-          } else {
-            opt_elem<HHFM_OPT_SGD>(pb_w, pb_acc, dummy, pb_g, p);
-          }
-          a.st1.bias[pb_id] = pb_w;
-          pb_id = -1;
-        }
-        const bool single = lane < F && cntbuf[st * kStagedMaxF + lane] == 1 &&
-                            !(a.hot.slot && slotbuf[st * kStagedMaxF + lane] >= 0);
-        unsigned rest = __ballot_sync(0xffffffffu, single);
-#pragma unroll
-        for (int q = 0; q < kSingleTouchCap; q++) {
-          if (rest) {
-            const int f = __ffs((int)rest) - 1;
-            rest &= rest - 1;
-            smask |= 1u << f;
-            pend.id[q] = ids[f];
-            if (a.st1.kind == HHFM_OPT_ADAGRAD && lane < kv)
-              pend.a[q] = reinterpret_cast<const float4*>(a.st1.acc + (size_t)ids[f] * K)[lane];
-            pend.n = q + 1;
-          }
-        }
-        if (((smask >> lane) & 1u) && a.gbias && a.st1.bias) {
-          pb_id = ids[lane];
-          pb_w = biasbuf[st * kStagedMaxF + lane];
-          if (a.st1.kind == HHFM_OPT_ADAGRAD) pb_acc = a.st1.bias_acc[pb_id];
-        }
-      }
       float4 S[4], Q[4];
 #pragma unroll
       for (int i = 0; i < 4; i++) { S[i] = f4_zero(); Q[i] = f4_zero(); }
@@ -519,23 +473,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fm_train_staged_kernel(const FmArg
         g0_acc += g;
         if (a.out) a.out[s] = out;
       }
-      {
-        unsigned rest = smask;
-#pragma unroll
-        for (int q = 0; q < kSingleTouchCap; q++) {           // in place, applied at the warp's next sample: keep w and the gradient
-          if (rest) {
-            const int f = __ffs((int)rest) - 1;
-            rest &= rest - 1;
-            if (lane < kv) {
-              const float4 e = r4[f * kv + lane];
-              pend.w[q] = e;
-              pend.g[q] = f4_scale(f4_sub(S[0], e), g);
-            }
-          }
-        }
-      }
       for (int f = 0; f < F; f++) {
-        if ((smask >> f) & 1u) continue;
         const int id = ids[f];
         const int slot = a.hot.slot ? slotbuf[st * kStagedMaxF + f] : -1;
         float* dst = (slot >= 0) ? a.hot.ghot + ((size_t)rep * a.hot.n_hot + slot) * K : a.gV + (size_t)id * K;
@@ -547,35 +485,17 @@ __global__ void __launch_bounds__(NW * 32, 1) fm_train_staged_kernel(const FmArg
       }
       if (lane < F) {
         const int id = ids[lane];
-        if ((smask >> lane) & 1u) {
-          pb_g = g;                                           // the row's bias element goes in place as well (next sample)
-        } else {
-          if (a.gbias) {
-            const int slot = a.hot.slot ? slotbuf[st * kStagedMaxF + lane] : -1;
-            float* p = (slot >= 0 && a.hot.ghot_bias != nullptr) ? a.hot.ghot_bias + (size_t)rep * a.hot.n_hot + slot : a.gbias + id;
-            atomicAdd(p, g);
-          }
-          if (a.touch_stamp) a.touch_stamp[id] = a.stamp;     // compacted into the list by touched_compact_kernel
+        if (a.gbias) {
+          const int slot = a.hot.slot ? slotbuf[st * kStagedMaxF + lane] : -1;
+          float* p = (slot >= 0 && a.hot.ghot_bias != nullptr) ? a.hot.ghot_bias + (size_t)rep * a.hot.n_hot + slot : a.gbias + id;
+          atomicAdd(p, g);
         }
+        if (a.touch_stamp) a.touch_stamp[id] = a.stamp;       // compacted into the list by touched_compact_kernel
       }
       __syncwarp();     // every lane is done with this stage before the next iteration re-arms it
     }
   }
   ldgsts_wait<0>();
-  if (a.st1.ref_count) {
-    pending_flush(a.st1, pend, K, kv, lane);
-    if (pb_id >= 0) {
-      const OptP p{a.st1.lr, 0.f, 0.f, 0.f, 0.f};
-      float dummy = 0.f;
-      if (a.st1.kind == HHFM_OPT_ADAGRAD) {
-        opt_elem<HHFM_OPT_ADAGRAD>(pb_w, pb_acc, dummy, pb_g, p);
-        a.st1.bias_acc[pb_id] = pb_acc;
-      } else {
-        opt_elem<HHFM_OPT_SGD>(pb_w, pb_acc, dummy, pb_g, p);
-      }
-      a.st1.bias[pb_id] = pb_w;
-    }
-  }
   const float bl = block_sum(loss_acc, scratch);
   write_partial(a.loss_partials, bl);
   if (a.gb0 != nullptr) {
@@ -674,8 +594,6 @@ static int dispatch_fm_staged(const FmArgs& a, int64_t M, cudaStream_t st) {
   const int force = env ? (env[0] == '1' ? 1 : 0) : 2;
   if (force == 0) return HHFM_ERR_UNSUPPORTED;
   if (force == 2 && (size_t)M * a.K * 4 < ((size_t)96 << 20)) return HHFM_ERR_UNSUPPORTED;
-  FmArgs b = a;
-  if (b.K > 128) b.st1 = SingleTouch{};                    // the deferred in-place step keeps one float4 chunk per lane
   const size_t cap = (size_t)224 * 1024;
   // measured at the c5 shape (F = 10, K = 128): 10 warps x 4 stages 5.95 ms per step, 10 x 3 5.91, 11 x 3 5.64, 12 x 3 5.74,
   // 13 x 3 5.81, 14 x 3 5.88, 16 x 2 5.92 -> eleven warps with three stages each when that fits
@@ -694,7 +612,7 @@ static int dispatch_fm_staged(const FmArgs& a, int64_t M, cudaStream_t st) {
 #define HHFM_LAUNCH_STAGED(NS_, NW_)                                                                                              \
   do {                                                                                                                            \
     e = cudaFuncSetAttribute(fm_train_staged_kernel<NS_, NW_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
-    if (e == cudaSuccess) fm_train_staged_kernel<NS_, NW_><<<grid, NW_ * 32, smem, st>>>(b);                                      \
+    if (e == cudaSuccess) fm_train_staged_kernel<NS_, NW_><<<grid, NW_ * 32, smem, st>>>(a);                                      \
   } while (0)
   if (nw == kStagedWarps) {
     if (ns == 4) HHFM_LAUNCH_STAGED(4, kStagedWarps);
@@ -761,33 +679,6 @@ static int dispatch_fm_train_dropout(const FmArgs& a, int deterministic, cudaStr
   return HHFM_ERR_UNSUPPORTED;
 }
 
-// ref_count[id] += 1 for every id of the [n_rows, n_cols] block of a row-major id matrix with row stride `stride` (K14)
-__global__ void __launch_bounds__(256) count_refs_kernel(const int32_t* __restrict__ ids, int64_t n_rows, int64_t stride, int n_cols,
-                                                         int32_t* __restrict__ ref_count) {
-  const int64_t n = n_rows * n_cols;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t r = i / n_cols;
-    const int id = __ldg(ids + r * stride + (i - r * n_cols));
-    if (id >= 0) atomicAdd(ref_count + id, 1);
-  }
-}
-
-int single_touch_from_abi(const void* abi_plan, const float* V, int64_t K, SingleTouch* out) {
-  *out = SingleTouch{};
-  if (abi_plan == nullptr) return HHFM_OK;
-  const hhfm_single_touch* p = reinterpret_cast<const hhfm_single_touch*>(abi_plan);
-  if (p->ref_count == nullptr) return HHFM_OK;
-  HHFM_REQUIRE(p->V == V, "single-touch plan: V must be the table the pass reads");
-  HHFM_REQUIRE(p->opt_kind == HHFM_OPT_ADAGRAD || p->opt_kind == HHFM_OPT_SGD,
-               "single-touch plan: only Adagrad and SGD leave untouched rows in place (opt_kind=%d)", (int)p->opt_kind);
-  HHFM_REQUIRE(p->opt_kind != HHFM_OPT_ADAGRAD || p->acc != nullptr, "single-touch plan: Adagrad needs the accumulator");
-  HHFM_REQUIRE((((uintptr_t)p->V | (uintptr_t)p->acc) & 15) == 0 && K % 4 == 0, "single-touch plan: V / acc must be 16-byte aligned");
-  HHFM_REQUIRE(p->bias == nullptr || p->opt_kind != HHFM_OPT_ADAGRAD || p->bias_acc != nullptr,
-               "single-touch plan: bias needs its accumulator");
-  *out = SingleTouch{p->ref_count, p->V, p->acc, p->bias, p->bias_acc, p->lr, (int)p->opt_kind};
-  return HHFM_OK;
-}
-
 static int check_common(int64_t B, int64_t F, const void* col, const void* V, int64_t M, int64_t K, int interaction,
                         const void* row_ptr) {
   HHFM_REQUIRE(B >= 0 && M > 0, "fm: bad sizes B=%lld M=%lld", (long long)B, (long long)M);
@@ -817,38 +708,15 @@ extern "C" int hhfm_fm_fwd(const int32_t* row_ptr, const int32_t* col, const flo
   return dispatch_fm<FM_FWD>(a, 0, (cudaStream_t)stream);
 }
 
-extern "C" int hhfm_count_refs(const int32_t* ids, int64_t n_rows, int64_t stride, int64_t n_cols, int64_t M, int32_t* ref_count,
-                               hhfm_stream_t stream) {
-  HHFM_REQUIRE(ids && ref_count && M > 0, "count_refs: NULL argument");
-  HHFM_REQUIRE(n_rows >= 0 && n_cols >= 0 && n_cols <= stride, "count_refs: bad shape rows=%lld cols=%lld stride=%lld",
-               (long long)n_rows, (long long)n_cols, (long long)stride);
-  cudaStream_t st = (cudaStream_t)stream;
-  cudaMemsetAsync(ref_count, 0, (size_t)M * sizeof(int32_t), st);
-  if (n_rows * n_cols == 0) return check_launch("count_refs memset");
-  int64_t blocks = (n_rows * n_cols + 255) / 256;
-  const int64_t cap = (int64_t)sm_count() * 16;
-  if (blocks > cap) blocks = cap;
-  count_refs_kernel<<<(int)blocks, 256, 0, st>>>(ids, n_rows, stride, (int)n_cols, ref_count);
-  return check_launch("count_refs_kernel");
-}
-
-extern "C" int hhfm_fm_fwd_bwd_sqloss_st(const int32_t* row_ptr, const int32_t* col, const float* val, int64_t B,
+extern "C" int hhfm_fm_fwd_bwd_sqloss_dropout(const int32_t* row_ptr, const int32_t* col, const float* val, int64_t B,
                                       int64_t F, const float* V, const float* bias, const float* b0, int64_t M,
                                       int64_t K, int32_t interaction, const float* labels, float* out, float* gV,
                                       float* gbias, float* gb0, float* loss_partials, int32_t* touch_stamp,
                                       int32_t stamp, int32_t* touched_rows, int32_t* touched_count,
                                       const int32_t* hot_slot, float* ghot, float* ghot_bias, int32_t n_rep,
-                                      int32_t n_hot, int32_t deterministic, float keep, uint64_t drop_seed,
-                                      const hhfm_single_touch* plan, hhfm_stream_t stream) {
+                                      int32_t n_hot, int32_t deterministic, float keep, uint64_t drop_seed, hhfm_stream_t stream) {
   int rc = check_common(B, F, col, V, M, K, interaction, row_ptr);
   if (rc) return rc;
-  SingleTouch st1;
-  if ((rc = single_touch_from_abi(plan, V, K, &st1))) return rc;
-  if (st1.ref_count != nullptr) {
-    HHFM_REQUIRE(touch_stamp != nullptr, "fm_fwd_bwd_sqloss_st: the plan needs touched-row tracking for the other rows");
-    HHFM_REQUIRE(gbias == nullptr || st1.bias != nullptr, "fm_fwd_bwd_sqloss_st: the model has a bias gradient, the plan no bias");
-    HHFM_REQUIRE(st1.bias == nullptr || st1.bias == bias, "fm_fwd_bwd_sqloss_st: plan.bias must be the bias the pass reads");
-  }
   HHFM_REQUIRE(!hot_slot || (ghot && n_rep >= 1 && n_hot >= 1), "fm_fwd_bwd_sqloss: hot_slot needs ghot, n_rep, n_hot");
   HHFM_REQUIRE(labels && gV && loss_partials, "fm_fwd_bwd_sqloss: labels, gV and loss_partials are required");
   HHFM_REQUIRE(B > 0, "fm_fwd_bwd_sqloss: empty batch");
@@ -863,7 +731,6 @@ extern "C" int hhfm_fm_fwd_bwd_sqloss_st(const int32_t* row_ptr, const int32_t* 
   HHFM_REQUIRE(keep > 0.f && keep <= 1.f, "fm_fwd_bwd_sqloss: dropout keep must be in (0, 1]");
   a.keep = keep;
   a.drop_seed = drop_seed;
-  a.st1 = st1;
   if (keep < 1.f) return dispatch_fm_train_dropout(a, deterministic, (cudaStream_t)stream);
   if (!deterministic) {
     rc = dispatch_fm_staged(a, M, (cudaStream_t)stream);
@@ -872,18 +739,6 @@ extern "C" int hhfm_fm_fwd_bwd_sqloss_st(const int32_t* row_ptr, const int32_t* 
     if (rc != HHFM_ERR_UNSUPPORTED) return rc;
   }
   return dispatch_fm<FM_TRAIN>(a, deterministic, (cudaStream_t)stream);
-}
-
-extern "C" int hhfm_fm_fwd_bwd_sqloss_dropout(const int32_t* row_ptr, const int32_t* col, const float* val, int64_t B,
-                                      int64_t F, const float* V, const float* bias, const float* b0, int64_t M,
-                                      int64_t K, int32_t interaction, const float* labels, float* out, float* gV,
-                                      float* gbias, float* gb0, float* loss_partials, int32_t* touch_stamp,
-                                      int32_t stamp, int32_t* touched_rows, int32_t* touched_count,
-                                      const int32_t* hot_slot, float* ghot, float* ghot_bias, int32_t n_rep,
-                                      int32_t n_hot, int32_t deterministic, float keep, uint64_t drop_seed, hhfm_stream_t stream) {
-  return hhfm_fm_fwd_bwd_sqloss_st(row_ptr, col, val, B, F, V, bias, b0, M, K, interaction, labels, out, gV, gbias, gb0,
-                                   loss_partials, touch_stamp, stamp, touched_rows, touched_count, hot_slot, ghot, ghot_bias,
-                                   n_rep, n_hot, deterministic, keep, drop_seed, nullptr, stream);
 }
 
 extern "C" int hhfm_fm_fwd_bwd_sqloss(const int32_t* row_ptr, const int32_t* col, const float* val, int64_t B,

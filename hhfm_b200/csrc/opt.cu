@@ -4,10 +4,38 @@
 // ApplyAdam with lr_t folded by the caller, ApplyMomentum `accum = accum*mu + g; var -= lr*accum`.
 // All kernels are pure streaming float4 passes (HBM-bound): read g,w,state -> write w,state,(g=0).
 #include "common.cuh"
-#include "opt_elem.cuh"
 #include "staged.cuh"
 
 namespace hhfm {
+
+struct OptP {
+  float lr, lamda, p1, p2, p3;   // adam: p1=beta1 p2=beta2 p3=eps ; momentum: p1=mu
+};
+
+template <int KIND>
+__device__ __forceinline__ void opt_elem(float& w, float& s1, float& s2, float g, const OptP& p) {
+  if (KIND == HHFM_OPT_ADAGRAD) {
+    s1 = fmaf(g, g, s1);                                // explicit contractions: the same bits as p2p.cu::opt_elem2
+    w = w - p.lr * g / sqrtf(s1);
+  } else if (KIND == HHFM_OPT_ADAM) {
+    s1 = fmaf(p.p1, s1, (1.f - p.p1) * g);
+    s2 = fmaf(p.p2, s2, (1.f - p.p2) * (g * g));
+    w = w - p.lr * s1 / (sqrtf(s2) + p.p3);
+  } else if (KIND == HHFM_OPT_MOMENTUM) {
+    s1 = fmaf(s1, p.p1, g);
+    w = fmaf(-p.lr, s1, w);
+  } else {
+    w = fmaf(-p.lr, g, w);
+  }
+}
+
+template <int KIND>
+__device__ __forceinline__ void opt_vec4(float4& w, float4& s1, float4& s2, float4 g, const OptP& p) {
+  opt_elem<KIND>(w.x, s1.x, s2.x, g.x, p);
+  opt_elem<KIND>(w.y, s1.y, s2.y, g.y, p);
+  opt_elem<KIND>(w.z, s1.z, s2.z, g.z, p);
+  opt_elem<KIND>(w.w, s1.w, s2.w, g.w, p);
+}
 
 // dense: n elements, g_eff = g + lamda*w.  Handles n % 4 != 0 with a scalar tail (bias vectors, scalars).
 template <int KIND>

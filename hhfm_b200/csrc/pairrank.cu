@@ -10,7 +10,6 @@
 #include <vector>
 
 #include "common.cuh"
-#include "opt_elem.cuh"
 #include "staged.cuh"
 
 namespace hhfm {
@@ -35,7 +34,6 @@ struct PrArgs {
   int32_t* touched_count;
   int groups_active;
   HotPlan hot;
-  SingleTouch st1;       // in-place optimizer step of single-touch rows (staged kernel only); ref_count == nullptr: off
 };
 
 enum { PR_FWD = 0, PR_TRAIN = 1, PR_BWD = 2 };
@@ -672,7 +670,7 @@ static int dispatch_pr_grouped(const PrArgs& a, int64_t M, cudaStream_t st, int*
   if (!pool_groups_enabled()) return 1;
   const bool all_sum = (a.n_ctx == 0 || a.pc == HHFM_POOL_SUM) && (a.n_time == 0 || a.pt == HHFM_POOL_SUM) &&
                        ((a.n_ctx == 0 && a.n_time == 0) || a.pf == HHFM_POOL_SUM);
-  if (!all_sum || a.touch_stamp || a.pos_out || a.neg_out || a.st1.ref_count || a.n_neg != 10) return 1;
+  if (!all_sum || a.touch_stamp || a.pos_out || a.neg_out || a.n_neg != 10) return 1;
   if (a.K != 32 && a.K != 64 && a.K != 128) return 1;
   int dev = -1;
   cudaGetDevice(&dev);
@@ -726,9 +724,11 @@ static int dispatch_pr_grouped(const PrArgs& a, int64_t M, cudaStream_t st, int*
 constexpr int kPrStagedWarps = 10;
 constexpr int kPrMaxW = 32;
 
+// shared memory per warp: NS row stages [W][K] floats, then (NS+PD) id slots and NS hot-slot slots of kPrMaxW words each,
+// then NS mbarriers.
 __host__ __device__ inline size_t pr_staged_warp_bytes(int NS, int W, int K) {
   const int PD = NS - 1;
-  const size_t b = (size_t)NS * W * K * 4 + (size_t)((NS + PD) + 2 * NS) * kPrMaxW * 4 + (size_t)NS * 8;
+  const size_t b = (size_t)NS * W * K * 4 + (size_t)((NS + PD) + NS) * kPrMaxW * 4 + (size_t)NS * 8;
   return (b + 127) / 128 * 128;
 }
 
@@ -747,8 +747,7 @@ __global__ void __launch_bounds__(NW * 32, 1) pairrank_sum_train_staged_kernel(c
   float* rows = reinterpret_cast<float*>(base);                                   // [NS][W][K]
   int* idring = reinterpret_cast<int*>(base + (size_t)NS * W * K * 4);             // [RI][32]
   int* slotbuf = idring + RI * kPrMaxW;                                            // [NS][32]
-  int* cntbuf = slotbuf + NS * kPrMaxW;                                            // [NS][32] reference counts (single-touch plan)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(cntbuf + NS * kPrMaxW);             // [NS]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(slotbuf + NS * kPrMaxW);            // [NS]
   if (lane == 0) {
 #pragma unroll
     for (int i = 0; i < NS; i++) mbar_init1(bars + i);
@@ -765,8 +764,6 @@ __global__ void __launch_bounds__(NW * 32, 1) pairrank_sum_train_staged_kernel(c
   const int64_t n = s_end > s_beg ? s_end - s_beg : 0;
   const int rep = a.hot.slot ? (int)(warp_g % a.hot.n_rep) : 0;
   float loss_acc = 0.f;
-  PendingRows pend;
-  pend.n = 0;
 
   for (int64_t t = 0; t < n + PD + NS - 1; t++) {
     if (t < n && lane < W) ldgsts4(idring + (t % RI) * kPrMaxW + lane, a.idx + (s_beg + t) * a.stride + lane);
@@ -781,7 +778,6 @@ __global__ void __launch_bounds__(NW * 32, 1) pairrank_sum_train_staged_kernel(c
         const int id = idring[(j % RI) * kPrMaxW + lane];
         bulk_row(rows + ((size_t)st * W + lane) * K, a.V + (size_t)id * K, row_bytes, bars + st);
         if (a.hot.slot) ldgsts4(slotbuf + st * kPrMaxW + lane, a.hot.slot + id);
-        if (a.st1.ref_count && lane < 2 + NP) ldgsts4(cntbuf + st * kPrMaxW + lane, a.st1.ref_count + id);
       }
     }
     ldgsts_commit();
@@ -792,26 +788,6 @@ __global__ void __launch_bounds__(NW * 32, 1) pairrank_sum_train_staged_kernel(c
       const float4* r4 = reinterpret_cast<const float4*>(rows + (size_t)st * W * K);
       const int* ids = idring + (c % RI) * kPrMaxW;
       const int* slots = slotbuf + st * kPrMaxW;
-      // single-touch rows (K14) among user / item+ / context rows: first the pending in-place steps of the previous sample
-      // (their accumulator loads have landed by now), then this sample's rows, whose accumulator loads go out here
-      unsigned smask = 0u;
-      if (a.st1.ref_count) {
-        pending_flush(a.st1, pend, K, kv, lane);
-        const bool single = lane < 2 + NP && cntbuf[st * kPrMaxW + lane] == 1 && !(a.hot.slot && slots[lane] >= 0);
-        unsigned rest = __ballot_sync(0xffffffffu, single);
-#pragma unroll
-        for (int q = 0; q < kSingleTouchCap; q++) {
-          if (rest) {
-            const int w = __ffs((int)rest) - 1;
-            rest &= rest - 1;
-            smask |= 1u << w;
-            pend.id[q] = ids[w];
-            if (a.st1.kind == HHFM_OPT_ADAGRAD && lane < kv)
-              pend.a[q] = reinterpret_cast<const float4*>(a.st1.acc + (size_t)ids[w] * K)[lane];
-            pend.n = q + 1;
-          }
-        }
-      }
       float4 hyb[4];
 #pragma unroll
       for (int i = 0; i < 4; i++) {
@@ -848,27 +824,15 @@ __global__ void __launch_bounds__(NW * 32, 1) pairrank_sum_train_staged_kernel(c
         const int slot = a.hot.slot ? slots[w] : -1;
         return (slot >= 0) ? a.hot.ghot + ((size_t)rep * a.hot.n_hot + slot) * K : a.gV + (size_t)ids[w] * K;
       };
-      // gradient row of operand w -> its line in the arena / hot replica, or (single-touch row) the pending in-place step
-      auto slot_of = [&](int w) { return __popc(smask & ((1u << w) - 1u)); };      // index of w among the in-place rows
-      auto keep_pending = [&](int w, float4 e, float4 gr) {
-        const int q = slot_of(w);
-#pragma unroll
-        for (int qq = 0; qq < kSingleTouchCap; qq++)
-          if (qq == q) { pend.w[qq] = e; pend.g[qq] = gr; }
-      };
       float4 dh[4];
       {
-        const bool inplace = (smask >> 1) & 1u;
         float* d = dst_of(1);
 #pragma unroll
         for (int i = 0; i < 4; i++) {
           const int cc = lane + 32 * i;
           if (cc < kv) {
-            const float4 e = r4[kv + cc];
-            dh[i] = f4_scale(e, gp);
-            const float4 gr = f4_scale(hyb[i], gp);
-            if (inplace) keep_pending(1, e, gr);              // kv <= 32 with a plan: i == 0 only
-            else red_add_v4(d + 4 * cc, gr);
+            dh[i] = f4_scale(r4[kv + cc], gp);
+            red_add_v4(d + 4 * cc, f4_scale(hyb[i], gp));
           }
         }
       }
@@ -889,10 +853,6 @@ __global__ void __launch_bounds__(NW * 32, 1) pairrank_sum_train_staged_kernel(c
       }
       for (int w = 0; w < 2 + NP; w++) {
         if (w == 1) continue;
-        if ((smask >> w) & 1u) {
-          if (lane < kv) keep_pending(w, r4[w * kv + lane], dh[0]);
-          continue;
-        }
         float* d = dst_of(w);
 #pragma unroll
         for (int i = 0; i < 4; i++) {
@@ -901,23 +861,20 @@ __global__ void __launch_bounds__(NW * 32, 1) pairrank_sum_train_staged_kernel(c
         }
       }
       if (a.touch_stamp && lane < W) {
-        const bool touched = ((lane < 2 + NP) && !((smask >> lane) & 1u)) || (lane >= 2 + NP && ((tie >> (lane - 2 - NP)) & 1u));
+        const bool touched = (lane < 2 + NP) || ((tie >> (lane - 2 - NP)) & 1u);
         if (touched) a.touch_stamp[ids[lane]] = a.stamp;       // compacted into the list afterwards
       }
       __syncwarp();     // every lane is done with this stage before the next iteration re-arms it
     }
   }
   ldgsts_wait<0>();
-  if (a.st1.ref_count) pending_flush(a.st1, pend, K, kv, lane);
   const float bl = block_sum(loss_acc, scratch);
   write_partial(a.loss_partials, bl);
 }
 
 // HHFM_ERR_UNSUPPORTED when the configuration is not covered or the table is small enough to live in L2 (the register
 // kernel wins there).  HHFM_PR_STAGED=0/1 forces the choice.
-static int dispatch_pr_staged(const PrArgs& a_in, int64_t M, cudaStream_t st) {
-  PrArgs a = a_in;
-  if (a.K > 128) a.st1 = SingleTouch{};                    // the deferred in-place step keeps one float4 chunk per lane
+static int dispatch_pr_staged(const PrArgs& a, int64_t M, cudaStream_t st) {
   const bool all_sum = (a.n_ctx == 0 || a.pc == HHFM_POOL_SUM) && (a.n_time == 0 || a.pt == HHFM_POOL_SUM) &&
                        ((a.n_ctx == 0 && a.n_time == 0) || a.pf == HHFM_POOL_SUM);
   if (!all_sum || a.pos_out || a.neg_out) return HHFM_ERR_UNSUPPORTED;
@@ -1050,24 +1007,8 @@ extern "C" int hhfm_pairrank_fwd_bwd(const int32_t* idx, int64_t B, int64_t stri
                                      float* loss_partials, int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows,
                                      int32_t* touched_count, const int32_t* hot_slot, float* ghot, int32_t n_rep,
                                      int32_t n_hot, int32_t deterministic, hhfm_stream_t stream) {
-  return hhfm_pairrank_fwd_bwd_st(idx, B, stride, n_ctx, n_time, n_neg, pool_ctx, pool_time, pool_stack, V, M, K, pos_out, neg_out,
-                                  gV, loss_partials, touch_stamp, stamp, touched_rows, touched_count, hot_slot, ghot, n_rep, n_hot,
-                                  deterministic, nullptr, stream);
-}
-
-extern "C" int hhfm_pairrank_fwd_bwd_st(const int32_t* idx, int64_t B, int64_t stride, int32_t n_ctx, int32_t n_time,
-                                        int32_t n_neg, int32_t pool_ctx, int32_t pool_time, int32_t pool_stack,
-                                        const float* V, int64_t M, int64_t K, float* pos_out, float* neg_out, float* gV,
-                                        float* loss_partials, int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows,
-                                        int32_t* touched_count, const int32_t* hot_slot, float* ghot, int32_t n_rep,
-                                        int32_t n_hot, int32_t deterministic, const hhfm_single_touch* plan,
-                                        hhfm_stream_t stream) {
   int rc = check_pr(idx, B, stride, n_ctx, n_time, n_neg, pool_ctx, pool_time, pool_stack, V, M, K);
   if (rc) return rc;
-  SingleTouch st1;
-  if ((rc = single_touch_from_abi(plan, V, K, &st1))) return rc;
-  HHFM_REQUIRE(st1.ref_count == nullptr || touch_stamp != nullptr,
-               "pairrank_fwd_bwd_st: the plan needs touched-row tracking for the other rows");
   HHFM_REQUIRE(!hot_slot || (ghot && n_rep >= 1 && n_hot >= 1), "pairrank_fwd_bwd: hot_slot needs ghot, n_rep, n_hot");
   HHFM_REQUIRE(B > 0 && n_neg >= 1, "pairrank_fwd_bwd: needs B > 0 and at least one negative");
   HHFM_REQUIRE(gV && loss_partials, "pairrank_fwd_bwd: gV and loss_partials are required");
@@ -1077,7 +1018,6 @@ extern "C" int hhfm_pairrank_fwd_bwd_st(const int32_t* idx, int64_t B, int64_t s
   a.pos_out = pos_out; a.neg_out = neg_out; a.gV = gV; a.loss_partials = loss_partials;
   a.touch_stamp = touch_stamp; a.stamp = stamp; a.touched_rows = touched_rows; a.touched_count = touched_count;
   a.hot = HotPlan{hot_slot, ghot, nullptr, n_rep, n_hot};
-  a.st1 = st1;
   if (!deterministic && hhfm_fast_path_enabled()) {
     int frc = dispatch_pr_staged(a, M, (cudaStream_t)stream);
     if (frc != HHFM_ERR_UNSUPPORTED) return frc;

@@ -324,12 +324,6 @@ class Optimizer:
             _lib.call("hhfm_opt_sgd_rows", ptr(w), ptr(g), ptr(rows), ptr(n_rows_dev), max_rows, K, self.lr, z, st)
 
 
-class SingleTouchPlan(C.Structure):
-    """hhfm_single_touch (include/hhfm_sm100.h, K14)."""
-    _fields_ = [("ref_count", C.c_void_p), ("V", C.c_void_p), ("acc", C.c_void_p), ("bias", C.c_void_p),
-                ("bias_acc", C.c_void_p), ("lr", C.c_float), ("opt_kind", C.c_int32)]
-
-
 class TouchTracker:
     """Per-step list of touched embedding rows, produced on the device by the scatter kernels."""
 

@@ -20,7 +20,7 @@ import torch
 
 from . import _lib
 from .engine import (NO_HOT, NO_HOT_BIAS, POOL_SUM, QUERY_FM, QUERY_HHFM, QUERY_USER, HotRows, Optimizer, PoolGroups,
-                     RecordUploader, SingleTouchPlan, Staging, TopN, TouchTracker, cur_stream, pack_records, ptr, require_cuda)
+                     RecordUploader, Staging, TopN, TouchTracker, cur_stream, pack_records, ptr, require_cuda)
 
 
 class PendingLoss:
@@ -139,37 +139,6 @@ class _Base:
         seed = (int(getattr(self, "random_seed", 2016)) * 0x9E3779B97F4A7C15 + self._opt.t) & 0xFFFFFFFFFFFFFFFF
         self._last_drop_seed = seed
         return seed
-
-    # ---- single-touch rows (include/hhfm_sm100.h K14) ---------------------------------------------------------------
-    def _single_touch(self, ids_dev, n_cols, with_bias, keep=1.0):
-        """The hhfm_single_touch plan of this step, or None.  Applicable when the staged (large-table) kernels run and the
-        rows optimizer is one under which untouched rows stay put: lamda == 0, Adagrad / SGD, one GPU, no dropout; the
-        reference counts of the step's ids are taken first (hhfm_count_refs)."""
-        # OFF by default: measured at the c5 shapes (profiles/r2_single_touch_summary.md) the reference count pass (0.5 ms: 10^7
-        # scattered 4-byte atomics run at the L2 atomic rate) and the 2 GB of extra traffic in the scatter kernel outweigh the
-        # 0.9 ms the rows optimizer saves.  HHFM_SINGLE_TOUCH=auto: on for large tables, =1: on for every table size (tests).
-        mode = os.environ.get("HHFM_SINGLE_TOUCH", "0")
-        if mode not in ("1", "auto"):
-            return None
-        if (self._lamda > 0 or self._opt.kind not in ("adagrad", "sgd") or self._dp_group is not None or self.deterministic
-                or keep < 1.0 or (mode != "1" and self._M * self._K * 4 < (96 << 20))):
-            return None
-        V = self.weights["feature_embeddings"]
-        if getattr(self, "_ref_count", None) is None:
-            self._ref_count = torch.empty(self._M, dtype=torch.int32, device=self.device)
-        B, stride = ids_dev.shape
-        _lib.call("hhfm_count_refs", ptr(ids_dev), B, stride, n_cols, self._M, ptr(self._ref_count), cur_stream())
-        plan = SingleTouchPlan()
-        plan.ref_count = ptr(self._ref_count)
-        plan.V = ptr(V)
-        plan.acc = ptr(self._opt.slots("feature_embeddings", V)[0]) if self._opt.kind == "adagrad" else None
-        bias = self.weights.get("feature_bias") if with_bias else None
-        if bias is not None:
-            plan.bias = ptr(bias)
-            plan.bias_acc = ptr(self._opt.slots("feature_bias", bias)[0]) if self._opt.kind == "adagrad" else None
-        plan.lr = self._opt.lr
-        plan.opt_kind = Optimizer.KIND_ID[self._opt.kind]
-        return plan
 
     # ---- lazy-exact dense L2 -----------------------------------------------------------------------------------------
     def _lazy(self):
@@ -684,16 +653,15 @@ class FM(_Base):
         if self._bn:
             self._fit_bn(idx, y, ts, stamp, tr, tc, hot, keep, dseed)
             return
-        plan = self._single_touch(idx, F, True, keep) if ts is not None else None
-        _lib.call("hhfm_fm_fwd_bwd_sqloss_st", None, ptr(idx), None, B, F, ptr(V), ptr(bias), ptr(self._b0), self._M,
+        _lib.call("hhfm_fm_fwd_bwd_sqloss_dropout", None, ptr(idx), None, B, F, ptr(V), ptr(bias), ptr(self._b0), self._M,
                   self._K, self.interaction, ptr(y), None, ptr(self._gV), ptr(self._gb), ptr(self._gb0),
                   ptr(self._loss_partials), ts, stamp, tr, tc, *(hot.args(True) if hot else NO_HOT_BIAS),
-                  1 if self.deterministic else 0, keep, dseed, C.addressof(plan) if plan is not None else None, cur_stream())
+                  1 if self.deterministic else 0, keep, dseed, cur_stream())
         self._finish_step(hot, True, self._apply_bias if bias is not None else None)
 
     def _fit_bn(self, idx, y, ts, stamp, tr, tc, hot, keep, dseed):
         """The step with batch normalisation (csrc/fm_bn.cu): V, feature_bias and the scalar bias go through the usual tail;
-        gamma and beta are dense variables without L2, stepped after it.  Single-touch rows (K14) stay off."""
+        gamma and beta are dense variables without L2, stepped after it."""
         B, F = idx.shape
         nbytes = int(_lib.load().hhfm_workspace_bytes_fm_bn(B, self._K))
         if self._bn_ws is None or self._bn_ws.numel() < nbytes:
@@ -849,11 +817,9 @@ class _PairRank(_Base):
             self._lazy_prepare(idx)                  # padding ids (-1) are skipped
         ts, stamp, tr, tc = self._touch_args()
         hot = self._hot_plan(idx, False)
-        plan = self._single_touch(idx, 2 + n_ctx + n_time + n_neg, False) if ts is not None else None
-        _lib.call("hhfm_pairrank_fwd_bwd_st", ptr(idx), B, stride, n_ctx, n_time, n_neg, pc, pt, pf, ptr(V), self._M,
+        _lib.call("hhfm_pairrank_fwd_bwd", ptr(idx), B, stride, n_ctx, n_time, n_neg, pc, pt, pf, ptr(V), self._M,
                   self._K, None, None, ptr(self._gV), ptr(self._loss_partials), ts, stamp, tr, tc,
-                  *(hot.args() if hot else NO_HOT), 1 if self.deterministic else 0,
-                  C.addressof(plan) if plan is not None else None, cur_stream())
+                  *(hot.args() if hot else NO_HOT), 1 if self.deterministic else 0, cur_stream())
         self._finish_step(hot, False)
 
     def _fused_segments(self):

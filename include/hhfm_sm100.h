@@ -166,33 +166,6 @@ int hhfm_fm_bn_fwd(const int32_t* col, int64_t B, int64_t F, const float* V, con
                    int64_t K, const float* gamma, const float* beta, const float* moving_mean, const float* moving_var,
                    float eps, float* out, hhfm_stream_t stream);
 
-/* K14  single-touch rows.  At the scaled shapes (M = 10^7, SURVEY.md 8d) ~40 % of the rows a step touches are referenced by
- * exactly one sample.  hhfm_count_refs counts the references of a step's id matrix (ref_count[M] is cleared first, ids < 0
- * are padding); the *_st variants of the training passes then apply the optimizer step of a row with ref_count == 1 on the
- * spot (TF ApplyAdagrad / ApplyGradientDescent, the same element update as hhfm_opt_*_rows -> the same bits) instead of
- * adding its gradient into gV: such a row is NOT stamped and does not appear in touched_rows.  Only the staged (large-table)
- * kernels use the plan, at most 3 rows per sample; every other row, and every row when another kernel is selected, goes the
- * usual way, so callers need no knowledge of which rows were taken.  Exactness needs an optimizer under which an untouched
- * row does not move (Adagrad, SGD) and lamda == 0 (FM.py:124 with lamda > 0 moves every row). */
-typedef struct hhfm_single_touch {
-  const int32_t* ref_count;  /* [M], from hhfm_count_refs over ALL ids the pass gathers (HHFM: the negatives too) */
-  float* V;                  /* the table the pass reads, writable */
-  float* acc;                /* Adagrad accumulator [M, K] (NULL for SGD) */
-  float* bias;               /* FM feature_bias [M], writable, and its accumulator; NULL when the model has no bias */
-  float* bias_acc;
-  float lr;
-  int32_t opt_kind;          /* HHFM_OPT_ADAGRAD or HHFM_OPT_SGD */
-} hhfm_single_touch;
-int hhfm_count_refs(const int32_t* ids, int64_t n_rows, int64_t stride, int64_t n_cols, int64_t M, int32_t* ref_count,
-                    hhfm_stream_t stream);
-int hhfm_fm_fwd_bwd_sqloss_st(const int32_t* row_ptr, const int32_t* col, const float* val, int64_t B, int64_t F,
-                           const float* V, const float* bias, const float* b0, int64_t M, int64_t K,
-                           int32_t interaction, const float* labels, float* out, float* gV, float* gbias, float* gb0,
-                           float* loss_partials, int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows,
-                           int32_t* touched_count, const int32_t* hot_slot, float* ghot, float* ghot_bias,
-                           int32_t n_rep, int32_t n_hot, int32_t deterministic, float keep, uint64_t drop_seed,
-                           const hhfm_single_touch* plan, hhfm_stream_t stream);
-
 /* Backward only, for torch.autograd: g = gout[s] given by the caller. */
 int hhfm_fm_bwd(const int32_t* row_ptr, const int32_t* col, const float* val, int64_t B, int64_t F,
                 const float* V, int64_t M, int64_t K, int32_t interaction, const float* gout,
@@ -348,14 +321,6 @@ int hhfm_pairrank_fwd_bwd(const int32_t* idx, int64_t B, int64_t stride, int32_t
                           const int32_t* hot_slot, float* ghot, int32_t n_rep, int32_t n_hot,
                           int32_t deterministic, hhfm_stream_t stream);
 
-/* The same pass with the single-touch plan of K14 (plan == NULL: the call above). */
-int hhfm_pairrank_fwd_bwd_st(const int32_t* idx, int64_t B, int64_t stride, int32_t n_ctx, int32_t n_time,
-                          int32_t n_neg, int32_t pool_ctx, int32_t pool_time, int32_t pool_stack, const float* V,
-                          int64_t M, int64_t K, float* pos_out, float* neg_out, float* gV, float* loss_partials,
-                          int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows, int32_t* touched_count,
-                          const int32_t* hot_slot, float* ghot, int32_t n_rep, int32_t n_hot,
-                          int32_t deterministic, const hhfm_single_touch* plan, hhfm_stream_t stream);
-
 /* Pooled context groups of the sum-pooling training pass.  With every pool mode HHFM_POOL_SUM only the sum of the pooled
  * rows enters the model, so pooled columns with small vocabularies can be pre-pooled: the columns of a group (id ranges
  * [col_lo[c], col_lo[c] + col_card[c]), disjoint, inside [0, M)) are replaced by one row of the group table
@@ -366,10 +331,10 @@ int hhfm_pairrank_fwd_bwd_st(const int32_t* idx, int64_t B, int64_t stride, int3
  *   hhfm_pool_groups_attach registers the plan under the table pointer V (col_group[c]: group number of pooled column c,
  *     c < n_pool = n_ctx + n_time, or -1 = ungrouped) and allocates S and G ([rows, K] each, G zero).  A later plan for
  *     the same V replaces it.  *handle identifies the plan for detach.
- *   hhfm_pairrank_fwd_bwd / _st then run, on the caller's stream: the pre-sum of S, the grouped training kernel, the
+ *   hhfm_pairrank_fwd_bwd then runs, on the caller's stream: the pre-sum of S, the grouped training kernel, the
  *     expansion of G into gV (fixed summation order) and the clearing of G.  The plan is used when M, K, n_ctx + n_time,
  *     stride and the current device match it, every pool mode is HHFM_POOL_SUM, n_neg == 10, K in {32, 64, 128},
- *     deterministic == 0 and no touched-row tracking, positive / negative outputs or single-touch plan is requested,
+ *     deterministic == 0 and no touched-row tracking or positive / negative outputs are requested,
  *     and the large-table (staged) kernel does not run; otherwise the call is the ungrouped one.  A sample whose member
  *     id lies outside the planned range pools and scatters that group's member rows individually (hot-row plan / gV).
  *     Member rows should not be hot rows: nothing but those fallback samples should reduce into them during the pass.

@@ -282,9 +282,9 @@ def test_batch_norm_0_step_calls_the_parent_entry_points(cuda):
     from hhfm_b200.models import FM
     rng = np.random.default_rng(2)
     M, B = 300, 4096
-    for keep, opt, want in ((1, "AdagradOptimizer", {"hhfm_fm_fwd_bwd_sqloss_st": 1, "hhfm_dp_step": 1}),
-                            (0.8, "AdagradOptimizer", {"hhfm_fm_fwd_bwd_sqloss_st": 1, "hhfm_dp_step": 1}),
-                            (1, "MomentumOptimizer", {"hhfm_fm_fwd_bwd_sqloss_st": 1, "hhfm_opt_momentum_dense_l2": 2,
+    for keep, opt, want in ((1, "AdagradOptimizer", {"hhfm_fm_fwd_bwd_sqloss_dropout": 1, "hhfm_dp_step": 1}),
+                            (0.8, "AdagradOptimizer", {"hhfm_fm_fwd_bwd_sqloss_dropout": 1, "hhfm_dp_step": 1}),
+                            (1, "MomentumOptimizer", {"hhfm_fm_fwd_bwd_sqloss_dropout": 1, "hhfm_opt_momentum_dense_l2": 2,
                                                       "hhfm_opt_momentum_rows": 1, "hhfm_loss_finalize": 1})):
         m = FM(6, M, 50, 100, 64, 0.05, 0.1, keep, opt, 0, 0)
         idx = dev(rng.integers(0, M, (B, 6)), cuda, torch.int32)
