@@ -351,9 +351,9 @@ static int dispatch_fm_fixed(const FmArgs& a, cudaStream_t st) {
   do {                                                        \
     if (a.F <= 8) return launch_fm_fixed<L, 8>(a, st);        \
     if (a.F <= 12) return launch_fm_fixed<L, 12>(a, st);      \
-    return launch_fm_fixed<L, (L >= 16 ? 16 : 8)>(a, st);     \
+    return launch_fm_fixed<L, 16>(a, st);                     \
   } while (0)
-  if (lps == 8) FIXED(8);
+  if (lps == 8) return launch_fm_fixed<8, 8>(a, st);          // F <= K/4 = 8
   if (lps == 16) FIXED(16);
   FIXED(32);
 #undef FIXED

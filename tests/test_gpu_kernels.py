@@ -88,10 +88,12 @@ def test_fm_forward_csr_ragged_with_values(cuda):
     assert_close(out.cpu().numpy(), ref, what="fm csr out")
 
 
-def _fm_train_call(cuda, X, Y, V, b, b0, interaction=0, deterministic=0, track=True, val=None):
+def _fm_train_call(cuda, X, Y, V, b, b0, interaction=0, deterministic=0, track=True, val=None, hot_rows=None):
     lib, ptr, st = _lib_ptr()
+    from hhfm_b200.engine import NO_HOT_BIAS, HotRows
     B, F = X.shape
     M, K = V.shape
+    hot = HotRows(hot_rows, M, K, cuda, with_bias=True, n_rep=4) if hot_rows is not None else None
     P = lib.partials_len()
     tV = dev(V, cuda); tb = dev(b, cuda) if b is not None else None
     tb0 = dev(np.array([b0], np.float32), cuda) if b0 is not None else None
@@ -103,7 +105,9 @@ def _fm_train_call(cuda, X, Y, V, b, b0, interaction=0, deterministic=0, track=T
     lib.call("hhfm_fm_fwd_bwd_sqloss", None, ptr(dev(X, cuda, torch.int32)), ptr(tval), B, F, ptr(tV), ptr(tb), ptr(tb0), M, K,
              interaction, ptr(dev(Y.reshape(-1), cuda)), ptr(out), ptr(gV), ptr(gb) if b is not None else None,
              ptr(gb0) if b0 is not None else None, ptr(lp), ptr(stamp) if track else None, 1, ptr(rows) if track else None,
-             ptr(cnt) if track else None, None, None, None, 0, 0, deterministic, st())
+             ptr(cnt) if track else None, *(hot.args(True) if hot is not None else NO_HOT_BIAS), deterministic, st())
+    if hot is not None:
+        hot.fold(gV, gb if b is not None else None)
     lib.call("hhfm_loss_finalize", ptr(lp), None, 0.0, ptr(loss), st())
     n = int(cnt.item())
     return dict(loss=float(loss.item()), out=out.cpu().numpy(), gV=gV.cpu().numpy(), gb=gb.cpu().numpy(),
@@ -771,17 +775,21 @@ def test_fm_staged_pipeline_matches_oracle(cuda, B, F, K, monkeypatch):
     if F > 4:
         X[:, 4] = X[:, 0]
     Y = rng.choice([1.0, 0.0], (B, 1)).astype(np.float32)
+    from test_kernel_instances import launched_kernels
     loss, out, dV, db, db0, touched = O.fm_loss_grads(X, Y, V, b, b0, lamda=0.0)
-    got = _fm_train_call(cuda, X, Y, V, b, b0)
+    names, got = launched_kernels(lambda: _fm_train_call(cuda, X, Y, V, b, b0))
+    assert len(names) == 1 and names.pop().startswith("fm_train_staged_kernel<")
     assert_close(got["out"], out, what="out")
     assert_close(got["loss"], loss, what="loss")
     assert_close(got["gV"], dV, what="gV")
     assert_close(got["gb"], db, what="gbias")
     assert_close(got["gb0"], db0, what="gb0")
     assert (got["touched"] == touched).all()
-    got2 = _fm_train_call(cuda, X, Y, V, None, None, track=False)          # no bias, no tracking
+    names, got2 = launched_kernels(lambda: _fm_train_call(cuda, X, Y, V, None, None, track=False))   # no bias, no tracking
+    assert len(names) == 1 and names.pop().startswith("fm_train_staged_kernel<")
     monkeypatch.setenv("HHFM_FM_STAGED", "0")
-    ref2 = _fm_train_call(cuda, X, Y, V, None, None, track=False)
+    names, ref2 = launched_kernels(lambda: _fm_train_call(cuda, X, Y, V, None, None, track=False))
+    assert len(names) == 1 and not names.pop().startswith("fm_train_staged_kernel<")
     assert_close(got2["out"], ref2["out"], what="staged vs register out"); assert_close(got2["gV"], ref2["gV"], what="staged vs register gV")
 
 
@@ -815,6 +823,9 @@ def test_pairrank_staged_pipeline_matches_oracle(cuda, K, fc, ft, NG, B, use_hot
     register kernel."""
     lib, ptr, st = _lib_ptr()
     from hhfm_b200.engine import NO_HOT, HotRows
+    from test_kernel_instances import launched_kernels
+    if (K, 2 + fc + ft + NG) in ((128, 22), (512, 6)):
+        monkeypatch.setenv("HHFM_PR_WARPS", "9")       # two stages of 10 warps exceed the 224 KB of shared memory
     rng = np.random.default_rng(K + fc + ft + NG)
     M = 700
     V = make_table(rng, M, K)
@@ -834,8 +845,12 @@ def test_pairrank_staged_pipeline_matches_oracle(cuda, K, fc, ft, NG, B, use_hot
         gV = torch.zeros(M, K, device=cuda); lp = torch.zeros(P, device=cuda); out = torch.zeros(1, device=cuda)
         stamp = torch.zeros(M, dtype=torch.int32, device=cuda); rows = torch.zeros(M, dtype=torch.int32, device=cuda)
         cnt = torch.zeros(1, dtype=torch.int32, device=cuda)
-        lib.call("hhfm_pairrank_fwd_bwd", ptr(dev(rec, cuda)), B, stride, fc, ft, NG, 0, 0, 0, ptr(dev(V, cuda)), M, K, None, None,
-                 ptr(gV), ptr(lp), ptr(stamp), 5, ptr(rows), ptr(cnt), *(hot.args() if hot else NO_HOT), 0, st())
+        names, _ = launched_kernels(lambda: lib.call(
+            "hhfm_pairrank_fwd_bwd", ptr(dev(rec, cuda)), B, stride, fc, ft, NG, 0, 0, 0, ptr(dev(V, cuda)), M, K, None, None,
+            ptr(gV), ptr(lp), ptr(stamp), 5, ptr(rows), ptr(cnt), *(hot.args() if hot else NO_HOT), 0, st()))
+        assert len(names) == 1
+        kernel = names.pop()
+        assert kernel.startswith("pairrank_sum_train_staged_kernel<" if mode == "1" else "pairrank_kernel<"), (mode, kernel)
         if hot:
             hot.fold(gV, None)
         lib.call("hhfm_loss_finalize", ptr(lp), None, 0.0, ptr(out), st())
