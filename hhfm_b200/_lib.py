@@ -40,6 +40,10 @@ SIGNATURES = {
     "hhfm_dfm_fwd_bwd_sqloss": [vp, i64, i64, vp, vp, i64, i64, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32,
                                 vp],
     "hhfm_dfm_topn_scores": [vp, i64, i64, i64, i32, vp, vp, i64, i64, vp, i32, vp, i64, i64, vp, vp, vp],
+    "hhfm_dfm_fwd_mode": [vp, i64, i64, vp, vp, i64, i64, vp, i32, vp, i32, vp, vp, vp],
+    "hhfm_dfm_fwd_bwd_mode": [vp, i64, i64, vp, vp, i64, i64, vp, i32, vp, i32, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp,
+                              i32, i32, vp],
+    "hhfm_dfm_topn_scores_mode": [vp, i64, i64, i64, i32, vp, vp, i64, i64, vp, i32, vp, i32, i64, i64, vp, vp, vp],
     "hhfm_wd_wide_fwd": [vp, i64, i64, vp, vp, vp, i64, i32, vp, vp],
     "hhfm_wd_wide_bwd": [vp, i64, i64, vp, i64, i32, vp, vp, vp, vp],
     "hhfm_wd_deep_fwd": [vp, i64, i64, vp, i64, i64, vp, i32, vp, vp, vp, vp, vp],
@@ -99,6 +103,10 @@ INT64_FUNCS = {
     "hhfm_dfm_param_count": [i64, i64, i32, vp],
     "hhfm_dfm_reg_count": [i64, i64, i32, vp],
     "hhfm_workspace_bytes_dfm": [i64, i64, i64, i32, vp],
+    "hhfm_dfm_param_count_mode": [i64, i64, i32, vp, i32],
+    "hhfm_dfm_reg_count_mode": [i64, i64, i32, vp, i32],
+    "hhfm_workspace_bytes_dfm_mode": [i64, i64, i64, i32, vp, i32],
+    "hhfm_workspace_bytes_dfm_topn_mode": [i64, i64, i64, i64, i32, vp, i32],
     "hhfm_workspace_bytes_fm_bn": [i64, i64],
 }
 OPTIONAL = {}   # symbols added by later kernels are appended by their modules via `declare`

@@ -4,6 +4,10 @@
 //   H_0 = reshape(E) [F*K];  H_i = relu(H_{i-1} W_{i-1} + b_{i-1}),  i = 1..L                     (DFM.py:125-128)
 //   out = [y1 | y2 | H_L] . proj + cbias;  loss = 0.5 sum (y - out)^2  (+ l2 through the optimizer)   (DFM.py:131-152)
 //
+// The reference's options select parts of this graph independently (hhfm_dfm_mode bits): use_fm=False drops y1 / y2,
+// use_deep=False drops the tower (out = [y1 | y2] . proj + cbias), loss_type='logloss' makes out = sigmoid(logit) and the loss
+// tf.losses.log_loss(y, out) = mean_s [-y log(out + 1e-7) - (1 - y) log((1 - out) + 1e-7)].
+//
 // Two kernels:
 //  * `sgemm_kernel<AMODE,BMODE,EPI>`: a 128x64x16 register-blocked fp32 SIMT GEMM (8x4 outputs per thread, double-
 //    buffered shared tiles) whose A operand can be GATHERED from the embedding table (layer 0 never materialises
@@ -251,17 +255,24 @@ struct HeadArgs {
   float* gblast;           // [D]  bias gradient of the last hidden layer = column sums of dZ_L
   float* loss_partials;
   HotPlan hot;             // optional hot-row replicas for the FM-part scatter
-  // Wide&Deep mode (WDMF.py:51-126): no FM terms, out = H_L . proj3 + cbias + extra[s] is a logit, loss = mean sigmoid
+  int fm;                  // 1: first- and second-order terms (and their gradients); 0: out = H_L . proj3 + cbias (+ extra)
+  int loss;                // HEAD_SQ / HEAD_WD / HEAD_LOGLOSS (HEAD_LOGLOSS: out[s] = sigmoid(logit))
+  // Wide&Deep (WDMF.py:51-126): no FM terms, out = H_L . proj3 + cbias + extra[s] is a logit, loss = mean sigmoid
   // cross-entropy over the batch, d loss / d out is also written per sample for the wide part's scatter
-  int wd;
   const float* extra;      // [B] additive logit (the wide part) or NULL
   float* gsample;          // [B] d loss / d out (TRAIN) or NULL
-  float inv_b;             // 1 / B
+  float inv_b;             // 1 / B (WD), 1 / B_total (log_loss: the batch the mean runs over, all ranks together)
 };
+
+// loss heads: 0.5 (y - out)^2 summed (DeepFM mse); WD's mean sigmoid cross-entropy on the logit; DeepFM's
+// tf.losses.log_loss on the sigmoid (DFM.py:139-141), TF's epsilon and evaluation order
+enum { HEAD_SQ = 0, HEAD_WD = 1, HEAD_LOGLOSS = 2 };
+constexpr float kLogLossEps = 1e-7f;
 
 constexpr int kHeadT = 8;    // D <= 32 * kHeadT
 
-template <int VPL, bool TRAIN>
+// LOG: the log_loss head (a.loss == HEAD_LOGLOSS) as its own instance, so the other heads keep their register budget
+template <int VPL, bool TRAIN, bool LOG>
 __global__ void __launch_bounds__(256) dfm_head_kernel(const HeadArgs a) {
   extern __shared__ float sred[];         // TRAIN: [F + K + 2*D + 1]
   __shared__ float scratch[32];
@@ -297,12 +308,12 @@ __global__ void __launch_bounds__(256) dfm_head_kernel(const HeadArgs a) {
   for (int t = 0; t < kHeadT; t++) { g3[t] = 0.f; gbl[t] = 0.f; }
 
   for (int64_t s = warp_g; s < a.B; s += n_warps) {
-    const int my_id = (lane < F && !a.wd) ? __ldg(a.idx + s * F + lane) : 0;
-    const float y1 = (lane < F && !a.wd) ? __ldg(a.fbias + my_id) : 0.f;
+    const int my_id = (lane < F && a.fm) ? __ldg(a.idx + s * F + lane) : 0;
+    const float y1 = (lane < F && a.fm) ? __ldg(a.fbias + my_id) : 0.f;
     float4 S[VPL], Q[VPL];
 #pragma unroll
     for (int i = 0; i < VPL; i++) { S[i] = f4_zero(); Q[i] = f4_zero(); }
-    for (int f = 0; f < (a.wd ? 0 : F); f++) {
+    for (int f = 0; f < (a.fm ? F : 0); f++) {
       const int id = __shfl_sync(0xffffffffu, my_id, f);
       const float4* row = reinterpret_cast<const float4*>(a.V) + (size_t)id * kv;
 #pragma unroll
@@ -331,12 +342,21 @@ __global__ void __launch_bounds__(256) dfm_head_kernel(const HeadArgs a) {
       part = fmaf(h[t], p3[t], part);
     }
     float out = warp_sum(part) + cb;
-    if (a.wd && a.extra) out += __ldg(a.extra + s);
-    if (lane == 0 && a.out) a.out[s] = out;
+    if (a.loss == HEAD_WD && a.extra) out += __ldg(a.extra + s);
+    const float pr = LOG ? 1.f / (1.f + expf(-out)) : out;
+    if (lane == 0 && a.out) a.out[s] = pr;
     if (!TRAIN) continue;
 
     float g;
-    if (a.wd) {
+    if (LOG) {
+      // per sample -y log(p + eps) - (1 - y) log((1 - p) + eps), mean over B_total; d/d logit = p (1 - p) d/dp (TF's
+      // SigmoidGrad).  Labels are used as given (the drop-in trainer's negatives are -1).
+      const float y = __ldg(a.labels + s);
+      const float q = 1.f - pr;
+      loss_acc += (lane == 0) ? (-(y * logf(pr + kLogLossEps)) - (1.f - y) * logf(q + kLogLossEps)) * a.inv_b : 0.f;
+      const float dp = (-y / (pr + kLogLossEps) + (1.f - y) / (q + kLogLossEps)) * a.inv_b;
+      g = dp * pr * q;
+    } else if (a.loss == HEAD_WD) {
       // mean sigmoid cross-entropy, labels in {0, 1}: loss = (max(z,0) - z y + log(1 + exp(-|z|))) / B, d/dz = (sigmoid(z) - y) / B
       const float y = __ldg(a.labels + s);
       const float pr = 1.f / (1.f + expf(-out));
@@ -359,7 +379,7 @@ __global__ void __launch_bounds__(256) dfm_head_kernel(const HeadArgs a) {
       gbl[t] += dz;
       if (j < D) hrow[j] = dz;
     }
-    if (a.wd) continue;
+    if (!a.fm) continue;
     // FM part of the embedding gradient: dV[x_f] += g * proj2 * (S - e_f);  d feature_bias[x_f] += g * proj1[f]
     const int my_slot = (a.hot.slot && lane < F) ? __ldg(a.hot.slot + my_id) : -1;
     if (lane < F) {
@@ -415,14 +435,20 @@ __global__ void __launch_bounds__(256) dfm_head_kernel(const HeadArgs a) {
   write_partial(a.loss_partials, bl);
 }
 
+template <bool TRAIN, bool LOG>
+static void launch_head_vpl(const HeadArgs& a, int grid, size_t smem, cudaStream_t st) {
+  const int kv = a.K >> 2;
+  if (kv <= 32) dfm_head_kernel<1, TRAIN, LOG><<<grid, 256, smem, st>>>(a);
+  else if (kv <= 64) dfm_head_kernel<2, TRAIN, LOG><<<grid, 256, smem, st>>>(a);
+  else dfm_head_kernel<4, TRAIN, LOG><<<grid, 256, smem, st>>>(a);
+}
+
 template <bool TRAIN>
 static int launch_head(const HeadArgs& a, cudaStream_t st) {
   const int grid = grid_for(a.B, 8, 4);
   const size_t smem = TRAIN ? (size_t)(a.F + a.K + 2 * a.D + 1) * sizeof(float) : 0;
-  const int kv = a.K >> 2;
-  if (kv <= 32) dfm_head_kernel<1, TRAIN><<<grid, 256, smem, st>>>(a);
-  else if (kv <= 64) dfm_head_kernel<2, TRAIN><<<grid, 256, smem, st>>>(a);
-  else dfm_head_kernel<4, TRAIN><<<grid, 256, smem, st>>>(a);
+  if (a.loss == HEAD_LOGLOSS) launch_head_vpl<TRAIN, true>(a, grid, smem, st);
+  else launch_head_vpl<TRAIN, false>(a, grid, smem, st);
   return check_launch("dfm_head_kernel");
 }
 
@@ -438,7 +464,28 @@ struct DfmLayout {
   int64_t ws_floats;
 };
 
-static int dfm_layout(int64_t B, int64_t F, int64_t K, int32_t L, const int32_t* sizes, DfmLayout& lo) {
+// Mode bits (hhfm_dfm_mode) plus one internal bit for the Wide&Deep head, which callers cannot pass
+constexpr int32_t kDfmPublicBits = HHFM_DFM_NO_FM | HHFM_DFM_NO_DEEP | HHFM_DFM_LOGLOSS;
+constexpr int32_t kDfmWd = 1 << 8;
+
+static bool dfm_fm(int32_t mode) { return !(mode & HHFM_DFM_NO_FM); }
+static bool dfm_deep(int32_t mode) { return !(mode & HHFM_DFM_NO_DEEP); }
+
+static int dfm_check_mode(int32_t mode) {
+  HHFM_REQUIRE((mode & ~kDfmPublicBits) == 0, "dfm: unknown mode bits 0x%x (known: NO_FM 1, NO_DEEP 2, LOGLOSS 4)",
+               (unsigned)(mode & ~kDfmPublicBits));
+  HHFM_REQUIRE(dfm_fm(mode) || dfm_deep(mode), "dfm: mode %d enables neither the FM part nor the tower", (int)mode);
+  return HHFM_OK;
+}
+
+static void dfm_head_mode(int32_t mode, HeadArgs& h) {
+  h.fm = dfm_fm(mode) ? 1 : 0;
+  h.loss = (mode & kDfmWd) ? HEAD_WD : (mode & HHFM_DFM_LOGLOSS) ? HEAD_LOGLOSS : HEAD_SQ;
+}
+
+// use_deep=False: the layer matrices keep their place (the model still owns them), the projection starts on a 16-byte
+// boundary so the optimizer can step [proj_off, reg_len) alone, and no activation workspace is needed
+static int dfm_layout(int64_t B, int64_t F, int64_t K, int32_t L, const int32_t* sizes, DfmLayout& lo, int32_t mode = 0) {
   HHFM_REQUIRE(L >= 1 && L <= kDfmMaxLayers && sizes, "dfm: 1 <= n_layers <= %d", kDfmMaxLayers);
   HHFM_REQUIRE(F >= 1 && F <= 32, "dfm: 1 <= field_size <= 32");
   HHFM_REQUIRE(K % 4 == 0 && K > 0 && K <= 512, "dfm: embedding_size must be a multiple of 4, <= 512");
@@ -452,6 +499,7 @@ static int dfm_layout(int64_t B, int64_t F, int64_t K, int32_t L, const int32_t*
     off += (int64_t)lo.d[i] * lo.d[i + 1];
   }
   HHFM_REQUIRE(lo.d[L] <= 32 * kHeadT, "dfm: last hidden layer must be <= %d wide", 32 * kHeadT);
+  if (!dfm_deep(mode)) off = (off + 3) / 4 * 4;
   lo.proj_off = off;
   off += F + K + lo.d[L];
   off = (off + 3) / 4 * 4;          // zero padding keeps the un-regularised tail 16-byte aligned for the optimizer
@@ -467,7 +515,7 @@ static int dfm_layout(int64_t B, int64_t F, int64_t K, int32_t L, const int32_t*
     lo.h_off[i] = ws;
     ws += B * lo.ld[i];
   }
-  lo.ws_floats = ws;
+  lo.ws_floats = dfm_deep(mode) ? ws : 0;
   return HHFM_OK;
 }
 
@@ -600,7 +648,8 @@ struct DfmTopnArgs {
   int64_t ld1;
   const float *V, *fbias, *W1, *b1, *proj;
   int64_t item_base, N;
-  float *U, *T, *SQ, *fo;      // [C, ld1], [N, ld1], [C, 2K], [C]
+  float *U, *T, *SQ, *fo;      // [C, ld1], [N, ld1] (tower only), [C, 2K], [C] (FM part only)
+  int fm, deep, sig;           // parts of the graph the mode keeps; sig: scores are sigmoid(logit)
 };
 
 __global__ void __launch_bounds__(256) dfm_topn_ctx_kernel(const DfmTopnArgs a) {
@@ -613,17 +662,19 @@ __global__ void __launch_bounds__(256) dfm_topn_ctx_kernel(const DfmTopnArgs a) 
     sE[i] = (f == a.item_col) ? 0.f : __ldg(a.V + (size_t)__ldg(rec + f) * K + k);
   }
   __syncthreads();
-  for (int k = threadIdx.x; k < K; k += blockDim.x) {
+  for (int k = threadIdx.x; k < (a.fm ? K : 0); k += blockDim.x) {
     float S = 0.f, Q = 0.f;
     for (int f = 0; f < F; f++) { const float e = sE[f * K + k]; S += e; Q = fmaf(e, e, Q); }
     a.SQ[(int64_t)c * 2 * K + k] = S;
     a.SQ[(int64_t)c * 2 * K + K + k] = Q;
   }
-  float fo = 0.f;
-  if ((int)threadIdx.x < F && (int)threadIdx.x != a.item_col) fo = __ldg(a.fbias + __ldg(rec + threadIdx.x)) * __ldg(a.proj + threadIdx.x);
-  fo = block_sum(fo, scratch);
-  if (threadIdx.x == 0) a.fo[c] = fo;
-  for (int j = threadIdx.x; j < a.ld1; j += blockDim.x) {
+  if (a.fm) {
+    float fo = 0.f;
+    if ((int)threadIdx.x < F && (int)threadIdx.x != a.item_col) fo = __ldg(a.fbias + __ldg(rec + threadIdx.x)) * __ldg(a.proj + threadIdx.x);
+    fo = block_sum(fo, scratch);
+    if (threadIdx.x == 0) a.fo[c] = fo;
+  }
+  for (int j = threadIdx.x; j < (a.deep ? a.ld1 : 0); j += blockDim.x) {
     float acc = 0.f;
     if (j < a.d1) {
       for (int f = 0; f < F; f++) {
@@ -691,7 +742,7 @@ __global__ void __launch_bounds__(256) dfm_topn_head_kernel(const DfmTopnArgs a,
   const int64_t n_warps = (int64_t)gridDim.x * (blockDim.x >> 5);
   const int64_t total = (int64_t)a.C * a.N;
   const float cb = __ldg(cbias);
-  const float pitem = __ldg(a.proj + a.item_col);
+  const float pitem = a.fm ? __ldg(a.proj + a.item_col) : 0.f;
   const float* p2 = a.proj + a.F;
   const float* p3 = a.proj + a.F + K;
   for (int64_t s = warp_g; s < total; s += n_warps) {
@@ -699,7 +750,7 @@ __global__ void __launch_bounds__(256) dfm_topn_head_kernel(const DfmTopnArgs a,
     const float* v = a.V + (size_t)(a.item_base + n) * K;
     const float* S = a.SQ + c * 2 * K;
     float part = 0.f;
-    for (int k = lane; k < K; k += 32) {
+    for (int k = lane; k < (a.fm ? K : 0); k += 32) {
       const float e = __ldg(v + k);
       const float sv = __ldg(S + k) + e, q = fmaf(e, e, __ldg(S + K + k));
       part = fmaf(0.5f * (sv * sv - q), __ldg(p2 + k), part);
@@ -714,36 +765,46 @@ __global__ void __launch_bounds__(256) dfm_topn_head_kernel(const DfmTopnArgs a,
     } else {
       for (int j = lane; j < D; j += 32) part = fmaf(hrow[j], __ldg(p3 + j), part);
     }
-    if (lane == 0) part += __ldg(a.fo + c) + __ldg(a.fbias + a.item_base + n) * pitem;
+    if (lane == 0 && a.fm) part += __ldg(a.fo + c) + __ldg(a.fbias + a.item_base + n) * pitem;
     const float out = warp_sum(part) + cb;
-    if (lane == 0) scores[s] = out;
+    if (lane == 0) scores[s] = a.sig ? 1.f / (1.f + expf(-out)) : out;      // what the model's `out` ranks by
   }
 }
 
-static int64_t dfm_topn_side_floats(int64_t C, int64_t N, int64_t K, int64_t ld1) {
-  return C * ld1 + N * ld1 + C * 2 * K + (C + 3) / 4 * 4;
+// side buffers of the evaluator, in this order: U [C, ld1] and T [N, ld1] (tower), SQ [C, 2K] and fo [C] (FM part)
+static int64_t dfm_topn_side_floats(int64_t C, int64_t N, int64_t K, int64_t ld1, int32_t mode = 0) {
+  return (dfm_deep(mode) ? C * ld1 + N * ld1 : 0) + (dfm_fm(mode) ? C * 2 * K + (C + 3) / 4 * 4 : 0);
 }
 
 }  // namespace hhfm
 
 using namespace hhfm;
 
-extern "C" int64_t hhfm_dfm_param_count(int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes) {
+extern "C" int64_t hhfm_dfm_param_count_mode(int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes, int32_t mode) {
   DfmLayout lo;
-  if (dfm_layout(1, F, K, n_layers, layer_sizes, lo) != HHFM_OK) return -1;
+  if (dfm_check_mode(mode) != HHFM_OK || dfm_layout(1, F, K, n_layers, layer_sizes, lo, mode) != HHFM_OK) return -1;
   return lo.total;
 }
 
-extern "C" int64_t hhfm_dfm_reg_count(int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes) {
+extern "C" int64_t hhfm_dfm_reg_count_mode(int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes, int32_t mode) {
   DfmLayout lo;
-  if (dfm_layout(1, F, K, n_layers, layer_sizes, lo) != HHFM_OK) return -1;
+  if (dfm_check_mode(mode) != HHFM_OK || dfm_layout(1, F, K, n_layers, layer_sizes, lo, mode) != HHFM_OK) return -1;
   return lo.reg_len;
 }
 
-extern "C" int64_t hhfm_workspace_bytes_dfm(int64_t B, int64_t F, int64_t K, int32_t n_layers,
-                                            const int32_t* layer_sizes) {
+extern "C" int64_t hhfm_dfm_param_count(int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes) {
+  return hhfm_dfm_param_count_mode(F, K, n_layers, layer_sizes, 0);
+}
+
+extern "C" int64_t hhfm_dfm_reg_count(int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes) {
+  return hhfm_dfm_reg_count_mode(F, K, n_layers, layer_sizes, 0);
+}
+
+extern "C" int64_t hhfm_workspace_bytes_dfm_mode(int64_t B, int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes,
+                                                 int32_t mode) {
   DfmLayout lo;
-  if (dfm_layout(B, F, K, n_layers, layer_sizes, lo) != HHFM_OK) return -1;
+  if (dfm_check_mode(mode) != HHFM_OK || dfm_layout(B, F, K, n_layers, layer_sizes, lo, mode) != HHFM_OK) return -1;
+  if (!dfm_deep(mode)) return 0;               // the head reads nothing but the parameters
   if (dfm_use_tc(K)) {
     DfmTcLayout t;
     dfm_tc_layout(B, lo, t);
@@ -752,20 +813,32 @@ extern "C" int64_t hhfm_workspace_bytes_dfm(int64_t B, int64_t F, int64_t K, int
   return lo.ws_floats * (int64_t)sizeof(float);
 }
 
+extern "C" int64_t hhfm_workspace_bytes_dfm(int64_t B, int64_t F, int64_t K, int32_t n_layers,
+                                            const int32_t* layer_sizes) {
+  return hhfm_workspace_bytes_dfm_mode(B, F, K, n_layers, layer_sizes, 0);
+}
+
+// mode: hhfm_dfm_mode bits, or HHFM_DFM_NO_FM | kDfmWd for the Wide&Deep deep part
 static int dfm_fwd_impl(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* feature_bias,
                         int64_t M, int64_t K, const float* params, int32_t n_layers, const int32_t* layer_sizes,
-                        float* workspace, float* out, hhfm_stream_t stream, int wd, const float* extra) {
-  HHFM_REQUIRE(idx && V && (feature_bias || wd) && params && workspace && out, "dfm_fwd: NULL argument");
+                        float* workspace, float* out, hhfm_stream_t stream, int32_t mode, const float* extra) {
+  const bool fm = dfm_fm(mode), deep = dfm_deep(mode);
+  HHFM_REQUIRE(idx && V && (feature_bias || !fm) && params && (workspace || !deep) && out, "dfm_fwd: NULL argument");
   HHFM_REQUIRE(B >= 0 && B < (1ll << 31) && M > 0, "dfm_fwd: bad sizes");
   if (B == 0) return HHFM_OK;
   DfmLayout lo;
-  int rc = dfm_layout(B, F, K, n_layers, layer_sizes, lo);
+  int rc = dfm_layout(B, F, K, n_layers, layer_sizes, lo, mode);
   if (rc != HHFM_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   HeadArgs h{};
   h.idx = idx; h.B = B; h.F = (int)F; h.K = (int)K; h.D = lo.d[lo.L];
   h.V = V; h.fbias = feature_bias; h.proj = params + lo.proj_off; h.cbias = params + lo.cbias_off; h.out = out;
-  h.wd = wd; h.extra = extra;
+  dfm_head_mode(mode, h);
+  h.extra = extra;
+  if (!deep) {                                  // FM part only: no GEMM, no tower input
+    h.D = 0; h.H = nullptr; h.ldh = 0;
+    return launch_head<false>(h, st);
+  }
   if (dfm_use_tc(K)) {
     DfmTcLayout t;
     dfm_tc_layout(B, lo, t);
@@ -786,14 +859,17 @@ static int dfm_fwd_bwd_impl(const int32_t* idx, int64_t B, int64_t F, const floa
                             int32_t n_layers, const int32_t* layer_sizes, const float* labels,
                             float* workspace, float* out, float* gV, float* gbias, float* gparams,
                             float* loss_partials, const int32_t* hot_slot, float* ghot, float* ghot_bias,
-                            int32_t n_rep, int32_t n_hot, hhfm_stream_t stream, int wd, const float* extra, float* gsample) {
-  HHFM_REQUIRE(idx && V && (feature_bias || wd) && params && workspace && labels && gV && (gbias || wd) && gparams && loss_partials,
-               "dfm_fwd_bwd_sqloss: NULL argument");
-  HHFM_REQUIRE(B > 0 && B < (1ll << 31) && M > 0, "dfm_fwd_bwd_sqloss: bad sizes");
+                            int32_t n_rep, int32_t n_hot, hhfm_stream_t stream, int32_t mode, int64_t B_total,
+                            const float* extra, float* gsample) {
+  const bool fm = dfm_fm(mode), deep = dfm_deep(mode);
+  HHFM_REQUIRE(idx && V && (feature_bias || !fm) && params && (workspace || !deep) && labels && gV && (gbias || !fm) && gparams &&
+               loss_partials, "dfm_fwd_bwd: NULL argument");
+  HHFM_REQUIRE(B > 0 && B < (1ll << 31) && M > 0, "dfm_fwd_bwd: bad sizes");
+  HHFM_REQUIRE(B_total >= B, "dfm_fwd_bwd: B_total (%lld) must be >= B (%lld)", (long long)B_total, (long long)B);
   DfmLayout lo;
-  int rc = dfm_layout(B, F, K, n_layers, layer_sizes, lo);
+  int rc = dfm_layout(B, F, K, n_layers, layer_sizes, lo, mode);
   if (rc != HHFM_OK) return rc;
-  HHFM_REQUIRE(!hot_slot || (ghot && n_rep >= 1 && n_hot >= 1), "dfm_fwd_bwd_sqloss: hot_slot needs ghot, n_rep, n_hot");
+  HHFM_REQUIRE(!hot_slot || (ghot && n_rep >= 1 && n_hot >= 1), "dfm_fwd_bwd: hot_slot needs ghot, n_rep, n_hot");
   cudaStream_t st = (cudaStream_t)stream;
   const int L = lo.L;
   const HotPlan hot{hot_slot, ghot, ghot_bias, n_rep, n_hot};
@@ -803,11 +879,16 @@ static int dfm_fwd_bwd_impl(const int32_t* idx, int64_t B, int64_t F, const floa
   h.labels = labels; h.out = out;
   h.gV = gV; h.gfbias = gbias; h.gproj = gparams + lo.proj_off; h.gcbias = gparams + lo.cbias_off;
   h.gblast = gparams + lo.b_off[L - 1]; h.loss_partials = loss_partials; h.hot = hot;
-  h.wd = wd; h.extra = extra; h.gsample = gsample; h.inv_b = 1.0f / (float)B;
+  dfm_head_mode(mode, h);
+  h.extra = extra; h.gsample = gsample; h.inv_b = 1.0f / (float)B_total;
+  if (!deep) {                                  // FM part only: D = 0, no dZ, no tower gradients
+    h.D = 0; h.H = nullptr; h.ldh = 0; h.gblast = nullptr;
+    return launch_head<true>(h, st);
+  }
   if (dfm_use_tc(K)) {
     DfmTcLayout t;
     dfm_tc_layout(B, lo, t);
-    HHFM_REQUIRE(((uintptr_t)workspace & 15) == 0, "dfm_fwd_bwd_sqloss: workspace must be 16-byte aligned");
+    HHFM_REQUIRE(((uintptr_t)workspace & 15) == 0, "dfm_fwd_bwd: workspace must be 16-byte aligned");
     float* ws = workspace;
     if ((rc = dfm_tc_forward(idx, B, F, V, K, params, lo, t, ws, true, st))) return rc;
     h.H = ws + t.x[L]; h.ldh = t.ldx[L];
@@ -884,10 +965,29 @@ static int dfm_fwd_bwd_impl(const int32_t* idx, int64_t B, int64_t F, const floa
   return HHFM_OK;
 }
 
+extern "C" int hhfm_dfm_fwd_mode(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* feature_bias, int64_t M,
+                                 int64_t K, const float* params, int32_t n_layers, const int32_t* layer_sizes, int32_t mode,
+                                 float* workspace, float* out, hhfm_stream_t stream) {
+  int rc = dfm_check_mode(mode);
+  if (rc != HHFM_OK) return rc;
+  return dfm_fwd_impl(idx, B, F, V, feature_bias, M, K, params, n_layers, layer_sizes, workspace, out, stream, mode, nullptr);
+}
+
+extern "C" int hhfm_dfm_fwd_bwd_mode(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* feature_bias,
+                                     int64_t M, int64_t K, const float* params, int32_t n_layers, const int32_t* layer_sizes,
+                                     int32_t mode, int64_t B_total, const float* labels, float* workspace, float* out, float* gV,
+                                     float* gbias, float* gparams, float* loss_partials, const int32_t* hot_slot, float* ghot,
+                                     float* ghot_bias, int32_t n_rep, int32_t n_hot, hhfm_stream_t stream) {
+  int rc = dfm_check_mode(mode);
+  if (rc != HHFM_OK) return rc;
+  return dfm_fwd_bwd_impl(idx, B, F, V, feature_bias, M, K, params, n_layers, layer_sizes, labels, workspace, out, gV, gbias,
+                          gparams, loss_partials, hot_slot, ghot, ghot_bias, n_rep, n_hot, stream, mode, B_total, nullptr, nullptr);
+}
+
 extern "C" int hhfm_dfm_fwd(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* feature_bias,
                             int64_t M, int64_t K, const float* params, int32_t n_layers, const int32_t* layer_sizes,
                             float* workspace, float* out, hhfm_stream_t stream) {
-  return dfm_fwd_impl(idx, B, F, V, feature_bias, M, K, params, n_layers, layer_sizes, workspace, out, stream, 0, nullptr);
+  return hhfm_dfm_fwd_mode(idx, B, F, V, feature_bias, M, K, params, n_layers, layer_sizes, 0, workspace, out, stream);
 }
 
 extern "C" int hhfm_dfm_fwd_bwd_sqloss(const int32_t* idx, int64_t B, int64_t F, const float* V,
@@ -896,8 +996,8 @@ extern "C" int hhfm_dfm_fwd_bwd_sqloss(const int32_t* idx, int64_t B, int64_t F,
                                        float* workspace, float* out, float* gV, float* gbias, float* gparams,
                                        float* loss_partials, const int32_t* hot_slot, float* ghot, float* ghot_bias,
                                        int32_t n_rep, int32_t n_hot, hhfm_stream_t stream) {
-  return dfm_fwd_bwd_impl(idx, B, F, V, feature_bias, M, K, params, n_layers, layer_sizes, labels, workspace, out, gV, gbias,
-                          gparams, loss_partials, hot_slot, ghot, ghot_bias, n_rep, n_hot, stream, 0, nullptr, nullptr);
+  return hhfm_dfm_fwd_bwd_mode(idx, B, F, V, feature_bias, M, K, params, n_layers, layer_sizes, 0, B, labels, workspace, out, gV,
+                               gbias, gparams, loss_partials, hot_slot, ghot, ghot_bias, n_rep, n_hot, stream);
 }
 
 // Wide&Deep deep part (WDMF.py:57-73): the DeepFM tower with its FM terms off; `extra` [B] is the wide logit, `out` the summed
@@ -906,7 +1006,8 @@ extern "C" int hhfm_dfm_fwd_bwd_sqloss(const int32_t* idx, int64_t B, int64_t F,
 extern "C" int hhfm_wd_deep_fwd(const int32_t* idx, int64_t B, int64_t F, const float* V, int64_t M, int64_t K,
                                 const float* params, int32_t n_layers, const int32_t* layer_sizes, const float* extra,
                                 float* workspace, float* out, hhfm_stream_t stream) {
-  return dfm_fwd_impl(idx, B, F, V, nullptr, M, K, params, n_layers, layer_sizes, workspace, out, stream, 1, extra);
+  return dfm_fwd_impl(idx, B, F, V, nullptr, M, K, params, n_layers, layer_sizes, workspace, out, stream, HHFM_DFM_NO_FM | kDfmWd,
+                      extra);
 }
 
 extern "C" int hhfm_wd_deep_fwd_bwd_logloss(const int32_t* idx, int64_t B, int64_t F, const float* V, int64_t M, int64_t K,
@@ -916,14 +1017,16 @@ extern "C" int hhfm_wd_deep_fwd_bwd_logloss(const int32_t* idx, int64_t B, int64
                                             const int32_t* hot_slot, float* ghot, int32_t n_rep, int32_t n_hot,
                                             hhfm_stream_t stream) {
   return dfm_fwd_bwd_impl(idx, B, F, V, nullptr, M, K, params, n_layers, layer_sizes, labels, workspace, out, gV, nullptr, gparams,
-                          loss_partials, hot_slot, ghot, nullptr, n_rep, n_hot, stream, 1, extra, gsample);
+                          loss_partials, hot_slot, ghot, nullptr, n_rep, n_hot, stream, HHFM_DFM_NO_FM | kDfmWd, B, extra, gsample);
 }
 
-extern "C" int64_t hhfm_workspace_bytes_dfm_topn(int64_t C, int64_t N, int64_t F, int64_t K, int32_t n_layers,
-                                                 const int32_t* layer_sizes) {
+extern "C" int64_t hhfm_workspace_bytes_dfm_topn_mode(int64_t C, int64_t N, int64_t F, int64_t K, int32_t n_layers,
+                                                      const int32_t* layer_sizes, int32_t mode) {
   DfmLayout lo;
-  if (C < 0 || N < 1 || dfm_layout(C * N, F, K, n_layers, layer_sizes, lo) != HHFM_OK) return -1;
-  const int64_t side = dfm_topn_side_floats(C, N, K, lo.ld[1]);
+  if (dfm_check_mode(mode) != HHFM_OK) return -1;
+  if (C < 0 || N < 1 || dfm_layout(C * N, F, K, n_layers, layer_sizes, lo, mode) != HHFM_OK) return -1;
+  const int64_t side = dfm_topn_side_floats(C, N, K, lo.ld[1], mode);
+  if (!dfm_deep(mode)) return side * (int64_t)sizeof(float);      // no tower activations for the C*N rows
   if (dfm_use_tc(K)) {
     DfmTcLayout t;
     dfm_tc_layout(C * N, lo, t, 1);
@@ -932,18 +1035,26 @@ extern "C" int64_t hhfm_workspace_bytes_dfm_topn(int64_t C, int64_t N, int64_t F
   return (side + lo.ws_floats) * (int64_t)sizeof(float);
 }
 
-extern "C" int hhfm_dfm_topn_scores(const int32_t* rows, int64_t row_stride, int64_t C, int64_t F, int32_t item_col,
-                                    const float* V, const float* feature_bias, int64_t M, int64_t K, const float* params,
-                                    int32_t n_layers, const int32_t* layer_sizes, int64_t item_base, int64_t N,
-                                    float* workspace, float* scores, hhfm_stream_t stream) {
-  HHFM_REQUIRE(rows && V && feature_bias && params && workspace && scores, "dfm_topn_scores: NULL argument");
+extern "C" int64_t hhfm_workspace_bytes_dfm_topn(int64_t C, int64_t N, int64_t F, int64_t K, int32_t n_layers,
+                                                 const int32_t* layer_sizes) {
+  return hhfm_workspace_bytes_dfm_topn_mode(C, N, F, K, n_layers, layer_sizes, 0);
+}
+
+extern "C" int hhfm_dfm_topn_scores_mode(const int32_t* rows, int64_t row_stride, int64_t C, int64_t F, int32_t item_col,
+                                         const float* V, const float* feature_bias, int64_t M, int64_t K, const float* params,
+                                         int32_t n_layers, const int32_t* layer_sizes, int32_t mode, int64_t item_base, int64_t N,
+                                         float* workspace, float* scores, hhfm_stream_t stream) {
+  int rc = dfm_check_mode(mode);
+  if (rc != HHFM_OK) return rc;
+  const bool fm = dfm_fm(mode), deep = dfm_deep(mode);
+  HHFM_REQUIRE(rows && V && (feature_bias || !fm) && params && workspace && scores, "dfm_topn_scores: NULL argument");
   HHFM_REQUIRE(C >= 0 && N >= 1 && C * N < (1ll << 31) && item_base >= 0 && item_base + N <= M, "dfm_topn_scores: bad C / N / item_base");
   HHFM_REQUIRE(item_col >= 0 && item_col < F && row_stride >= F, "dfm_topn_scores: bad item_col / row_stride");
   HHFM_REQUIRE(((uintptr_t)workspace & 15) == 0, "dfm_topn_scores: workspace must be 16-byte aligned");
   if (C == 0) return HHFM_OK;
   const int64_t B = C * N;
   DfmLayout lo;
-  int rc = dfm_layout(B, F, K, n_layers, layer_sizes, lo);
+  rc = dfm_layout(B, F, K, n_layers, layer_sizes, lo, mode);
   if (rc != HHFM_OK) return rc;
   HHFM_REQUIRE(F * K * sizeof(float) <= 200 * 1024, "dfm_topn_scores: F*K too large for the context kernel");
   cudaStream_t st = (cudaStream_t)stream;
@@ -952,8 +1063,9 @@ extern "C" int hhfm_dfm_topn_scores(const int32_t* rows, int64_t row_stride, int
   a.rows = rows; a.row_stride = row_stride; a.C = (int)C; a.F = (int)F; a.K = (int)K; a.item_col = item_col; a.d1 = lo.d[1]; a.ld1 = ld1;
   a.V = V; a.fbias = feature_bias; a.W1 = params + lo.w_off[0]; a.b1 = params + lo.b_off[0]; a.proj = params + lo.proj_off;
   a.item_base = item_base; a.N = N;
-  a.U = workspace; a.T = a.U + C * ld1; a.SQ = a.T + N * ld1; a.fo = a.SQ + C * 2 * K;
-  float* main_ws = workspace + dfm_topn_side_floats(C, N, K, ld1);
+  a.fm = fm ? 1 : 0; a.deep = deep ? 1 : 0; a.sig = (mode & HHFM_DFM_LOGLOSS) ? 1 : 0;
+  a.U = workspace; a.T = a.U + (deep ? C * ld1 : 0); a.SQ = a.T + (deep ? N * ld1 : 0); a.fo = a.SQ + C * 2 * K;
+  float* main_ws = workspace + dfm_topn_side_floats(C, N, K, ld1, mode);
   {
     const size_t smem = (size_t)F * K * sizeof(float);
     if (smem > 48 * 1024 &&
@@ -963,14 +1075,17 @@ extern "C" int hhfm_dfm_topn_scores(const int32_t* rows, int64_t row_stride, int
     }
     dfm_topn_ctx_kernel<<<(unsigned)C, 256, smem, st>>>(a);
     if ((rc = check_launch("dfm_topn_ctx_kernel"))) return rc;
-    dfm_topn_item_kernel<<<(unsigned)((N + 7) / 8), 256, 8 * K * sizeof(float), st>>>(a);
-    if ((rc = check_launch("dfm_topn_item_kernel"))) return rc;
+    if (deep) {
+      dfm_topn_item_kernel<<<(unsigned)((N + 7) / 8), 256, 8 * K * sizeof(float), st>>>(a);
+      if ((rc = check_launch("dfm_topn_item_kernel"))) return rc;
+    }
   }
-  const float* H;
-  int64_t ldh;
-  int n_part = 0;
+  const float* H = nullptr;
+  int64_t ldh = 0;
+  int n_part = 0, D = 0;
   const int h1_grid = (int)std::min<int64_t>((B * (ld1 >> 2) + 255) / 256, (int64_t)sm_count() * 16);
-  if (dfm_use_tc(K)) {
+  // FM part only (!deep): the head kernel reads SQ / fo and the item's row; nothing per (row, item) is materialised
+  if (deep && dfm_use_tc(K)) {
     DfmTcLayout t;
     dfm_tc_layout(B, lo, t, 1);
     dfm_topn_h1_kernel<<<h1_grid, 256, 0, st>>>(a.U, a.T, C, N, ld1, main_ws + t.x[1], main_ws + t.xlo[1], t.ldx[1]);
@@ -979,15 +1094,23 @@ extern "C" int hhfm_dfm_topn_scores(const int32_t* rows, int64_t row_stride, int
     if ((rc = dfm_tc_forward(nullptr, B, F, V, K, params, lo, t, main_ws, false, st, 1, true,
                              fuse_proj ? params + lo.proj_off + F + K : nullptr)))
       return rc;
-    H = main_ws + t.x[lo.L]; ldh = t.ldx[lo.L];
+    H = main_ws + t.x[lo.L]; ldh = t.ldx[lo.L]; D = lo.d[lo.L];
     n_part = fuse_proj ? tf_proj_partials(lo.d[lo.L]) : 0;
-  } else {
+  } else if (deep) {
     dfm_topn_h1_kernel<<<h1_grid, 256, 0, st>>>(a.U, a.T, C, N, ld1, main_ws + lo.h_off[1], nullptr, lo.ld[1]);
     if ((rc = check_launch("dfm_topn_h1_kernel"))) return rc;
     if ((rc = dfm_forward(nullptr, B, F, V, K, params, lo, main_ws, st, 1))) return rc;
-    H = main_ws + lo.h_off[lo.L]; ldh = lo.ld[lo.L];
+    H = main_ws + lo.h_off[lo.L]; ldh = lo.ld[lo.L]; D = lo.d[lo.L];
   }
   const int head_grid = (int)std::min<int64_t>((B + 7) / 8, (int64_t)sm_count() * 8);
-  dfm_topn_head_kernel<<<head_grid, 256, 0, st>>>(a, H, ldh, lo.d[lo.L], n_part, params + lo.cbias_off, scores);
+  dfm_topn_head_kernel<<<head_grid, 256, 0, st>>>(a, H, ldh, D, n_part, params + lo.cbias_off, scores);
   return check_launch("dfm_topn_head_kernel");
+}
+
+extern "C" int hhfm_dfm_topn_scores(const int32_t* rows, int64_t row_stride, int64_t C, int64_t F, int32_t item_col,
+                                    const float* V, const float* feature_bias, int64_t M, int64_t K, const float* params,
+                                    int32_t n_layers, const int32_t* layer_sizes, int64_t item_base, int64_t N,
+                                    float* workspace, float* scores, hhfm_stream_t stream) {
+  return hhfm_dfm_topn_scores_mode(rows, row_stride, C, F, item_col, V, feature_bias, M, K, params, n_layers, layer_sizes, 0,
+                                   item_base, N, workspace, scores, stream);
 }

@@ -1156,9 +1156,16 @@ class AFM(FM):
 
 
 # ====================================================================================================
+DFM_NO_FM, DFM_NO_DEEP, DFM_LOGLOSS = 1, 2, 4      # hhfm_dfm_mode (include/hhfm_sm100.h)
+
+
 class DeepFM(_Base):
     """DeepFM, Newcode/DFM.py:50-232.  FM first/second-order parts + a relu MLP tower over the flattened embeddings,
     joined by `concat_projection`; Adagrad only (DFM.py:153); l2 on the projection and the layer matrices (:145-150).
+
+    use_fm=False / use_deep=False drop the FM part / the tower from the graph (their variables are still created and
+    initialised, and never move); loss_type='logloss' makes `out` the sigmoid and the loss tf.losses.log_loss (mean over
+    the batch, epsilon 1e-7).
 
     All dense variables live in ONE flat device buffer (layout: include/hhfm_sm100.h, K8); `weights[...]` are views."""
 
@@ -1184,9 +1191,6 @@ class DeepFM(_Base):
         self._init_graph()
 
     def _init_graph(self):
-        if not (self.use_fm and self.use_deep) or self.loss_type != "mse":
-            raise NotImplementedError("only use_fm=use_deep=True, loss_type='mse' (what DFM.py:257-259 builds) is on the "
-                                      "accelerated path")
         act = self.deep_layers_activation
         if not (act == "relu" or getattr(act, "__name__", "") == "relu"):
             raise NotImplementedError("deep_layers_activation must be relu (DFM.py:258 passes tf.nn.relu)")
@@ -1201,10 +1205,12 @@ class DeepFM(_Base):
         gen.manual_seed(int(self.random_seed) + 1)
         self.weights["feature_bias"].copy_(torch.empty(self._M, 1).uniform_(0.0, 1.0, generator=gen))   # DFM.py:180-181
         self._sizes = np.asarray(self.deep_layers, dtype=np.int32)
+        self._mode = (0 if self.use_fm else DFM_NO_FM) | (0 if self.use_deep else DFM_NO_DEEP) | \
+            (DFM_LOGLOSS if self.loss_type == "logloss" else 0)
         lib = _lib.load()
         sp = self._sizes.ctypes.data
-        n_par = int(lib.hhfm_dfm_param_count(F, K, L, sp))
-        self._n_reg = int(lib.hhfm_dfm_reg_count(F, K, L, sp))
+        n_par = int(lib.hhfm_dfm_param_count_mode(F, K, L, sp, self._mode))
+        self._n_reg = int(lib.hhfm_dfm_reg_count_mode(F, K, L, sp, self._mode))
         if n_par < 0:
             raise _lib.HhfmError("DeepFM: %s" % lib.hhfm_last_error().decode())
         self._params = torch.zeros(n_par, dtype=torch.float32, device=dev)
@@ -1218,8 +1224,12 @@ class DeepFM(_Base):
             self.weights["layer_%d" % i] = self._params[off:off + n].view(dims[i], dims[i + 1])
             self.weights["layer_%d" % i].copy_(torch.tensor(rs.normal(0, glorot, (dims[i], dims[i + 1])), dtype=torch.float32))
             off += n
-        n_in = F + K + dims[-1]
-        self.weights["concat_projection"] = self._params[off:off + n_in].view(n_in, 1)        # DFM.py:201-210
+        # the projection block is F + K + D wide in every mode; the reference's (input_size, 1) variable is the slice the
+        # mode uses (DFM.py:201-210), the rest stays zero.  Without the tower the block starts on a multiple of 4 elements.
+        self._proj_off = off if self.use_deep else (off + 3) // 4 * 4
+        p0 = self._proj_off + (0 if self.use_fm else F + K)
+        n_in = (F + K if self.use_fm else 0) + (dims[-1] if self.use_deep else 0)
+        self.weights["concat_projection"] = self._params[p0:p0 + n_in].view(n_in, 1)
         self.weights["concat_projection"].copy_(torch.tensor(rs.normal(0, np.sqrt(2.0 / (n_in + 1)), (n_in, 1)), dtype=torch.float32))
         off = self._n_reg                      # the regularised block is zero-padded to a multiple of 4 elements
         for i in range(L):
@@ -1227,13 +1237,14 @@ class DeepFM(_Base):
             self.weights["bias_%d" % i] = self._params[off:off + dims[i + 1]].view(1, dims[i + 1])
             self.weights["bias_%d" % i].copy_(torch.tensor(rs.normal(0, glorot, (1, dims[i + 1])), dtype=torch.float32))
             off += dims[i + 1]
+        self._cbias_off = off
         self.weights["concat_bias"] = self._params[off:off + 1].view(())
         self.weights["concat_bias"].fill_(0.01)                                               # DFM.py:211
         self._ws = None
 
     def _workspace(self, B):
-        need = int(_lib.load().hhfm_workspace_bytes_dfm(B, int(self.field_size), self._K, len(self.deep_layers),
-                                                        self._sizes.ctypes.data)) // 4
+        need = int(_lib.load().hhfm_workspace_bytes_dfm_mode(B, int(self.field_size), self._K, len(self.deep_layers),
+                                                             self._sizes.ctypes.data, self._mode)) // 4
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(max(need, 1), dtype=torch.float32, device=self.device)
         return self._ws
@@ -1244,10 +1255,23 @@ class DeepFM(_Base):
     def _forward_dev(self, idx):
         B, F = idx.shape
         out = torch.empty(B, dtype=torch.float32, device=self.device)
-        _lib.call("hhfm_dfm_fwd", ptr(idx), B, F, ptr(self.weights["feature_embeddings"]), ptr(self.weights["feature_bias"]),
-                  self._M, self._K, ptr(self._params), len(self.deep_layers), self._sizes.ctypes.data,
+        _lib.call("hhfm_dfm_fwd_mode", ptr(idx), B, F, ptr(self.weights["feature_embeddings"]), self._fbias_arg(), self._M,
+                  self._K, ptr(self._params), len(self.deep_layers), self._sizes.ctypes.data, self._mode,
                   ptr(self._workspace(B)), ptr(out), cur_stream())
         return out
+
+    def _fbias_arg(self):
+        return ptr(self.weights["feature_bias"]) if self.use_fm else None
+
+    def _global_batch(self, B):
+        """The batch the log_loss mean runs over: B on one GPU, the sum of the ranks' batch sizes under data parallelism."""
+        if self._dp_group is None:
+            return B
+        import torch.distributed as dist
+        ws = dist.get_world_size(self._dp_group)
+        sizes = [torch.zeros(1, dtype=torch.int64, device=self.device) for _ in range(ws)]
+        dist.all_gather(sizes, torch.tensor([B], dtype=torch.int64, device=self.device), group=self._dp_group)
+        return int(sum(int(t.item()) for t in sizes))
 
     def predict(self, X):
         X = np.asarray(X)
@@ -1267,32 +1291,47 @@ class DeepFM(_Base):
             raise _lib.HhfmError("DeepFM: X has %d columns, field_size is %d" % (F, self.field_size))
         self._opt.begin_step()
         V, fb = self.weights["feature_embeddings"], self.weights["feature_bias"]
-        hot = self._hot_plan(idx, True)
-        _lib.call("hhfm_dfm_fwd_bwd_sqloss", ptr(idx), B, F, ptr(V), ptr(fb), self._M, self._K, ptr(self._params),
-                  len(self.deep_layers), self._sizes.ctypes.data, ptr(y), ptr(self._workspace(B)), None, ptr(self._gV),
-                  ptr(self._gb), ptr(self._gparams), ptr(self._loss_partials), *(hot.args(True) if hot else NO_HOT_BIAS),
+        fm = self.use_fm
+        B_total = self._global_batch(B) if self.loss_type == "logloss" else B
+        hot = self._hot_plan(idx, fm)
+        if hot is None:
+            hargs = NO_HOT_BIAS
+        elif fm:
+            hargs = hot.args(True)
+        else:
+            slot, ghot, n_rep, n_hot = hot.args()
+            hargs = (slot, ghot, None, n_rep, n_hot)
+        _lib.call("hhfm_dfm_fwd_bwd_mode", ptr(idx), B, F, ptr(V), self._fbias_arg(), self._M, self._K, ptr(self._params),
+                  len(self.deep_layers), self._sizes.ctypes.data, self._mode, B_total, ptr(y), ptr(self._workspace(B)), None,
+                  ptr(self._gV), ptr(self._gb) if fm else None, ptr(self._gparams), ptr(self._loss_partials), *hargs,
                   cur_stream())
         if hot:
-            hot.fold(self._gV, self._gb)
+            hot.fold(self._gV, self._gb if fm else None)
         if self._dp_group is not None:
             import torch.distributed as dist
             self._allreduce_grads()
             dist.all_reduce(self._gparams, group=self._dp_group)
-        # V / feature_bias get IndexedSlices: Adagrad leaves rows with g = 0 untouched, so the dense kernel is exact
+        # V / feature_bias get IndexedSlices: Adagrad leaves rows with g = 0 untouched, so the dense kernel is exact.
+        # Variables outside the mode's graph (feature_bias without the FM part, the layers without the tower) get no
+        # gradient in TF and are not stepped here: they and their accumulators stay as they are.
         o = self._opt
         self._apply_arena_dense("feature_embeddings", V, self._gV, 0.0, None)
-        self._apply_arena_dense("feature_bias", fb, self._gb, 0.0, None)
+        if fm:
+            self._apply_arena_dense("feature_bias", fb, self._gb, 0.0, None)
         lam = float(self.l2_reg)
         nr = self._n_reg
-        o.apply_dense("dense_reg", self._params[:nr], self._gparams[:nr], lam if lam > 0 else 0.0,
+        r0 = 0 if self.use_deep else self._proj_off         # without the tower: the projection block alone, 16-byte aligned
+        b0 = nr if self.use_deep else self._cbias_off       # without the tower: concat_bias alone
+        o.apply_dense("dense_reg", self._params[r0:nr], self._gparams[r0:nr], lam if lam > 0 else 0.0,
                       self._sq_partials if lam > 0 else None)
-        o.apply_dense("dense_bias", self._params[nr:], self._gparams[nr:], 0.0, None)
+        o.apply_dense("dense_bias", self._params[b0:], self._gparams[b0:], 0.0, None)
         self._enqueue_loss(lam > 0, 0.5 * lam)
 
     def topk(self, A, tp):
         """DFM.py:220-231: every (row, item) pair scored by the forward graph, then top_k (lowest index first on ties).  The
-        item-separable evaluator (hhfm_dfm_topn_scores) pays the first hidden layer once per row and once per item;
-        HHFM_DFM_TOPN_SEPARABLE=0 sends every expanded row through hhfm_dfm_fwd instead (A/B runs, tests)."""
+        item-separable evaluator (hhfm_dfm_topn_scores_mode) pays the first hidden layer once per row and once per item;
+        HHFM_DFM_TOPN_SEPARABLE=0 sends every expanded row through hhfm_dfm_fwd_mode instead (A/B runs, tests).  Under
+        loss_type='logloss' both rank the sigmoid, as the reference's `out` does (saturated items tie at 1.0)."""
         A = np.asarray(A)
         A_dev, stride = self._topn.upload_rows(A, self._M)
         C_rows, F = A.shape
@@ -1301,7 +1340,8 @@ class DeepFM(_Base):
         chunk = max(1, (1 << 21) // max(N, 1))
         if os.environ.get("HHFM_DFM_TOPN_SEPARABLE", "1") != "0":
             L = len(self.deep_layers)
-            need = int(_lib.load().hhfm_workspace_bytes_dfm_topn(min(chunk, C_rows), N, F, self._K, L, self._sizes.ctypes.data)) // 4
+            need = int(_lib.load().hhfm_workspace_bytes_dfm_topn_mode(min(chunk, C_rows), N, F, self._K, L, self._sizes.ctypes.data,
+                                                                      self._mode)) // 4
             if need < 0:
                 raise _lib.HhfmError("hhfm_workspace_bytes_dfm_topn: bad shape")
             if self._ws is None or self._ws.numel() < need:
@@ -1309,9 +1349,9 @@ class DeepFM(_Base):
             for c0 in range(0, C_rows, chunk):
                 c1 = min(C_rows, c0 + chunk)
                 sc = torch.empty(c1 - c0, N, dtype=torch.float32, device=self.device)
-                _lib.call("hhfm_dfm_topn_scores", ptr(A_dev[c0:c1]), stride, c1 - c0, F, 1, ptr(self.weights["feature_embeddings"]),
-                          ptr(self.weights["feature_bias"]), self._M, self._K, ptr(self._params), L, self._sizes.ctypes.data,
-                          self.n_user, N, ptr(self._ws), ptr(sc), cur_stream())
+                _lib.call("hhfm_dfm_topn_scores_mode", ptr(A_dev[c0:c1]), stride, c1 - c0, F, 1,
+                          ptr(self.weights["feature_embeddings"]), self._fbias_arg(), self._M, self._K, ptr(self._params), L,
+                          self._sizes.ctypes.data, self._mode, self.n_user, N, ptr(self._ws), ptr(sc), cur_stream())
                 _lib.call("hhfm_topn_select", ptr(sc), None, None, c1 - c0, N, N, tp, 0, None, ptr(out_ids[c0:c1]), cur_stream())
             return out_ids.cpu().numpy()
         items = torch.arange(self.n_user, self.n_user + N, dtype=torch.int32, device=self.device)

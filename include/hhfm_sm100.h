@@ -45,6 +45,10 @@ typedef enum { HHFM_POOL_SUM = 0, HHFM_POOL_MAX = 1, HHFM_POOL_MEAN = 2 } hhfm_p
 /* optimizer kinds: FM.py:129-136 (tf.train.{Adagrad,Adam,Momentum,GradientDescent}Optimizer) */
 typedef enum { HHFM_OPT_ADAGRAD = 0, HHFM_OPT_ADAM = 1, HHFM_OPT_MOMENTUM = 2, HHFM_OPT_SGD = 3 } hhfm_opt;
 
+/* DeepFM options (K8 *_mode entry points), OR-ed: use_fm=False, use_deep=False, loss_type='logloss'.  0 = the reference's
+ * default (both parts, mse).  NO_FM | NO_DEEP and unknown bits are rejected. */
+typedef enum { HHFM_DFM_NO_FM = 1, HHFM_DFM_NO_DEEP = 2, HHFM_DFM_LOGLOSS = 4 } hhfm_dfm_mode;
+
 /* top-N query kinds */
 typedef enum {
   HHFM_QUERY_USER = 0, /* q = V[user]                      BPR.py:132, MF.py:145          */
@@ -252,6 +256,32 @@ int hhfm_dfm_fwd_bwd_sqloss(const int32_t* idx, int64_t B, int64_t F, const floa
                             float* gparams, float* loss_partials, const int32_t* hot_slot, float* ghot,
                             float* ghot_bias, int32_t n_rep, int32_t n_hot, hhfm_stream_t stream);
 
+/* K8 with the reference's options (mode: hhfm_dfm_mode bits).  The calls above are these with mode 0 (and B_total = B).
+ *   NO_FM     out = H_L . proj3 + cbias: no feature_bias gather / gradient (feature_bias and gbias may be NULL), no FM part
+ *             of gV; the first F + K projection entries are unused and receive zero gradient.
+ *   NO_DEEP   out = [y1 | y2] . proj12 + cbias: no GEMM, no workspace (the queries return 0 bytes; workspace may be NULL),
+ *             the layer matrices / biases receive no gradient.  The projection block starts on a multiple of 4 elements
+ *             (zero padding after the layer matrices), so [proj_off, reg_count) can be stepped and regularised alone.
+ *   LOGLOSS   out = p = sigmoid(logit); loss = tf.losses.log_loss(y, p): sum_s [-y log(p + 1e-7) - (1 - y) log((1 - p) + 1e-7)]
+ *             / B_total, d/d logit = p (1 - p) (-y / (p + 1e-7) + (1 - y) / ((1 - p) + 1e-7)) / B_total.  Labels are used
+ *             as given.  B_total (>= B) is the batch the mean runs over: the sum of the ranks' B under data parallelism.
+ *   Under mse the loss stays 0.5 sum (y - out)^2 and B_total is only checked.  Bad modes fail with HHFM_ERR_BAD_ARG (the
+ *   int64 queries return -1); hhfm_last_error() says why.
+ *   hhfm_dfm_topn_scores_mode: the same scorer per mode; under LOGLOSS the scores are the sigmoid (the reference ranks by
+ *   `out`, so saturated items tie at 1.0f and the lowest index wins in hhfm_topn_select). */
+int64_t hhfm_dfm_param_count_mode(int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes, int32_t mode);
+int64_t hhfm_dfm_reg_count_mode(int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes, int32_t mode);
+int64_t hhfm_workspace_bytes_dfm_mode(int64_t B, int64_t F, int64_t K, int32_t n_layers, const int32_t* layer_sizes,
+                                      int32_t mode);
+int hhfm_dfm_fwd_mode(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* feature_bias, int64_t M,
+                      int64_t K, const float* params, int32_t n_layers, const int32_t* layer_sizes, int32_t mode,
+                      float* workspace, float* out, hhfm_stream_t stream);
+int hhfm_dfm_fwd_bwd_mode(const int32_t* idx, int64_t B, int64_t F, const float* V, const float* feature_bias, int64_t M,
+                          int64_t K, const float* params, int32_t n_layers, const int32_t* layer_sizes, int32_t mode,
+                          int64_t B_total, const float* labels, float* workspace, float* out, float* gV, float* gbias,
+                          float* gparams, float* loss_partials, const int32_t* hot_slot, float* ghot, float* ghot_bias,
+                          int32_t n_rep, int32_t n_hot, hhfm_stream_t stream);
+
 /* K8 full-catalog scorer (DFM.py:219-231): scores [C, N] = the DeepFM forward of every context row with field item_col
  * replaced by item n (table row item_base + n).  The first hidden layer is item-separable, relu((b1 + sum_{f != item}
  * E_f W1_f) + E_n W1_item): its context part is computed once per row and its item part once per item; the remaining layers
@@ -264,6 +294,12 @@ int hhfm_dfm_topn_scores(const int32_t* rows, int64_t row_stride, int64_t C, int
                          const float* feature_bias, int64_t M, int64_t K, const float* params, int32_t n_layers,
                          const int32_t* layer_sizes, int64_t item_base, int64_t N, float* workspace, float* scores,
                          hhfm_stream_t stream);
+int64_t hhfm_workspace_bytes_dfm_topn_mode(int64_t C, int64_t N, int64_t F, int64_t K, int32_t n_layers,
+                                           const int32_t* layer_sizes, int32_t mode);
+int hhfm_dfm_topn_scores_mode(const int32_t* rows, int64_t row_stride, int64_t C, int64_t F, int32_t item_col, const float* V,
+                              const float* feature_bias, int64_t M, int64_t K, const float* params, int32_t n_layers,
+                              const int32_t* layer_sizes, int32_t mode, int64_t item_base, int64_t N, float* workspace,
+                              float* scores, hhfm_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K11  Wide&Deep (WDMF.py:51-126: tf.contrib.learn.DNNLinearCombinedClassifier over hashed columns, crossed columns and
