@@ -29,6 +29,11 @@ SIGNATURES = {
                                   vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64, vp, vp, vp, vp, vp, vp, f32, f32, vp, i64,
                                   vp],
     "hhfm_fm_bn_fwd": [vp, i64, i64, vp, vp, vp, i64, i64, vp, vp, vp, vp, f32, vp, vp],
+    "hhfm_fm_bn_sync_stats": [vp, i64, i64, vp, vp, i64, i64, vp, vp, i64, vp],
+    "hhfm_fm_bn_sync_loss": [i64, i64, vp, vp, vp, vp, vp, f32, C.c_uint64, vp, vp, vp, vp, f32, f32, vp, i32, i32, vp, vp, i64,
+                             vp],
+    "hhfm_fm_bn_sync_scatter": [vp, i64, i64, vp, i64, i64, vp, vp, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64,
+                                vp, vp, vp, i32, vp, i64, vp],
     "hhfm_fm_bwd": [vp, vp, vp, i64, i64, vp, i64, i64, i32, vp, vp, vp, vp, i32, vp],
     "hhfm_afm_fwd": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, vp, vp],
     "hhfm_afm_fwd_bwd_sqloss": [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp,
@@ -108,6 +113,8 @@ INT64_FUNCS = {
     "hhfm_workspace_bytes_dfm_mode": [i64, i64, i64, i32, vp, i32],
     "hhfm_workspace_bytes_dfm_topn_mode": [i64, i64, i64, i64, i32, vp, i32],
     "hhfm_workspace_bytes_fm_bn": [i64, i64],
+    "hhfm_workspace_bytes_fm_bn_sync": [i64, i64],
+    "hhfm_fm_bn_sync_len": [i64],
 }
 OPTIONAL = {}   # symbols added by later kernels are appended by their modules via `declare`
 

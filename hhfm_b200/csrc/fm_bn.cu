@@ -14,6 +14,11 @@
 //                            gV[x_f] += dx (S - e_f), gbias[x_f] += g with the hot-row plan and the touched-row list
 // Every value that leaves the step except the row gradients (float atomics, as in fm_kernel) is a fixed-order reduction,
 // so the batch statistics, the loss, d gamma, d beta, d b0 and the moving statistics are bit-identical from run to run.
+// Synchronised batch norm (data parallelism, DESIGN.md 7) runs the same passes as three phases with an all-gather of one
+// small double vector per rank between them: passes 2 and 4 stop before finalising and write this rank's merged
+// (n, mean, M2) / (sum g, sum d, sum d xhat); the next phase merges the gathered vectors of all ranks in rank order
+// (fm_bn_rank_merge_kernel) and finalises with the same code as the single call.  With one rank the phases reproduce
+// the single call bit for bit: a double partial merged into an empty state is itself.
 // Lane mapping: fm.cu's Frag<LPS, VPL> (one sample per aligned group of LPS lanes, VPL float4 per lane).
 #include <math.h>
 
@@ -55,6 +60,7 @@ struct FmBnArgs {
   float* g;          // [B]  d loss / d out
   float* part;       // [kPartials, 2K + 1]: pass 1 (mean, M2, n), pass 3 (sum d, sum d xhat, sum g) per CTA
   float* colv;       // [5, K]: mu, 1/sqrt(var + eps), gamma/sqrt(var + eps), dbeta / B, dgamma / B
+  int64_t* glob;     // synchronised phases only (NULL in the single call): [global batch size, global index of sample 0]
 };
 
 static inline size_t bn_align(size_t b) { return (b + 255) / 256 * 256; }
@@ -64,13 +70,17 @@ static size_t fm_bn_ws_bytes(int64_t B, int64_t K) {
          bn_align((size_t)5 * K * 4);
 }
 
-static void fm_bn_ws_bind(FmBnArgs& a, void* ws) {
+// the synchronised phases: the same layout plus the global batch size and index base
+static size_t fm_bn_sync_ws_bytes(int64_t B, int64_t K) { return fm_bn_ws_bytes(B, K) + bn_align(2 * sizeof(int64_t)); }
+
+static void fm_bn_ws_bind(FmBnArgs& a, void* ws, bool sync = false) {
   char* p = static_cast<char*>(ws);
   a.x = reinterpret_cast<float*>(p);     p += bn_align((size_t)a.B * a.K * 4);
   a.bsum = reinterpret_cast<float*>(p);  p += bn_align((size_t)a.B * 4);
   a.g = reinterpret_cast<float*>(p);     p += bn_align((size_t)a.B * 4);
   a.part = reinterpret_cast<float*>(p);  p += bn_align((size_t)kPartials * (2 * a.K + 1) * 4);
-  a.colv = reinterpret_cast<float*>(p);
+  a.colv = reinterpret_cast<float*>(p);  p += bn_align((size_t)5 * a.K * 4);
+  a.glob = sync ? reinterpret_cast<int64_t*>(p) : nullptr;
 }
 
 __device__ __forceinline__ float4 f4_div(float4 a, float s) { return make_float4(a.x / s, a.y / s, a.z / s, a.w / s); }
@@ -118,6 +128,51 @@ __device__ __forceinline__ void chan_merge(float& n, float& mean, float& m2, flo
   mean = mean + d * (nb / nn);
   m2 = m2 + m2b + d * d * (n * nb / nn);
   n = nn;
+}
+
+// Chan's formula in double: the merge of CTA partials (pass 2) and of the ranks' partials (synchronised phases)
+__device__ __forceinline__ void chan_merge_d(double& n, double& mean, double& m2, double nb, double mb, double m2b) {
+  if (nb == 0.0) return;
+  const double nn = n + nb, d = mb - mean;
+  mean += d * (nb / nn);
+  m2 += m2b + d * d * (n * nb / nn);
+  n = nn;
+}
+
+// Global index of local sample 0 for the dropout mask: the synchronised phases draw the mask of the sample's index in the
+// global batch (the sizes of the lower ranks before it); the single call starts at 0.
+__device__ __forceinline__ int64_t bn_index_base(const FmBnArgs& a) { return a.glob ? a.glob[1] : 0; }
+
+// Column c from the merged (n, mean, M2) of the batch: mu, 1/sqrt(var + eps), gamma/sqrt(var + eps); the moving statistics
+// move towards mu and the Bessel-corrected variance.  Biased batch variance for the normalisation, n - 1 taken as 1 when
+// n = 1 (the fused batch-norm kernel of tf.contrib.layers.batch_norm, DESIGN.md 7).  An empty batch leaves the layer as is.
+__device__ __forceinline__ void bn_finish_stats(const FmBnArgs& a, int c, double n, double mean, double m2) {
+  const int K = a.K;
+  if (n == 0.0) {
+    a.colv[c] = 0.f;
+    a.colv[K + c] = 0.f;
+    a.colv[2 * K + c] = 0.f;
+    return;
+  }
+  const float mu = (float)mean, var = (float)(m2 / n);
+  const float var_u = (float)(m2 / (n > 1.0 ? n - 1.0 : 1.0));
+  const float is = 1.f / sqrtf(var + a.eps);
+  const float f = 1.f - a.decay;
+  a.mm[c] = a.mm[c] - (a.mm[c] - mu) * f;
+  a.mv[c] = a.mv[c] - (a.mv[c] - var_u) * f;
+  a.colv[c] = mu;
+  a.colv[K + c] = is;
+  a.colv[2 * K + c] = a.gamma[c] * is;
+}
+
+// Column c from the batch sums of d and d xhat: d beta, d gamma and their means over the n samples of the batch.
+__device__ __forceinline__ void bn_finish_sums(const FmBnArgs& a, int c, double n, double sd, double sdx) {
+  const int K = a.K;
+  const float db = (float)sd, dg = (float)sdx;
+  a.dbeta[c] = db;
+  a.dgamma[c] = dg;
+  a.colv[3 * K + c] = n > 0.0 ? db / (float)n : 0.f;
+  a.colv[4 * K + c] = n > 0.0 ? dg / (float)n : 0.f;
 }
 
 // ---- pass 1 -----------------------------------------------------------------------------------------------------
@@ -199,6 +254,7 @@ __global__ void __launch_bounds__(kBlock, 1) fm_bn_loss_kernel(const FmBnArgs a)
   frag_load(ga, a.gamma, 0, K, lg);
   frag_load(be, a.beta, 0, K, lg);
   float loss_acc = 0.f, g_acc = 0.f;
+  const int64_t sb = bn_index_base(a);
   for (int64_t s0 = warp_g * G; s0 < a.B; s0 += n_warps * G) {
     const int64_t s = s0 + grp;
     const bool valid = s < a.B;
@@ -210,7 +266,7 @@ __global__ void __launch_bounds__(kBlock, 1) fm_bn_loss_kernel(const FmBnArgs a)
       xh.v[i] = f4_mul(f4_sub(x.v[i], mu.v[i]), is.v[i]);
       float4 z = f4_add(f4_mul(ga.v[i], xh.v[i]), be.v[i]);         // zero in the padding columns (gamma, beta read 0)
       if constexpr (DROP) {
-        m.v[i] = bn_mask(a, valid ? s : 0, 4 * (lg + i * LPS));
+        m.v[i] = bn_mask(a, sb + (valid ? s : 0), 4 * (lg + i * LPS));
         z = f4_mul(f4_div(z, a.keep), m.v[i]);
       }
       part += f4_hsum(z);
@@ -266,11 +322,13 @@ __global__ void __launch_bounds__(kBlock, 1) fm_bn_loss_kernel(const FmBnArgs a)
 
 // ---- passes 2 and 4: the CTA partials of `n_part` CTAs, one CTA, fixed order --------------------------------------
 // Thread t takes column c = cb + t % cols and the partials seg, seg + nseg, ... (seg = t / cols); the nseg segment results
-// of a column are merged in segment order by the thread of segment 0.
+// of a column are merged in segment order by the thread of segment 0.  vec == NULL: finalised for this batch (the single
+// call).  Otherwise the merged partials go to vec [2K + 1] as doubles for the all-gather of the synchronised phases:
+// pass 2 (n, mean[K], M2[K]), pass 4 (sum g, sum d[K], sum d xhat[K]).
 constexpr int kReduceThreads = 1024;     // one CTA does the whole merge: more threads, fewer partials each
 
 template <bool STATS>
-__global__ void __launch_bounds__(kReduceThreads) fm_bn_reduce_kernel(const FmBnArgs a, int n_part) {
+__global__ void __launch_bounds__(kReduceThreads) fm_bn_reduce_kernel(const FmBnArgs a, int n_part, double* vec) {
   __shared__ double sh[3][kReduceThreads];
   const int K = a.K, W = 2 * K + 1;
   const int cols = K < (int)blockDim.x ? K : (int)blockDim.x;
@@ -283,12 +341,7 @@ __global__ void __launch_bounds__(kReduceThreads) fm_bn_reduce_kernel(const FmBn
       for (int p = seg; p < n_part; p += nseg) {
         const float* q = a.part + (size_t)p * W;
         if (STATS) {
-          const double nb = q[2 * K];
-          if (nb == 0.0) continue;
-          const double nn = r0 + nb, d = (double)q[c] - r1;
-          r1 += d * (nb / nn);
-          r2 += (double)q[K + c] + d * d * (r0 * nb / nn);
-          r0 = nn;
+          chan_merge_d(r0, r1, r2, q[2 * K], q[c], q[K + c]);
         } else {
           r0 += q[c];
           r1 += q[K + c];
@@ -305,43 +358,66 @@ __global__ void __launch_bounds__(kReduceThreads) fm_bn_reduce_kernel(const FmBn
       for (int t = 1; t < nseg; t++) {
         const int o = t * cols + threadIdx.x;
         if (STATS) {
-          const double nb = sh[0][o];
-          if (nb == 0.0) continue;
-          const double nn = r0 + nb, d = sh[1][o] - r1;
-          r1 += d * (nb / nn);
-          r2 += sh[2][o] + d * d * (r0 * nb / nn);
-          r0 = nn;
+          chan_merge_d(r0, r1, r2, sh[0][o], sh[1][o], sh[2][o]);
         } else {
           r0 += sh[0][o];
           r1 += sh[1][o];
         }
       }
-      if (STATS) {
-        // normalisation: biased batch variance; moving variance: Bessel-corrected, B - 1 taken as 1 when B = 1 (the fused
-        // batch-norm kernel of tf.contrib.layers.batch_norm, DESIGN.md 7)
-        const float mu = (float)r1, var = (float)(r2 / (double)a.B);
-        const float var_u = (float)(r2 / (double)(a.B > 1 ? a.B - 1 : 1));
-        const float is = 1.f / sqrtf(var + a.eps);
-        const float f = 1.f - a.decay;
-        a.mm[c] = a.mm[c] - (a.mm[c] - mu) * f;
-        a.mv[c] = a.mv[c] - (a.mv[c] - var_u) * f;
-        a.colv[c] = mu;
-        a.colv[K + c] = is;
-        a.colv[2 * K + c] = a.gamma[c] * is;
+      if (vec != nullptr) {
+        if (STATS && c == 0) vec[0] = r0;
+        vec[1 + c] = STATS ? r1 : r0;
+        vec[1 + K + c] = STATS ? r2 : r1;
+      } else if (STATS) {
+        bn_finish_stats(a, c, (double)a.B, r1, r2);
       } else {
-        const float db = (float)r0, dg = (float)r1;
-        a.dbeta[c] = db;
-        a.dgamma[c] = dg;
-        a.colv[3 * K + c] = db / (float)a.B;
-        a.colv[4 * K + c] = dg / (float)a.B;
+        bn_finish_sums(a, c, (double)a.B, r0, r1);
       }
     }
     __syncthreads();
   }
-  if (!STATS && threadIdx.x == 0 && a.gb0 != nullptr) {
+  if (!STATS && threadIdx.x == 0 && (a.gb0 != nullptr || vec != nullptr)) {
     double t = 0.0;
     for (int p = 0; p < n_part; p++) t += a.part[(size_t)p * W + 2 * K];
-    *a.gb0 += (float)t;
+    if (a.gb0 != nullptr) *a.gb0 += (float)t;
+    if (vec != nullptr) vec[0] = t;
+  }
+}
+
+// ---- synchronised phases: the gathered per-rank vectors [n_ranks, 2K + 1], merged in rank order, one CTA ------------
+// STATS: (n, mean, M2) of every rank (Chan) -> finalised as pass 2 does for the global batch; thread 0 records the global
+// batch size and the global index of this rank's first sample.  Else: the sums of d and d xhat of every rank -> d beta,
+// d gamma and their means over the global batch.
+template <bool STATS>
+__global__ void __launch_bounds__(kReduceThreads) fm_bn_rank_merge_kernel(const FmBnArgs a, const double* all, int n_ranks,
+                                                                          int rank) {
+  const int K = a.K, W = 2 * K + 1;
+  if (STATS && threadIdx.x == 0) {
+    int64_t n = 0, base = 0;
+    for (int r = 0; r < n_ranks; r++) {
+      const int64_t nr = (int64_t)all[(size_t)r * W];
+      if (r < rank) base += nr;
+      n += nr;
+    }
+    a.glob[0] = n;
+    a.glob[1] = base;
+  }
+  const double n_glob = STATS ? 0.0 : (double)a.glob[0];      // written by the STATS merge of this step
+  for (int c = threadIdx.x; c < K; c += blockDim.x) {
+    double r0 = 0.0, r1 = 0.0, r2 = 0.0;
+    for (int r = 0; r < n_ranks; r++) {
+      const double* v = all + (size_t)r * W;
+      if (STATS) {
+        chan_merge_d(r0, r1, r2, v[0], v[1 + c], v[1 + K + c]);
+      } else {
+        r0 += v[1 + c];
+        r1 += v[1 + K + c];
+      }
+    }
+    if (STATS)
+      bn_finish_stats(a, c, r0, r1, r2);
+    else
+      bn_finish_sums(a, c, n_glob, r0, r1);
   }
 }
 
@@ -356,6 +432,7 @@ __global__ void __launch_bounds__(kBlock) fm_bn_scatter_kernel(const FmBnArgs a)
   const int K = a.K, kv = K >> 2;
   const int rep = a.hot.slot ? (int)((warp_g * (32 / LPS) + grp) % a.hot.n_rep) : 0;
   const float4* cv = reinterpret_cast<const float4*>(a.colv);
+  const int64_t sb = bn_index_base(a);
   for (int64_t s0 = warp_g * ga; s0 < a.B; s0 += n_warps * ga) {
     const int64_t s = s0 + grp;
     const bool valid = (grp < ga) && (s < a.B);
@@ -370,7 +447,7 @@ __global__ void __launch_bounds__(kBlock) fm_bn_scatter_kernel(const FmBnArgs a)
       dx.v[i] = f4_zero();
       if (c < kv) {
         const float4 xh = f4_mul(f4_sub(bn_interaction(S.v[i], Q.v[i]), ldg4(cv + c)), ldg4(cv + kv + c));
-        const float4 d = DROP ? f4_mul(make_float4(g, g, g, g), f4_div(bn_mask(a, s, 4 * c), a.keep)) : make_float4(g, g, g, g);
+        const float4 d = DROP ? f4_mul(make_float4(g, g, g, g), f4_div(bn_mask(a, sb + s, 4 * c), a.keep)) : make_float4(g, g, g, g);
         dx.v[i] = f4_mul(ldg4(cv + 2 * kv + c), f4_sub(f4_sub(d, ldg4(cv + 3 * kv + c)), f4_mul(xh, ldg4(cv + 4 * kv + c))));
       }
     }
@@ -446,29 +523,77 @@ static int bn_grid(KERN k, int64_t B, int lps) {
   return grid_for(B, (kBlock / 32) * (32 / lps), occ);
 }
 
+// CTAs per SM of passes 1, 3 and 5 (the grid is this times the SMs, capped by B)
+struct BnCaps {
+  int g1, g3, g5;
+};
+
 template <int LPS, int VPL, bool DROP>
-static int launch_fm_bn_train(FmBnArgs a, int deterministic, cudaStream_t st) {
-  static int g1 = 0, g3 = 0, g5 = 0;          // CTAs per SM of each pass (the grid is this times the SMs, capped by B)
-  if (g1 == 0) {
-    g1 = bn_grid(fm_bn_gather_kernel<LPS, VPL>, (int64_t)1 << 40, LPS);
-    g3 = bn_grid(fm_bn_loss_kernel<LPS, VPL, DROP>, (int64_t)1 << 40, LPS);
-    g5 = bn_grid(fm_bn_scatter_kernel<LPS, VPL, DROP>, (int64_t)1 << 40, LPS);
-  }
-  const int64_t per_cta = (kBlock / 32) * (32 / LPS);
-  auto grid = [&](int cap) { const int64_t need = (a.B + per_cta - 1) / per_cta; return (int)(need < cap ? need : cap); };
-  const int n1 = grid(g1), n3 = grid(g3);
-  fm_bn_gather_kernel<LPS, VPL><<<n1, kBlock, 0, st>>>(a);
-  fm_bn_reduce_kernel<true><<<1, kReduceThreads, 0, st>>>(a, n1);
-  fm_bn_loss_kernel<LPS, VPL, DROP><<<n3, kBlock, 0, st>>>(a);
-  fm_bn_reduce_kernel<false><<<1, kReduceThreads, 0, st>>>(a, n3);
+static const BnCaps& bn_caps() {
+  static const BnCaps c{bn_grid(fm_bn_gather_kernel<LPS, VPL>, (int64_t)1 << 40, LPS),
+                        bn_grid(fm_bn_loss_kernel<LPS, VPL, DROP>, (int64_t)1 << 40, LPS),
+                        bn_grid(fm_bn_scatter_kernel<LPS, VPL, DROP>, (int64_t)1 << 40, LPS)};
+  return c;
+}
+
+// CTAs of a pass over B samples: one per (kBlock / 32) * (32 / LPS) samples, at most `cap`, at least one (an empty rank
+// of the synchronised phases still writes its zero partials)
+static int bn_ctas(int64_t B, int lps, int cap) {
+  const int64_t per_cta = (kBlock / 32) * (32 / lps);
+  const int64_t need = (B + per_cta - 1) / per_cta;
+  return need < 1 ? 1 : (int)(need < cap ? need : cap);
+}
+
+template <int LPS, int VPL, bool DROP>
+static void launch_fm_bn_scatter(FmBnArgs a, int deterministic, cudaStream_t st) {
   if (deterministic) {                          // one warp in program order: bit-reproducible row gradients
     a.groups_active = 1;
     fm_bn_scatter_kernel<LPS, VPL, DROP><<<1, 32, 0, st>>>(a);
   } else {
     a.groups_active = 32 / LPS;
-    fm_bn_scatter_kernel<LPS, VPL, DROP><<<grid(g5), kBlock, 0, st>>>(a);
+    fm_bn_scatter_kernel<LPS, VPL, DROP><<<bn_ctas(a.B, LPS, bn_caps<LPS, VPL, DROP>().g5), kBlock, 0, st>>>(a);
   }
+}
+
+template <int LPS, int VPL, bool DROP>
+static int launch_fm_bn_train(FmBnArgs a, int deterministic, cudaStream_t st) {
+  const BnCaps& cap = bn_caps<LPS, VPL, DROP>();
+  const int n1 = bn_ctas(a.B, LPS, cap.g1), n3 = bn_ctas(a.B, LPS, cap.g3);
+  fm_bn_gather_kernel<LPS, VPL><<<n1, kBlock, 0, st>>>(a);
+  fm_bn_reduce_kernel<true><<<1, kReduceThreads, 0, st>>>(a, n1, nullptr);
+  fm_bn_loss_kernel<LPS, VPL, DROP><<<n3, kBlock, 0, st>>>(a);
+  fm_bn_reduce_kernel<false><<<1, kReduceThreads, 0, st>>>(a, n3, nullptr);
+  launch_fm_bn_scatter<LPS, VPL, DROP>(a, deterministic, st);
   return check_launch("fm_bn training kernels");
+}
+
+// synchronised phase 1: pass 1 and the merge of pass 2 into this rank's (n, mean, M2)
+template <int LPS, int VPL>
+static int launch_fm_bn_sync_stats(const FmBnArgs& a, double* stats, cudaStream_t st) {
+  const int n1 = bn_ctas(a.B, LPS, bn_caps<LPS, VPL, false>().g1);
+  fm_bn_gather_kernel<LPS, VPL><<<n1, kBlock, 0, st>>>(a);
+  fm_bn_reduce_kernel<true><<<1, kReduceThreads, 0, st>>>(a, n1, stats);
+  return check_launch("fm_bn_sync_stats kernels");
+}
+
+// synchronised phase 2: the ranks' statistics merged and finalised, pass 3, the merge of pass 4 into this rank's sums
+template <int LPS, int VPL, bool DROP>
+static int launch_fm_bn_sync_loss(const FmBnArgs& a, const double* stats_all, int n_ranks, int rank, double* sums,
+                                  cudaStream_t st) {
+  const int n3 = bn_ctas(a.B, LPS, bn_caps<LPS, VPL, DROP>().g3);
+  fm_bn_rank_merge_kernel<true><<<1, kReduceThreads, 0, st>>>(a, stats_all, n_ranks, rank);
+  fm_bn_loss_kernel<LPS, VPL, DROP><<<n3, kBlock, 0, st>>>(a);
+  fm_bn_reduce_kernel<false><<<1, kReduceThreads, 0, st>>>(a, n3, sums);
+  return check_launch("fm_bn_sync_loss kernels");
+}
+
+// synchronised phase 3: the ranks' sums added in rank order, pass 5
+template <int LPS, int VPL, bool DROP>
+static int launch_fm_bn_sync_scatter(const FmBnArgs& a, const double* sums_all, int n_ranks, int deterministic,
+                                     cudaStream_t st) {
+  fm_bn_rank_merge_kernel<false><<<1, kReduceThreads, 0, st>>>(a, sums_all, n_ranks, 0);
+  launch_fm_bn_scatter<LPS, VPL, DROP>(a, deterministic, st);
+  return check_launch("fm_bn_sync_scatter kernels");
 }
 
 template <int LPS, int VPL>
@@ -481,17 +606,52 @@ static int launch_fm_bn_fwd(const FmBnArgs& a, cudaStream_t st) {
   return check_launch("fm_bn_fwd_kernel");
 }
 
-static int check_bn_common(int64_t B, int64_t F, const void* col, const void* V, int64_t M, int64_t K, const float* gamma,
-                           const float* beta, const float* mm, const float* mv, float eps) {
+static int check_bn_rows(int64_t B, int64_t F, const void* col, const void* V, int64_t M, int64_t K) {
   HHFM_REQUIRE(B >= 0 && M > 0, "fm_bn: bad sizes B=%lld M=%lld", (long long)B, (long long)M);
   HHFM_REQUIRE(col != nullptr && V != nullptr, "fm_bn: col and V must not be NULL");
   HHFM_REQUIRE(K > 0 && K % 4 == 0 && K <= 512, "fm_bn: K=%lld unsupported (need K %% 4 == 0, K <= 512)", (long long)K);
   HHFM_REQUIRE(F > 0, "fm_bn: F=%lld, need F > 0", (long long)F);
-  HHFM_REQUIRE(gamma && beta && mm && mv, "fm_bn: gamma, beta, moving_mean and moving_var must not be NULL");
   HHFM_REQUIRE(((uintptr_t)V & 15) == 0, "fm_bn: V must be 16-byte aligned");
+  return HHFM_OK;
+}
+
+static int check_bn_layer(const float* gamma, const float* beta, const float* mm, const float* mv, float eps) {
+  HHFM_REQUIRE(gamma && beta && mm && mv, "fm_bn: gamma, beta, moving_mean and moving_var must not be NULL");
   HHFM_REQUIRE((((uintptr_t)gamma | (uintptr_t)beta | (uintptr_t)mm | (uintptr_t)mv) & 15) == 0,
                "fm_bn: gamma, beta, moving_mean and moving_var must be 16-byte aligned");
   HHFM_REQUIRE(eps > 0.f && eps < INFINITY, "fm_bn: eps must be > 0 (got %g)", (double)eps);
+  return HHFM_OK;
+}
+
+static int check_bn_common(int64_t B, int64_t F, const void* col, const void* V, int64_t M, int64_t K, const float* gamma,
+                           const float* beta, const float* mm, const float* mv, float eps) {
+  int rc = check_bn_rows(B, F, col, V, M, K);
+  return rc ? rc : check_bn_layer(gamma, beta, mm, mv, eps);
+}
+
+static int check_bn_scatter(const int32_t* touch_stamp, int32_t* touched_rows, int32_t* touched_count, const int32_t* hot_slot,
+                            float* ghot, int32_t n_rep, int32_t n_hot, const float* gV, float keep) {
+  HHFM_REQUIRE(!hot_slot || (ghot && n_rep >= 1 && n_hot >= 1), "fm_bn: hot_slot needs ghot, n_rep, n_hot");
+  HHFM_REQUIRE(!touch_stamp || (touched_rows && touched_count), "fm_bn: touch_stamp needs touched_rows/count");
+  HHFM_REQUIRE(((uintptr_t)gV & 15) == 0, "fm_bn: gV must be 16-byte aligned");
+  HHFM_REQUIRE(keep > 0.f && keep <= 1.f, "fm_bn: dropout keep must be in (0, 1]");
+  return HHFM_OK;
+}
+
+// the arguments every synchronised phase shares: the batch (B may be 0: an empty rank takes part in both all-gathers),
+// the rank layout and the workspace
+static int check_bn_sync(const char* what, int64_t B, int64_t K, int32_t n_ranks, int32_t rank, const void* vec,
+                         const void* workspace, int64_t workspace_bytes) {
+  HHFM_REQUIRE(B >= 0, "%s: bad size B=%lld", what, (long long)B);
+  HHFM_REQUIRE(K > 0 && K % 4 == 0 && K <= 512, "%s: K=%lld unsupported (need K %% 4 == 0, K <= 512)", what, (long long)K);
+  HHFM_REQUIRE(n_ranks >= 1, "%s: n_ranks=%d, need n_ranks >= 1", what, (int)n_ranks);
+  HHFM_REQUIRE(rank >= 0 && rank < n_ranks, "%s: rank=%d outside [0, n_ranks=%d)", what, (int)rank, (int)n_ranks);
+  HHFM_REQUIRE(vec != nullptr, "%s: the per-rank vector must not be NULL", what);
+  HHFM_REQUIRE(((uintptr_t)vec & 7) == 0, "%s: the per-rank vector must be 8-byte aligned", what);
+  const int64_t need = (int64_t)fm_bn_sync_ws_bytes(B, K);
+  HHFM_REQUIRE(workspace != nullptr && ((uintptr_t)workspace & 15) == 0, "%s: workspace must be non-NULL and 16-byte aligned", what);
+  HHFM_REQUIRE(workspace_bytes >= need, "%s: workspace of %lld bytes, need %lld (hhfm_workspace_bytes_fm_bn_sync)", what,
+               (long long)workspace_bytes, (long long)need);
   return HHFM_OK;
 }
 
@@ -520,10 +680,8 @@ extern "C" int hhfm_fm_bn_fwd_bwd_sqloss(const int32_t* row_ptr, const int32_t* 
   HHFM_REQUIRE(labels && gV && loss_partials, "fm_bn: labels, gV and loss_partials are required");
   HHFM_REQUIRE(dgamma && dbeta, "fm_bn: dgamma and dbeta must not be NULL");
   HHFM_REQUIRE(B > 0, "fm_bn: empty batch");
-  HHFM_REQUIRE(!hot_slot || (ghot && n_rep >= 1 && n_hot >= 1), "fm_bn: hot_slot needs ghot, n_rep, n_hot");
-  HHFM_REQUIRE(!touch_stamp || (touched_rows && touched_count), "fm_bn: touch_stamp needs touched_rows/count");
-  HHFM_REQUIRE(((uintptr_t)gV & 15) == 0, "fm_bn: gV must be 16-byte aligned");
-  HHFM_REQUIRE(keep > 0.f && keep <= 1.f, "fm_bn: dropout keep must be in (0, 1]");
+  rc = check_bn_scatter(touch_stamp, touched_rows, touched_count, hot_slot, ghot, n_rep, n_hot, gV, keep);
+  if (rc) return rc;
   HHFM_REQUIRE(decay >= 0.f && decay < 1.f, "fm_bn: decay must be in [0, 1) (got %g)", (double)decay);
   const int64_t need = (int64_t)fm_bn_ws_bytes(B, K);
   HHFM_REQUIRE(workspace != nullptr && ((uintptr_t)workspace & 15) == 0, "fm_bn: workspace must be non-NULL and 16-byte aligned");
@@ -545,6 +703,95 @@ extern "C" int hhfm_fm_bn_fwd_bwd_sqloss(const int32_t* row_ptr, const int32_t* 
 #undef CALL
   } else {
 #define CALL(L, Vp) return launch_fm_bn_train<L, Vp, false>(a, deterministic, st)
+    HHFM_DISPATCH_K(a.K, CALL);
+#undef CALL
+  }
+  return HHFM_ERR_UNSUPPORTED;
+}
+
+extern "C" int64_t hhfm_workspace_bytes_fm_bn_sync(int64_t B, int64_t K) {
+  if (B < 0 || K <= 0 || K > 512) return -1;
+  return (int64_t)fm_bn_sync_ws_bytes(B, K);
+}
+
+extern "C" int64_t hhfm_fm_bn_sync_len(int64_t K) {
+  if (K <= 0 || K > 512) return -1;
+  return 2 * K + 1;
+}
+
+extern "C" int hhfm_fm_bn_sync_stats(const int32_t* col, int64_t B, int64_t F, const float* V, const float* bias, int64_t M,
+                                     int64_t K, double* stats, void* workspace, int64_t workspace_bytes, hhfm_stream_t stream) {
+  int rc = check_bn_sync("fm_bn_sync_stats", B, K, 1, 0, stats, workspace, workspace_bytes);
+  if (rc) return rc;
+  rc = check_bn_rows(B, F, B == 0 && col == nullptr ? (const void*)V : col, V, M, K);     // an empty rank may pass col = NULL
+  if (rc) return rc;
+  FmBnArgs a{};
+  a.col = col; a.B = B; a.F = (int)F; a.K = (int)K; a.V = V; a.bias = bias;
+  fm_bn_ws_bind(a, workspace, true);
+#define CALL(L, Vp) return launch_fm_bn_sync_stats<L, Vp>(a, stats, (cudaStream_t)stream)
+  HHFM_DISPATCH_K(a.K, CALL);
+#undef CALL
+  return HHFM_ERR_UNSUPPORTED;
+}
+
+extern "C" int hhfm_fm_bn_sync_loss(int64_t B, int64_t K, const float* b0, const float* labels, float* out, float* gb0,
+                                    float* loss_partials, float keep, uint64_t drop_seed, const float* gamma, const float* beta,
+                                    float* moving_mean, float* moving_var, float eps, float decay, const double* stats_all,
+                                    int32_t n_ranks, int32_t rank, double* sums, void* workspace, int64_t workspace_bytes,
+                                    hhfm_stream_t stream) {
+  int rc = check_bn_sync("fm_bn_sync_loss", B, K, n_ranks, rank, stats_all, workspace, workspace_bytes);
+  if (rc) return rc;
+  rc = check_bn_layer(gamma, beta, moving_mean, moving_var, eps);
+  if (rc) return rc;
+  HHFM_REQUIRE(sums != nullptr && ((uintptr_t)sums & 7) == 0, "fm_bn_sync_loss: sums must be non-NULL and 8-byte aligned");
+  HHFM_REQUIRE((labels || B == 0) && loss_partials, "fm_bn: labels and loss_partials are required");
+  HHFM_REQUIRE(keep > 0.f && keep <= 1.f, "fm_bn: dropout keep must be in (0, 1]");
+  HHFM_REQUIRE(decay >= 0.f && decay < 1.f, "fm_bn: decay must be in [0, 1) (got %g)", (double)decay);
+  FmBnArgs a{};
+  a.B = B; a.K = (int)K; a.b0 = b0; a.labels = labels; a.out = out; a.gb0 = gb0; a.loss_partials = loss_partials;
+  a.keep = keep; a.drop_seed = drop_seed;
+  a.gamma = gamma; a.beta = beta; a.mm = moving_mean; a.mv = moving_var; a.eps = eps; a.decay = decay;
+  fm_bn_ws_bind(a, workspace, true);
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (keep < 1.f) {
+#define CALL(L, Vp) return launch_fm_bn_sync_loss<L, Vp, true>(a, stats_all, n_ranks, rank, sums, st)
+    HHFM_DISPATCH_K(a.K, CALL);
+#undef CALL
+  } else {
+#define CALL(L, Vp) return launch_fm_bn_sync_loss<L, Vp, false>(a, stats_all, n_ranks, rank, sums, st)
+    HHFM_DISPATCH_K(a.K, CALL);
+#undef CALL
+  }
+  return HHFM_ERR_UNSUPPORTED;
+}
+
+extern "C" int hhfm_fm_bn_sync_scatter(const int32_t* col, int64_t B, int64_t F, const float* V, int64_t M, int64_t K,
+                                       float* gV, float* gbias, int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows,
+                                       int32_t* touched_count, const int32_t* hot_slot, float* ghot, float* ghot_bias,
+                                       int32_t n_rep, int32_t n_hot, int32_t deterministic, float keep, uint64_t drop_seed,
+                                       float* dgamma, float* dbeta, const double* sums_all, int32_t n_ranks, void* workspace,
+                                       int64_t workspace_bytes, hhfm_stream_t stream) {
+  int rc = check_bn_sync("fm_bn_sync_scatter", B, K, n_ranks, 0, sums_all, workspace, workspace_bytes);
+  if (rc) return rc;
+  rc = check_bn_rows(B, F, B == 0 && col == nullptr ? (const void*)V : col, V, M, K);
+  if (rc) return rc;
+  HHFM_REQUIRE(gV != nullptr, "fm_bn: gV is required");
+  HHFM_REQUIRE(dgamma && dbeta, "fm_bn: dgamma and dbeta must not be NULL");
+  rc = check_bn_scatter(touch_stamp, touched_rows, touched_count, hot_slot, ghot, n_rep, n_hot, gV, keep);
+  if (rc) return rc;
+  FmBnArgs a{};
+  a.col = col; a.B = B; a.F = (int)F; a.K = (int)K; a.V = V; a.gV = gV; a.gbias = gbias;
+  a.touch_stamp = touch_stamp; a.stamp = stamp; a.touched_rows = touched_rows; a.touched_count = touched_count;
+  a.hot = HotPlan{hot_slot, ghot, ghot_bias, n_rep, n_hot};
+  a.keep = keep; a.drop_seed = drop_seed; a.dgamma = dgamma; a.dbeta = dbeta;
+  fm_bn_ws_bind(a, workspace, true);
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (keep < 1.f) {
+#define CALL(L, Vp) return launch_fm_bn_sync_scatter<L, Vp, true>(a, sums_all, n_ranks, deterministic, st)
+    HHFM_DISPATCH_K(a.K, CALL);
+#undef CALL
+  } else {
+#define CALL(L, Vp) return launch_fm_bn_sync_scatter<L, Vp, false>(a, sums_all, n_ranks, deterministic, st)
     HHFM_DISPATCH_K(a.K, CALL);
 #undef CALL
   }

@@ -603,10 +603,14 @@ class FM(_Base):
             self._g_bn = torch.zeros(2, K, dtype=torch.float32, device=dev)         # d gamma, d beta
             self._bn_ws = None
 
-    def enable_data_parallel(self, *args, **kwargs):
-        if self._bn:
+    def enable_data_parallel(self, *args, sync_batch_norm=False, **kwargs):
+        """`_Base.enable_data_parallel`.  `sync_batch_norm=True` is required with batch_norm=1: the batch statistics are
+        taken over the global batch (the ranks' shards concatenated in rank order), so the step is the single-GPU step on
+        that batch, at the cost of two small all-gathers per step (DESIGN.md 7).  No effect with batch_norm=0."""
+        if self._bn and not sync_batch_norm:
             raise NotImplementedError("batch_norm=1 under data parallelism: per-rank batch statistics are not the single-GPU "
-                                      "step, and global statistics need two more collectives per step")
+                                      "step; pass sync_batch_norm=True for statistics over the global batch (two more "
+                                      "collectives per step)")
         return super().enable_data_parallel(*args, **kwargs)
 
     def _bn_args(self):
@@ -662,6 +666,9 @@ class FM(_Base):
     def _fit_bn(self, idx, y, ts, stamp, tr, tc, hot, keep, dseed):
         """The step with batch normalisation (csrc/fm_bn.cu): V, feature_bias and the scalar bias go through the usual tail;
         gamma and beta are dense variables without L2, stepped after it."""
+        if self._dp_group is not None:
+            self._fit_bn_sync(idx, y, ts, stamp, tr, tc, hot, keep, dseed)
+            return
         B, F = idx.shape
         nbytes = int(_lib.load().hhfm_workspace_bytes_fm_bn(B, self._K))
         if self._bn_ws is None or self._bn_ws.numel() < nbytes:
@@ -675,6 +682,40 @@ class FM(_Base):
         self._finish_step(hot, True, self._apply_bias)
         self._opt.apply_dense("bn_fm/gamma", self.weights["bn_fm/gamma"], self._g_bn[0], 0.0, None)
         self._opt.apply_dense("bn_fm/beta", self.weights["bn_fm/beta"], self._g_bn[1], 0.0, None)
+
+    def _fit_bn_sync(self, idx, y, ts, stamp, tr, tc, hot, keep, dseed):
+        """Synchronised batch norm: the three phases of csrc/fm_bn.cu with an all-gather of this rank's double vector
+        (statistics, then the sums of d and d xhat) between them, on the current stream and without a host sync.  Every
+        rank merges the same gathered vectors in the same order, so d gamma, d beta and the moving statistics agree bit for
+        bit and gamma / beta take the same optimizer step everywhere (their gradients are global already and are not
+        exchanged); the row gradients, gb0 and the loss partials go through the usual exchange."""
+        import torch.distributed as dist
+        B, F = idx.shape
+        lib = _lib.load()
+        ws_n = dist.get_world_size(self._dp_group)
+        rank = dist.get_rank(self._dp_group)
+        nbytes = int(lib.hhfm_workspace_bytes_fm_bn_sync(B, self._K))
+        if self._bn_ws is None or self._bn_ws.numel() < nbytes:
+            self._bn_ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        L = int(lib.hhfm_fm_bn_sync_len(self._K))
+        if getattr(self, "_bn_vec", None) is None or self._bn_vec.shape != (L,) or self._bn_all.shape[0] != ws_n:
+            self._bn_vec = torch.empty(L, dtype=torch.float64, device=self.device)
+            self._bn_all = torch.empty(ws_n, L, dtype=torch.float64, device=self.device)
+        V, fb, ws, st = self.weights["feature_embeddings"], self.weights["feature_bias"], self._bn_ws, cur_stream()
+        _lib.call("hhfm_fm_bn_sync_stats", ptr(idx), B, F, ptr(V), ptr(fb), self._M, self._K, ptr(self._bn_vec), ptr(ws),
+                  ws.numel(), st)
+        dist.all_gather_into_tensor(self._bn_all, self._bn_vec, group=self._dp_group)
+        w = self.weights
+        _lib.call("hhfm_fm_bn_sync_loss", B, self._K, ptr(self._b0), ptr(y), None, ptr(self._gb0), ptr(self._loss_partials),
+                  keep, dseed, *self._bn_args(), self.BN_EPS, self.BN_DECAY, ptr(self._bn_all), ws_n, rank, ptr(self._bn_vec),
+                  ptr(ws), ws.numel(), st)
+        dist.all_gather_into_tensor(self._bn_all, self._bn_vec, group=self._dp_group)
+        _lib.call("hhfm_fm_bn_sync_scatter", ptr(idx), B, F, ptr(V), self._M, self._K, ptr(self._gV), ptr(self._gb), ts, stamp,
+                  tr, tc, *(hot.args(True) if hot else NO_HOT_BIAS), 1 if self.deterministic else 0, keep, dseed,
+                  ptr(self._g_bn[0]), ptr(self._g_bn[1]), ptr(self._bn_all), ws_n, ptr(ws), ws.numel(), cur_stream())
+        self._finish_step(hot, True, self._apply_bias)
+        self._opt.apply_dense("bn_fm/gamma", w["bn_fm/gamma"], self._g_bn[0], 0.0, None)
+        self._opt.apply_dense("bn_fm/beta", w["bn_fm/beta"], self._g_bn[1], 0.0, None)
 
     def _fused_segments(self):
         n_v, n_b, _ = self._arena_layout

@@ -169,6 +169,41 @@ int64_t hhfm_workspace_bytes_fm_bn(int64_t B, int64_t K);
 int hhfm_fm_bn_fwd(const int32_t* col, int64_t B, int64_t F, const float* V, const float* bias, const float* b0, int64_t M,
                    int64_t K, const float* gamma, const float* beta, const float* moving_mean, const float* moving_var,
                    float eps, float* out, hhfm_stream_t stream);
+/* Synchronised batch norm (data parallelism): the step of hhfm_fm_bn_fwd_bwd_sqloss on the GLOBAL batch (the ranks'
+ * shards concatenated in rank order) as three phases; the caller all-gathers one vector of hhfm_fm_bn_sync_len(K) doubles
+ * per rank between them, stacked in rank order ([n_ranks, 2K + 1]).
+ *   1. hhfm_fm_bn_sync_stats   the interaction vectors of the local rows -> workspace; stats = this rank's
+ *                              (n, mean[K], M2[K]), not finalised.
+ *   2. hhfm_fm_bn_sync_loss    stats_all merged in rank order (Chan's formula in double) -> mu, 1/sqrt(var + eps) and the
+ *                              moving statistics of the global batch (Bessel correction with the global n); out, the loss
+ *                              partials and gb0 (+= local sum g) of the local rows, the dropout mask drawn at each
+ *                              sample's GLOBAL index (lower ranks' sizes + local index); sums = (sum g, sum d[K],
+ *                              sum d xhat[K]) of the local rows.
+ *   3. hhfm_fm_bn_sync_scatter sums_all added in rank order -> dgamma, dbeta (written; the global sums) and the row
+ *                              gradients gV / gbias of the local rows, hot rows and touched-row list as in the single call.
+ * Every rank derives dgamma, dbeta and the moving statistics from the same gathered vectors in the same order, so they
+ * are bit-identical across ranks; gV, gbias, gb0 and the loss partials stay rank-local (the gradient exchange sums them).
+ * B may be 0 (the rank still takes part; col, labels and out may then be NULL); when the global batch is empty the layer
+ * does not move and dgamma = dbeta = 0.  With n_ranks = 1 the phases reproduce hhfm_fm_bn_fwd_bwd_sqloss bit for bit.
+ * The three calls of one step take the same B, K, keep, drop_seed and workspace (hhfm_workspace_bytes_fm_bn_sync(B, K)
+ * bytes, 16-byte aligned); per-rank vectors 8-byte aligned. */
+int hhfm_fm_bn_sync_stats(const int32_t* col, int64_t B, int64_t F, const float* V, const float* bias, int64_t M, int64_t K,
+                          double* stats, void* workspace, int64_t workspace_bytes, hhfm_stream_t stream);
+int hhfm_fm_bn_sync_loss(int64_t B, int64_t K, const float* b0, const float* labels, float* out, float* gb0,
+                         float* loss_partials, float keep, uint64_t drop_seed, const float* gamma, const float* beta,
+                         float* moving_mean, float* moving_var, float eps, float decay, const double* stats_all,
+                         int32_t n_ranks, int32_t rank, double* sums, void* workspace, int64_t workspace_bytes,
+                         hhfm_stream_t stream);
+int hhfm_fm_bn_sync_scatter(const int32_t* col, int64_t B, int64_t F, const float* V, int64_t M, int64_t K, float* gV,
+                            float* gbias, int32_t* touch_stamp, int32_t stamp, int32_t* touched_rows, int32_t* touched_count,
+                            const int32_t* hot_slot, float* ghot, float* ghot_bias, int32_t n_rep, int32_t n_hot,
+                            int32_t deterministic, float keep, uint64_t drop_seed, float* dgamma, float* dbeta,
+                            const double* sums_all, int32_t n_ranks, void* workspace, int64_t workspace_bytes,
+                            hhfm_stream_t stream);
+/* Doubles in one rank's vector of the synchronised phases (2K + 1); -1 for a bad K. */
+int64_t hhfm_fm_bn_sync_len(int64_t K);
+/* Bytes of the workspace of the synchronised phases for B local samples and K factors; -1 for bad sizes. */
+int64_t hhfm_workspace_bytes_fm_bn_sync(int64_t B, int64_t K);
 
 /* Backward only, for torch.autograd: g = gout[s] given by the caller. */
 int hhfm_fm_bwd(const int32_t* row_ptr, const int32_t* col, const float* val, int64_t B, int64_t F,
