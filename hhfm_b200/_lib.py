@@ -68,6 +68,7 @@ SIGNATURES = {
     "hhfm_gather_rows": [vp, vp, i64, i64, i64, vp, i32, vp],
     "hhfm_touch_rows": [vp, i64, vp, i32, vp, vp, vp],
     "hhfm_mark_rows": [vp, i64, vp, i32, i64, vp, vp, vp],
+    "hhfm_touched_compact": [vp, i32, i64, vp, vp, vp],
     "hhfm_opt_adagrad_l2_replay": [vp, vp, vp, vp, vp, i64, i64, i64, f32, f32, i32, vp],
     "hhfm_opt_adagrad_rows_l2": [vp, vp, vp, vp, vp, i64, i64, f32, f32, i32, vp, i32, vp],
     "hhfm_opt_adagrad_dense_l2": [vp, vp, vp, i64, f32, f32, i32, vp, vp],
@@ -85,6 +86,8 @@ SIGNATURES = {
     "hhfm_auc_count": [vp, vp, i64, i32, vp, vp],
     "hhfm_dp_step": [i32, vp, i32, vp, i64, vp, vp, i32, i32, i64, i64, vp, i64, vp, vp, vp, vp, vp, i32, i32, vp, f32, f32, f32,
                      f32, vp, vp, C.c_double, vp],
+    "hhfm_dp_step_touched": [i32, vp, i32, vp, vp, i32, vp, i64, vp, vp, i32, i32, i64, i64, vp, i64, vp, vp, vp, vp, vp, i32,
+                             i32, vp, f32, f32, f32, f32, vp, vp, C.c_double, vp],
     "hhfm_hot_fold": [vp, vp, i32, i32, i64, vp, vp, vp, vp],
     "hhfm_l2_read_sweep": [vp, i64, i32, vp, vp],
     "hhfm_topn_build_query": [i32, vp, i64, i64, i32, i32, i32, i32, i32, vp, i64, i64, vp, vp, vp],
@@ -101,6 +104,7 @@ INT64_FUNCS = {
     "hhfm_workspace_bytes_topn": [i32, i64, i64, i64, i32],
     "hhfm_pack_upload_staging_bytes": [i64, i64, i64],
     "hhfm_dp_exchange_floats": [i64],
+    "hhfm_dp_exchange_floats_touched": [i64],
     "hhfm_dp_flag_ints": [],
     "hhfm_workspace_bytes_dfm_topn": [i64, i64, i64, i64, i32, vp],
     "hhfm_cars2_param_count": [i64, i64, i64, i64, i64, i64],

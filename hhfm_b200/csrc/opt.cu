@@ -480,3 +480,15 @@ extern "C" int hhfm_touch_rows(const int32_t* ids, int64_t n, int32_t* stamp_arr
   touch_rows_kernel<<<(int)(need < cap ? need : cap), 256, 0, (cudaStream_t)stream>>>(ids, n, stamp_arr, stamp, rows, count);
   return check_launch("touch_rows_kernel");
 }
+
+extern "C" int hhfm_touched_compact(const int32_t* stamp_arr, int32_t stamp, int64_t M, int32_t* rows, int32_t* count,
+                                    hhfm_stream_t stream) {
+  HHFM_REQUIRE(stamp_arr && rows && count && M > 0, "touched_compact: bad argument");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (cudaMemsetAsync(count, 0, sizeof(int32_t), st) != cudaSuccess) {
+    set_error("touched_compact: clearing the count failed");
+    cudaGetLastError();
+    return HHFM_ERR_LAUNCH;
+  }
+  return launch_touched_compact(stamp_arr, stamp, M, rows, count, st);
+}

@@ -40,6 +40,7 @@ struct DpSeg {
   int64_t off;   // gradient of w[0, n) = X[off, off + n)
   int64_t n;
   float lamda;
+  int width;     // hhfm_dp_step_touched: row width of an IndexedSlices variable (only touched rows move), 0 = dense
 };
 
 struct OptP2 {
@@ -69,6 +70,8 @@ struct DpArgs {
   float* loss_out;
   long long timeout_cycles;
   int fences;            // 1: explicit system fences around the flag release / acquire (HHFM_DP_FENCES, A/B)
+  const int32_t* stamps; // hhfm_dp_step_touched: [M] touched-row stamps of this rank's scatter kernels
+  int32_t stamp;         //   the current step's stamp
 };
 
 // same expressions as opt.cu::opt_elem, so the fused step is bit-identical to the separate optimizer kernel
@@ -132,7 +135,12 @@ __device__ __forceinline__ bool cross_rank_flags(const DpArgs& a, int phase, int
 
 constexpr int kPiece = 32;      // float4 per piece (512 bytes)
 
-template <int KIND>
+// TOUCHED (hhfm_dp_step_touched): segments with a row width move only the rows stamped on SOME rank.  Every float of a
+// piece has one bit in a 4-word mask stored behind the gradient floats of X (piece p: words 4p .. 4p+3, lane l's float4 in
+// bits 4(l%8) .. 4(l%8)+3 of word l/8).  A: each rank writes the bits of its local stamps; B: the owner ORs the ranks'
+// masks together with the piece sum; C: the update reads the OR.  The bit of a float is the stamp of its row, so a row that
+// straddles two pieces gets the same decision in both.
+template <int KIND, bool TOUCHED>
 __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
   __shared__ float scratch[32];
   __shared__ float s_loss;
@@ -152,6 +160,7 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
   const bool owns_loss = ((p_loss / N) % G) == b;
   float4* arena4 = reinterpret_cast<float4*>(a.arena);
   float4* x4 = reinterpret_cast<float4*>(a.x);
+  uint32_t* xmask = reinterpret_cast<uint32_t*>(x4 + total4);      // TOUCHED, n_ranks > 1: [n_pieces][4] words
 
   // this rank's data loss (sum of the per-CTA partials of the scatter kernel), by the CTA that owns the loss slot
   if (owns_loss) {                                   // CTA-uniform; all threads: four independent loads each, not 64 in a chain
@@ -222,16 +231,37 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
   };
 
   // optimizer update of the (up to four) parameters whose gradient is flat element i; returns the regulariser share
-  auto apply = [&](int64_t i, float4 gv) {
+  // the touched bits (bit j: float 4i+j) of flat element i from this rank's stamps
+  auto local_bits = [&](int64_t i) {
+    uint32_t m = 0;
+    if (!TOUCHED || i >= n_g4) return m;
+    for (int sgi = 0; sgi < a.n_seg; sgi++) {
+      const DpSeg& sg = a.seg[sgi];
+      if (sg.width == 0) continue;
+#pragma unroll
+      for (int j = 0; j < 4; j++) {
+        const int64_t e = 4 * i + j - sg.off;
+        if (e >= 0 && e < sg.n && __ldg(a.stamps + e / sg.width) == a.stamp) m |= 1u << j;
+      }
+    }
+    return m;
+  };
+
+  // optimizer update of the (up to four) parameters whose gradient is flat element i; returns the regulariser share.
+  // TOUCHED: a float of a segment with a row width moves only if its bit in `tbits` is set, with g_eff = g (no L2 term),
+  // as in opt.cu::opt_rows_kernel
+  auto apply = [&](int64_t i, float4 gv, uint32_t tbits) {
     float reg = 0.f;
     const int64_t f0 = 4 * i;
     for (int sgi = 0; sgi < a.n_seg; sgi++) {
       const DpSeg& sg = a.seg[sgi];
       if (f0 + 4 <= sg.off || f0 >= sg.off + sg.n) continue;
+      const bool rows = TOUCHED && sg.width > 0;
+      if (rows && tbits == 0) continue;
       OptP2 p = a.p;
       p.lamda = sg.lamda;
       const int64_t e0 = f0 - sg.off;
-      if (e0 >= 0 && e0 + 4 <= sg.n && (e0 & 3) == 0) {
+      if (e0 >= 0 && e0 + 4 <= sg.n && (e0 & 3) == 0 && (!rows || tbits == 0xFu)) {
         float4* w4 = reinterpret_cast<float4*>(sg.w + e0);
         float4* a4 = reinterpret_cast<float4*>(sg.s1 + e0);
         float4* b4 = reinterpret_cast<float4*>(sg.s2 + e0);
@@ -239,7 +269,7 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
         float4 av = (KIND != HHFM_OPT_SGD) ? *a4 : f4_zero();
         float4 bv = (KIND == HHFM_OPT_ADAM) ? *b4 : f4_zero();
         const float sq = f4_dot(wv, wv);
-        float4 ge = f4_fma(wv, p.lamda, gv);
+        float4 ge = rows ? gv : f4_fma(wv, p.lamda, gv);
         opt_elem2<KIND>(wv.x, av.x, bv.x, ge.x, p);
         opt_elem2<KIND>(wv.y, av.y, bv.y, ge.y, p);
         opt_elem2<KIND>(wv.z, av.z, bv.z, ge.z, p);
@@ -255,11 +285,12 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
       for (int j = 0; j < 4; j++) {
         const int64_t e = e0 + j;
         if (e < 0 || e >= sg.n) continue;
+        if (rows && !((tbits >> j) & 1u)) continue;
         float wv = sg.w[e];
         float av = (KIND != HHFM_OPT_SGD) ? sg.s1[e] : 0.f;
         float bv = (KIND == HHFM_OPT_ADAM) ? sg.s2[e] : 0.f;
         if (sg.lamda > 0.f) reg += 0.5f * sg.lamda * wv * wv;
-        float ge = fmaf(wv, p.lamda, gs[j]);
+        float ge = rows ? gs[j] : fmaf(wv, p.lamda, gs[j]);
         opt_elem2<KIND>(wv, av, bv, ge, p);
         sg.w[e] = wv;
         if (KIND != HHFM_OPT_SGD) sg.s1[e] = av;
@@ -280,7 +311,7 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
       if (i >= total4) continue;
       const float4 v = take(i);
       if (i == n_g4) { loss_all = v.x; has_loss = true; }
-      else reg += apply(i, v);
+      else reg += apply(i, v, local_bits(i));
     }
   } else {
     // ---- A: my pieces -> X ----
@@ -289,6 +320,14 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
       if (p >= n_pieces) break;
       const int64_t i = p * kPiece + lane;
       if (i < total4) x4[i] = take(i);
+      if (TOUCHED) {
+        const uint32_t nib = (i < total4) ? local_bits(i) << (4 * (lane & 7)) : 0u;
+#pragma unroll
+        for (int w = 0; w < 4; w++) {
+          const uint32_t word = __reduce_or_sync(0xffffffffu, (lane >> 3) == w ? nib : 0u);
+          if (lane == w) xmask[4 * p + w] = word;
+        }
+      }
     }
     // the CTA barrier orders every thread's stores before the signalling lanes, whose system-scope fence + release store is
     // cumulative over them: no per-thread system fence
@@ -300,6 +339,12 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
       const int64_t p = piece_of(L);
       if (p >= n_pieces) break;
       const int64_t i = p * kPiece + lane;
+      if (TOUCHED && lane < 4) {                     // the piece's touched mask: OR over the ranks, into every rank's X
+        const int64_t wi = (reinterpret_cast<float*>(xmask) - a.x) + 4 * p + lane;
+        uint32_t m = 0;
+        for (int r = 0; r < N; r++) m |= __ldcv(reinterpret_cast<const unsigned int*>(a.x_peer[r] + wi));
+        for (int r = 0; r < N; r++) *reinterpret_cast<uint32_t*>(a.x_peer[r] + wi) = m;
+      }
       if (i >= total4) continue;
       if (a.x_mc != nullptr) {
         const float4 v = multimem_ld_reduce4(a.x_mc + 4 * i);
@@ -328,8 +373,10 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
       const int64_t i = p * kPiece + lane;
       if (i >= total4) continue;
       const float4 v = ld_cv4(x4 + i);
+      const uint32_t tbits = TOUCHED ? (__ldcv(reinterpret_cast<const unsigned int*>(xmask) + 4 * p + (lane >> 3)) >> (4 * (lane & 7))) & 0xFu
+                                     : 0u;
       if (i == n_g4) { loss_all = v.x; has_loss = true; }
-      else reg += apply(i, v);
+      else reg += apply(i, v, tbits);
     }
   }
 
@@ -356,12 +403,12 @@ __global__ void __launch_bounds__(kDpThreads) dp_step_kernel(const DpArgs a) {
   }
 }
 
-template <int KIND>
+template <int KIND, bool TOUCHED>
 static int launch_dp(const DpArgs& a, cudaStream_t st) {
   static int grid_cached = 0;
   if (grid_cached == 0) {
     int per_sm = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, dp_step_kernel<KIND>, kDpThreads, 0);
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, dp_step_kernel<KIND, TOUCHED>, kDpThreads, 0);
     if (e != cudaSuccess || per_sm < 1) {
       set_error("dp_step: occupancy query failed: %s", cudaGetErrorString(e));
       cudaGetLastError();
@@ -375,10 +422,10 @@ static int launch_dp(const DpArgs& a, cudaStream_t st) {
   static const bool coop = [] { const char* e = getenv("HHFM_DP_COOP"); return e && e[0] == '1'; }();
   cudaError_t e = cudaSuccess;
   if (a.n_ranks == 1 || !coop) {
-    dp_step_kernel<KIND><<<grid_cached, kDpThreads, 0, st>>>(a);
+    dp_step_kernel<KIND, TOUCHED><<<grid_cached, kDpThreads, 0, st>>>(a);
   } else {
     void* params[] = {(void*)&a};
-    e = cudaLaunchCooperativeKernel((const void*)dp_step_kernel<KIND>, dim3(grid_cached), dim3(kDpThreads), params, 0, st);
+    e = cudaLaunchCooperativeKernel((const void*)dp_step_kernel<KIND, TOUCHED>, dim3(grid_cached), dim3(kDpThreads), params, 0, st);
   }
   if (e != cudaSuccess) {
     set_error("dp_step_kernel: cooperative launch failed: %s", cudaGetErrorString(e));
@@ -399,12 +446,12 @@ extern "C" int64_t hhfm_dp_exchange_floats(int64_t n_grad) {
 
 extern "C" int64_t hhfm_dp_flag_ints(void) { return 2 * 256 * kMaxPeers; }
 
-extern "C" int hhfm_dp_step(int32_t kind, const hhfm_dp_segment* segs, int32_t n_segs, float* arena, int64_t n_grad,
-                            float* ghot, float* ghot_bias, int32_t n_rep, int32_t n_hot, int64_t K, int64_t M,
-                            const int32_t* hot_slot, int64_t bias_off, const float* loss_partials, float* x_local, float* x_multicast,
-                            const int64_t* x_peers_host, const int64_t* flag_peers_host, int32_t rank, int32_t n_ranks,
-                            int32_t* state, float lr, float beta1, float beta2, float eps, float* reg_workspace,
-                            float* loss_out, double timeout_s, hhfm_stream_t stream) {
+// argument checks and DpArgs of hhfm_dp_step / hhfm_dp_step_touched (the segments' widths are 0: dense)
+static int dp_prepare(DpArgs& a, int32_t kind, const hhfm_dp_segment* segs, int32_t n_segs, float* arena, int64_t n_grad,
+                      float* ghot, float* ghot_bias, int32_t n_rep, int32_t n_hot, int64_t K, int64_t M, const int32_t* hot_slot,
+                      int64_t bias_off, const float* loss_partials, float* x_local, float* x_multicast, const int64_t* x_peers_host,
+                      const int64_t* flag_peers_host, int32_t rank, int32_t n_ranks, int32_t* state, float lr, float beta1,
+                      float beta2, float eps, float* reg_workspace, float* loss_out, double timeout_s) {
   HHFM_REQUIRE(segs && n_segs >= 1 && n_segs <= kMaxSegs, "dp_step: 1..4 segments");
   HHFM_REQUIRE(arena && n_grad > 0 && loss_partials && x_local && state && reg_workspace && loss_out, "dp_step: NULL argument");
   HHFM_REQUIRE(n_ranks >= 1 && n_ranks <= kMaxPeers && rank >= 0 && rank < n_ranks, "dp_step: bad rank / n_ranks");
@@ -413,7 +460,7 @@ extern "C" int hhfm_dp_step(int32_t kind, const hhfm_dp_segment* segs, int32_t n
   HHFM_REQUIRE((((uintptr_t)arena | (uintptr_t)x_local | (uintptr_t)x_multicast) & 15) == 0, "dp_step: buffers must be 16-byte aligned");
   HHFM_REQUIRE(K > 0 && K % 4 == 0 && M > 0 && M * K <= n_grad, "dp_step: the table gradient [M, K] must lead the arena");
   HHFM_REQUIRE(ghot == nullptr || (n_rep >= 1 && n_hot >= 1 && hot_slot), "dp_step: bad hot-row plan");
-  DpArgs a;
+  HHFM_REQUIRE(kind >= HHFM_OPT_ADAGRAD && kind <= HHFM_OPT_SGD, "dp_step: unknown optimizer kind %d", kind);
   memset(&a, 0, sizeof(a));
   a.n_seg = n_segs;
   for (int i = 0; i < n_segs; i++) {
@@ -423,7 +470,7 @@ extern "C" int hhfm_dp_step(int32_t kind, const hhfm_dp_segment* segs, int32_t n
     HHFM_REQUIRE(kind != HHFM_OPT_ADAM || s.s2, "dp_step: adam needs two state buffers");
     HHFM_REQUIRE((s.offset & 3) != 0 || s.n < 4 || (((uintptr_t)s.w | (uintptr_t)s.s1 | (uintptr_t)s.s2) & 15) == 0,
                  "dp_step: segment buffers must be 16-byte aligned");
-    a.seg[i] = DpSeg{s.w, s.s1, s.s2, s.offset, s.n, s.lamda};
+    a.seg[i] = DpSeg{s.w, s.s1, s.s2, s.offset, s.n, s.lamda, 0};
   }
   a.arena = arena;
   a.n_g = n_grad;
@@ -458,12 +505,63 @@ extern "C" int hhfm_dp_step(int32_t kind, const hhfm_dp_segment* segs, int32_t n
     static const int fences = [] { const char* e = getenv("HHFM_DP_FENCES"); return (e && e[0] == '1') ? 1 : 0; }();
     a.fences = fences;
   }
-  cudaStream_t st = (cudaStream_t)stream;
+  return HHFM_OK;
+}
+
+template <bool TOUCHED>
+static int launch_dp_kind(int32_t kind, const DpArgs& a, cudaStream_t st) {
   switch (kind) {
-    case HHFM_OPT_ADAGRAD: return launch_dp<HHFM_OPT_ADAGRAD>(a, st);
-    case HHFM_OPT_ADAM: return launch_dp<HHFM_OPT_ADAM>(a, st);
-    case HHFM_OPT_MOMENTUM: return launch_dp<HHFM_OPT_MOMENTUM>(a, st);
-    case HHFM_OPT_SGD: return launch_dp<HHFM_OPT_SGD>(a, st);
+    case HHFM_OPT_ADAGRAD: return launch_dp<HHFM_OPT_ADAGRAD, TOUCHED>(a, st);
+    case HHFM_OPT_ADAM: return launch_dp<HHFM_OPT_ADAM, TOUCHED>(a, st);
+    case HHFM_OPT_MOMENTUM: return launch_dp<HHFM_OPT_MOMENTUM, TOUCHED>(a, st);
+    case HHFM_OPT_SGD: return launch_dp<HHFM_OPT_SGD, TOUCHED>(a, st);
     default: set_error("dp_step: unknown optimizer kind %d", kind); return HHFM_ERR_BAD_ARG;
   }
+}
+
+extern "C" int hhfm_dp_step(int32_t kind, const hhfm_dp_segment* segs, int32_t n_segs, float* arena, int64_t n_grad,
+                            float* ghot, float* ghot_bias, int32_t n_rep, int32_t n_hot, int64_t K, int64_t M,
+                            const int32_t* hot_slot, int64_t bias_off, const float* loss_partials, float* x_local, float* x_multicast,
+                            const int64_t* x_peers_host, const int64_t* flag_peers_host, int32_t rank, int32_t n_ranks,
+                            int32_t* state, float lr, float beta1, float beta2, float eps, float* reg_workspace,
+                            float* loss_out, double timeout_s, hhfm_stream_t stream) {
+  DpArgs a;
+  const int rc = dp_prepare(a, kind, segs, n_segs, arena, n_grad, ghot, ghot_bias, n_rep, n_hot, K, M, hot_slot, bias_off,
+                            loss_partials, x_local, x_multicast, x_peers_host, flag_peers_host, rank, n_ranks, state, lr, beta1,
+                            beta2, eps, reg_workspace, loss_out, timeout_s);
+  if (rc != HHFM_OK) return rc;
+  return launch_dp_kind<false>(kind, a, (cudaStream_t)stream);
+}
+
+extern "C" int64_t hhfm_dp_exchange_floats_touched(int64_t n_grad) {
+  if (n_grad < 1) return -1;
+  const int64_t total4 = (n_grad + 3) / 4 + 1;
+  return (total4 + (total4 + kPiece - 1) / kPiece) * 4;
+}
+
+extern "C" int hhfm_dp_step_touched(int32_t kind, const hhfm_dp_segment* segs, int32_t n_segs, const int32_t* seg_widths,
+                                    const int32_t* stamps, int32_t stamp, float* arena, int64_t n_grad, float* ghot,
+                                    float* ghot_bias, int32_t n_rep, int32_t n_hot, int64_t K, int64_t M,
+                                    const int32_t* hot_slot, int64_t bias_off, const float* loss_partials, float* x_local,
+                                    float* x_multicast, const int64_t* x_peers_host, const int64_t* flag_peers_host,
+                                    int32_t rank, int32_t n_ranks, int32_t* state, float lr, float beta1, float beta2,
+                                    float eps, float* reg_workspace, float* loss_out, double timeout_s, hhfm_stream_t stream) {
+  HHFM_REQUIRE(seg_widths, "dp_step_touched: seg_widths is NULL");
+  DpArgs a;
+  const int rc = dp_prepare(a, kind, segs, n_segs, arena, n_grad, ghot, ghot_bias, n_rep, n_hot, K, M, hot_slot, bias_off,
+                            loss_partials, x_local, x_multicast, x_peers_host, flag_peers_host, rank, n_ranks, state, lr, beta1,
+                            beta2, eps, reg_workspace, loss_out, timeout_s);
+  if (rc != HHFM_OK) return rc;
+  for (int i = 0; i < n_segs; i++) {
+    const int32_t wd = seg_widths[i];
+    HHFM_REQUIRE(wd >= 0, "dp_step_touched: negative row width");
+    if (wd == 0) continue;
+    HHFM_REQUIRE(stamps, "dp_step_touched: a segment with a row width needs the stamp array");
+    HHFM_REQUIRE(segs[i].n % wd == 0 && segs[i].n / wd <= M, "dp_step_touched: segment %d is not [rows <= M, width]", i);
+    HHFM_REQUIRE(segs[i].lamda == 0.f, "dp_step_touched: a segment with a row width takes no L2 term");
+    a.seg[i].width = wd;
+  }
+  a.stamps = stamps;
+  a.stamp = stamp;
+  return launch_dp_kind<true>(kind, a, (cudaStream_t)stream);
 }

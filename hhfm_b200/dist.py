@@ -38,6 +38,16 @@ def allreduce_arena(arena, group=None):
     return arena
 
 
+def union_touched(stamp_arr, group=None):
+    """Rows touched on any rank (TF1 SparseApplyMomentum over the global batch): every rank stamps the rows its shard touched
+    with the step's stamp, which is the same on every rank and larger than any earlier one, so an element-wise MAX over the
+    ranks carries the stamp exactly on the union.  One all-reduce of the int32 stamp array (4 B per row), in place; the
+    arrays are identical on every rank afterwards."""
+    if dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(stamp_arr, op=dist.ReduceOp.MAX, group=group)
+    return stamp_arr
+
+
 def gather_candidates(local_scores, local_ids, group=None):
     """All-gather of the per-shard candidate lists: [C, tl] per rank -> [C, ws*tl] (rank order).  torch.distributed
     plumbing only (NCCL on the GPUs, gloo in the CPU tests)."""

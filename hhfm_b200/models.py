@@ -102,6 +102,7 @@ class _Base:
         self._opt = Optimizer(optimizer_type, learning_rate, initial_accumulator_value=acc0)
         self._lamda = float(lamda)
         self._touch = TouchTracker(self._M, self.device)
+        self._touch_live = False   # the scatter kernels of this step stamp touched rows (set by _touch_args)
         self._idx_stage = Staging(torch.int32, self.device)
         self._uploader = RecordUploader(self.device)
         self._f32_stage = Staging(torch.float32, self.device)
@@ -215,7 +216,10 @@ class _Base:
         `sparse`: exchange the COALESCED touched rows (row id + gradient row, all-gather) instead of the dense [M, K]
         gradient, then add the ranks' lists in rank order and run the touched-row optimizer on the union.  Only for
         lamda == 0 (IndexedSlices semantics; a dense L2 term touches every row anyway).  "auto": tables above 64 MB
-        (SURVEY 8e); `HHFM_DP_SPARSE=0/1` forces either."""
+        (SURVEY 8e); `HHFM_DP_SPARSE=0/1` forces either.
+
+        MomentumOptimizer runs on all three exchanges: its IndexedSlices variables (feature_bias, and V with lamda == 0)
+        take SparseApplyMomentum over the union of the rows touched on any rank (DESIGN.md 6)."""
         import torch.distributed as dist
         from . import dist as hd
         if not dist.is_initialized():
@@ -236,16 +240,13 @@ class _Base:
             sparse = self._M * self._K * 4 > (64 << 20)
         self._dp_sparse = bool(sparse) and self._lamda <= 0 and ws > 1 and self._supports_sparse_dp
         if self._dp_sparse:
-            if self._opt.kind == "momentum":
-                raise NotImplementedError("sparse Momentum under data parallelism is not implemented")
             return
         env = os.environ.get("HHFM_DP_FUSED", os.environ.get("HHFM_DP_P2P"))      # 0 / 1 force NCCL / the fused exchange
         if env == "0":
             fused = False
         elif env == "1":
             fused = True
-        want = bool(fused) and ws > 1 and self.device.type == "cuda" and self._fused_segments() is not None \
-            and self._opt.kind != "momentum"
+        want = bool(fused) and ws > 1 and self.device.type == "cuda" and self._fused_segments() is not None
         if not want:
             if fused is True and ws > 1:
                 raise _lib.HhfmError("enable_data_parallel: the fused exchange does not cover this model / optimizer")
@@ -265,7 +266,9 @@ class _Base:
         if agree(err is None):
             try:
                 n_v, n_b, _ = self._arena_layout
-                n_x = int(_lib.load().hhfm_dp_exchange_floats(n_v + n_b + 1))
+                lib = _lib.load()
+                n_x = int(lib.hhfm_dp_exchange_floats_touched(n_v + n_b + 1) if self._opt.kind == "momentum"
+                          else lib.hhfm_dp_exchange_floats(n_v + n_b + 1))
                 dpx = hd.SymmExchange(n_x, self.device, self._dp_group)      # collective (phase 2)
             except Exception as e:
                 err = e
@@ -287,12 +290,14 @@ class _Base:
 
     def _use_fused_tail(self):
         """The one-kernel tail (csrc/p2p.cu) replaces hot_fold + [all-reduce] + dense optimizer + loss_finalize whenever the
-        dense optimizer kernels would run; the touched-row (IndexedSlices) path and Momentum keep their own kernels."""
-        if not self._fused or self._fused_segments() is None or self._opt.kind == "momentum":
+        dense optimizer kernels would run; the touched-row (IndexedSlices) path keeps its own kernels on one GPU, and so
+        does Momentum.  Under the fused exchange (n_ranks > 1) Momentum's IndexedSlices variables move in the same kernel
+        (hhfm_dp_step_touched)."""
+        if not self._fused or self._fused_segments() is None:
             return False
         if self._dp_group is not None:
             return self._dpx is not None
-        return self._lamda > 0 and not self._lazy()
+        return self._lamda > 0 and not self._lazy() and self._opt.kind != "momentum"
 
     def _fused_tail(self, hot, with_hot_bias):
         from . import dist as hd
@@ -313,6 +318,7 @@ class _Base:
         n_g = n_v + n_b + 1
         o = self._opt
         lr = o._lr_t() if o.kind == "adam" else o.lr
+        b1 = o.momentum if o.kind == "momentum" else o.beta1
         dpx = self._dpx
         if dpx is None:
             if self._x_local is None:
@@ -326,9 +332,17 @@ class _Base:
                      ptr(hot.slot), n_v)
         else:
             hargs = (None, None, 0, 0, self._K, self._M, None, n_v)
-        _lib.call("hhfm_dp_step", o.KIND_ID[o.kind], C.cast(arr, C.c_void_p), n_seg, ptr(self._arena), n_g, *hargs,
-                  ptr(self._loss_partials), ptr(x), mc, xt, ft, rank, ws, ptr(self._dp_state), lr, o.beta1, o.beta2, o.eps,
-                  ptr(self._reg_ws), ptr(self._loss_dev), float(os.environ.get("HHFM_DP_TIMEOUT_S", "120")), cur_stream())
+        tail = (ptr(self._loss_partials), ptr(x), mc, xt, ft, rank, ws, ptr(self._dp_state), lr, b1, o.beta2, o.eps,
+                ptr(self._reg_ws), ptr(self._loss_dev), float(os.environ.get("HHFM_DP_TIMEOUT_S", "120")), cur_stream())
+        if o.kind == "momentum":
+            # IndexedSlices variables (lamda 0; feature_bias always) move on the rows touched on some rank only
+            widths = (C.c_int32 * n_seg)(*[int(n) // self._M if (lam == 0.0 and self._sparse_var(name)) else 0
+                                          for name, w, off, n, lam in self._fused_segments()])
+            t = self._touch
+            _lib.call("hhfm_dp_step_touched", o.KIND_ID[o.kind], C.cast(arr, C.c_void_p), n_seg, widths, ptr(t.stamp_arr),
+                      t.stamp, ptr(self._arena), n_g, *hargs, *tail)
+        else:
+            _lib.call("hhfm_dp_step", o.KIND_ID[o.kind], C.cast(arr, C.c_void_p), n_seg, ptr(self._arena), n_g, *hargs, *tail)
         self._version += 1
 
     def _finish_step(self, hot, with_hot_bias, bias_step=None):
@@ -355,14 +369,21 @@ class _Base:
         self._enqueue_loss(with_reg)
 
     def _allreduce_grads(self):
-        """NCCL path: one all-reduce of the arena (dense) or the coalesced-sparse row exchange."""
+        """NCCL path: one all-reduce of the arena (dense) or the coalesced-sparse row exchange.  With Momentum the dense
+        exchange also takes the union of the touched rows: one MAX all-reduce of the stamp array (4 B per row, no host
+        sync), then the rows carrying this step's stamp are compacted into the touched-row list."""
         if self._dp_group is None:
             return
         if self._dp_sparse:
             self._exchange_sparse_rows()
             return
         import torch.distributed as dist
+        from . import dist as hd
         dist.all_reduce(self._arena, group=self._dp_group)
+        if self._opt.kind == "momentum" and self._touch_live:
+            t = self._touch
+            hd.union_touched(t.stamp_arr, self._dp_group)
+            _lib.call("hhfm_touched_compact", ptr(t.stamp_arr), t.stamp, self._M, ptr(t.rows), ptr(t.count), cur_stream())
 
     def _exchange_sparse_rows(self):
         """SURVEY 8e, tables too large for a dense all-reduce: all-gather the coalesced (row id, gradient row) lists, clear
@@ -451,10 +472,16 @@ class _Base:
         ids, _ = hd.merge_topk(sc, ids, tp, grp)
         return ids.cpu().numpy()
 
+    def _sparse_var(self, name):
+        """True for the variables that receive IndexedSlices: feature_bias, and V without the dense L2 term."""
+        return name == "feature_bias" or (name == "feature_embeddings" and self._lamda <= 0)
+
     def _touch_args(self, extra=False):
-        """Touched-row tracking is only paid for when a *_rows optimizer will consume the list."""
-        need = (self._dp_group is None or self._dp_sparse) and (self._lamda <= 0 or extra)
-        if not need or self._lazy():            # lazy mode: the list was built from the ids before the forward
+        """Touched-row tracking is only paid for when a *_rows optimizer (or, for Momentum under data parallelism, the
+        union of the ranks' touched rows) will consume the stamps."""
+        need = (self._dp_group is None or self._dp_sparse or self._opt.kind == "momentum") and (self._lamda <= 0 or extra)
+        self._touch_live = need and not self._lazy()
+        if not self._touch_live:                # lazy mode: the list was built from the ids before the forward
             return (None, 0, None, None)
         self._touch.begin_step()
         return (ptr(self._touch.stamp_arr), self._touch.stamp, ptr(self._touch.rows), ptr(self._touch.count))
@@ -465,12 +492,10 @@ class _Base:
         lamda == 0: IndexedSlices semantics; Adagrad/SGD/Adam dense kernels are exactly equivalent on untouched
         rows (g = 0), Momentum needs the touched-row list."""
         V = self.weights["feature_embeddings"]
-        use_rows = sparse_ok and self._lamda <= 0 and (self._dp_group is None or self._dp_sparse)
+        use_rows = sparse_ok and self._lamda <= 0 and (self._dp_group is None or self._dp_sparse or self._opt.kind == "momentum")
         if use_rows:
             self._opt.apply_rows("feature_embeddings", V, self._gV, self._touch.rows, self._touch.count, self._K)
             return False
-        if self._lamda <= 0 and self._opt.kind == "momentum":
-            raise NotImplementedError("sparse Momentum under data parallelism is not implemented")
         sq = self._sq_partials if self._lamda > 0 else None
         self._apply_arena_dense("feature_embeddings", V, self._gV, self._lamda if self._lamda > 0 else 0.0, sq)
         return self._lamda > 0
@@ -732,8 +757,6 @@ class FM(_Base):
         # feature_bias receives IndexedSlices (only touched rows move); the scalar bias is dense.
         bias = self.weights["feature_bias"]
         if self._opt.kind == "momentum":
-            if self._dp_group is not None:
-                raise NotImplementedError("sparse Momentum under data parallelism is not implemented")
             self._opt.apply_rows("feature_bias", bias, self._gb, self._touch.rows, self._touch.count, 1)
         else:
             self._apply_arena_dense("feature_bias", bias, self._gb, 0.0, None)

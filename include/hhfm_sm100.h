@@ -477,6 +477,11 @@ int hhfm_opt_sgd_rows(float* w, float* g, const int32_t* rows, const int32_t* n_
  *   hhfm_opt_adagrad_rows_l2: step `step` on the listed rows with g_eff = g + lamda*w; sets last_step = step. */
 int hhfm_mark_rows(const int32_t* ids, int64_t n, int32_t* stamp_arr, int32_t stamp, int64_t M, int32_t* rows, int32_t* count,
                    hhfm_stream_t stream);
+/* hhfm_touched_compact: rows[0, *count) = the rows r < M with stamp_arr[r] == stamp (any order; *count is cleared first).
+ *   Under data parallelism with Momentum the ranks' stamp arrays are MAX all-reduced (one int32 per row) and compacted
+ *   here: the list is then the union of the rows touched on any rank, which SparseApplyMomentum (K5 *_rows) consumes. */
+int hhfm_touched_compact(const int32_t* stamp_arr, int32_t stamp, int64_t M, int32_t* rows, int32_t* count,
+                         hhfm_stream_t stream);
 int hhfm_opt_adagrad_l2_replay(float* w, float* acc, int32_t* last_step, const int32_t* rows, const int32_t* n_rows_dev,
                                int64_t max_rows, int64_t M, int64_t K, float lr, float lamda, int32_t upto, hhfm_stream_t stream);
 int hhfm_opt_adagrad_rows_l2(float* w, float* acc, float* g, const int32_t* rows, const int32_t* n_rows_dev, int64_t max_rows,
@@ -534,6 +539,21 @@ int hhfm_dp_step(int32_t kind, const hhfm_dp_segment* segs, int32_t n_segs, floa
                  const float* loss_partials, float* x_local, float* x_multicast, const int64_t* x_peers_host,
                  const int64_t* flag_peers_host, int32_t rank, int32_t n_ranks, int32_t* state, float lr, float beta1,
                  float beta2, float eps, float* reg_workspace, float* loss_out, double timeout_s, hhfm_stream_t stream);
+/* hhfm_dp_step_touched: hhfm_dp_step with IndexedSlices variables (TF1 SparseApply*: only the rows touched on SOME rank
+ *   move; a touched row whose summed gradient is 0 still takes the step, e.g. Momentum's accum decays).  seg_widths (host,
+ *   n_segs): row width of each segment, 0 = dense as in hhfm_dp_step; a segment with a width w covers rows [0, n / w) of
+ *   the table (n / w <= M, lamda 0).  stamps [M] / stamp: this rank's touched-row stamps from the scatter kernels (K1).
+ *   Each rank's touched bits travel with its gradient and are OR-reduced with it, so every replica makes the same
+ *   decision; with n_ranks == 1 the local stamps decide.  x_local then holds hhfm_dp_exchange_floats_touched(n_grad)
+ *   floats.  Other arguments as hhfm_dp_step; any optimizer kind. */
+int64_t hhfm_dp_exchange_floats_touched(int64_t n_grad);
+int hhfm_dp_step_touched(int32_t kind, const hhfm_dp_segment* segs, int32_t n_segs, const int32_t* seg_widths,
+                         const int32_t* stamps, int32_t stamp, float* arena, int64_t n_grad, float* ghot, float* ghot_bias,
+                         int32_t n_rep, int32_t n_hot, int64_t K, int64_t M, const int32_t* hot_slot, int64_t bias_off,
+                         const float* loss_partials, float* x_local, float* x_multicast, const int64_t* x_peers_host,
+                         const int64_t* flag_peers_host, int32_t rank, int32_t n_ranks, int32_t* state, float lr,
+                         float beta1, float beta2, float eps, float* reg_workspace, float* loss_out, double timeout_s,
+                         hhfm_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K10  CARS2 (CARS2.py:66-187), the context-aware baseline of main.py:50-63.
